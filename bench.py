@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark contract for the B200-native RRDBNet generator (MiNeves00/SR-GAN-FD hot path).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 Workload at every N = BASELINE.json configs[1]/[2]: RRDBNet x4 (23 RRDB, 64 ch, growth 32) L1 pre-training step,
 forward + backward, 16 synthetic 64x64 LR images per GPU -> 256x256 GT, bf16 tensor-core arithmetic with fp32
@@ -179,6 +179,30 @@ def bench_config(world):
             "l2_policy": "activation working set per step (3.1 GB) is far larger than the 126 MB L2, no flush needed",
             "host": "python cyclic GC collected before and disabled inside each timed region",
             "precision": "bf16 operands / fp32 accumulate in the trunk, fp32 residual carrier, hi+lo split bf16 in head/tail"}
+
+
+def seeded_inputs(rank=0):
+    """The LR and GT batches of one rank's training step: the same on every run."""
+    import torch
+    torch.manual_seed(1234 + rank)
+    return torch.rand(BATCH_PER_GPU, 3, LR_HW, LR_HW), torch.rand(BATCH_PER_GPU, 3, LR_HW * SCALE, LR_HW * SCALE)
+
+
+GRAD_SAMPLE = 1 << 23  # entries of the 16.7 M-entry flat gradient that --dump-outputs writes (34 MB; 46 MB with sr.npy)
+
+
+def dump_outputs(out_dir, sr, loss, net):
+    """Write what one training step hands its caller, as float32 .npy files under `out_dir`: `sr` (the SR batch), `loss` (the L1
+    loss) and `grad_sample` -- the parameter gradients flattened in `net.parameters()` order, sampled at GRAD_SAMPLE fixed
+    positions (a seed-0 permutation, ascending), because the whole gradient (67 MB) next to the SR batch (13 MB) would not fit
+    the dump's 64 MB."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    flat = torch.cat([p.grad.flatten() for p in net.parameters()])
+    idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(0))[:GRAD_SAMPLE].sort().values
+    for name, t in (("sr", sr), ("loss", loss), ("grad_sample", flat[idx.to(flat.device)])):
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
 
 
 def run_reference(args):
@@ -383,15 +407,16 @@ def run_b200(args):
         if not dp_err < 2e-3:
             raise RuntimeError(f"data-parallel gradients differ from the single-replica gradients: rel-L2 {dp_err:.3e}")
 
-    torch.manual_seed(1234 + rank)
-    lr_host = torch.rand(BATCH_PER_GPU, 3, LR_HW, LR_HW).pin_memory()
-    gt_host = torch.rand(BATCH_PER_GPU, 3, LR_HW * SCALE, LR_HW * SCALE).pin_memory()
+    lr_host, gt_host = (t.pin_memory() for t in seeded_inputs(rank))
     lr_dev, gt_dev = lr_host.to(dev), gt_host.to(dev)
+    last = {}  # what the latest resident step returned (detached: the autograd graph is not kept alive), for --dump-outputs
 
     def step_resident():
         net.zero_grad(set_to_none=True)
-        loss = F.l1_loss(net(lr_dev), gt_dev)
+        sr = net(lr_dev)
+        loss = F.l1_loss(sr, gt_dev)
         loss.backward()
+        last.update(sr=sr.detach(), loss=loss.detach())
         return loss
 
     # End to end through the public API.  Like the reference's CUDAPrefetcher (ESRGAN/dataset.py:196-236) the NEXT batch is
@@ -485,6 +510,9 @@ def run_b200(args):
         sampler.start()
     ms_total = timed(step_resident, args.steps)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last["sr"], last["loss"], net)
+    last.clear()
     plan = net._runtime().last_plan
     bucketed = world > 1 and net._runtime().grad_bucket_hook is not None
     ms_step = ms_total / args.steps
@@ -691,7 +719,12 @@ def main():
     ap.add_argument("--frame", type=int, default=1024)
     ap.add_argument("--halo", type=int, default=16)
     ap.add_argument("--bands-per-rank", type=int, default=1)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/{sr,loss,grad_sample}.npy (see dump_outputs); "
+                         "the inputs are seeded, so two builds run with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "train"):
+        ap.error("--dump-outputs applies to the train workload of --impl b200")
     if args.gpus > 1 and "WORLD_SIZE" not in os.environ:
         # convenience: the driver launches N>1 through torch.distributed.run itself; do the same when run by hand
         os.execvp(sys.executable, [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={args.gpus}",

@@ -18,9 +18,19 @@ import pytest
 import torch
 
 from oracle import disc_oracle as do
+from oracle import make_golden
 from oracle import reference_loader as rl
 
 GOLDEN = sorted(glob.glob(os.path.join(os.path.dirname(__file__), "golden", "disc", "*.pt")))
+
+
+@pytest.fixture
+def golden_threads():
+    """the thread count the fixture was computed with (bit equality depends on it), whatever the host or an earlier test set"""
+    n = torch.get_num_threads()
+    torch.set_num_threads(make_golden.THREADS)
+    yield
+    torch.set_num_threads(n)
 
 
 def rel_l2(a, b):
@@ -145,6 +155,7 @@ def test_disc_plan_host_bookkeeping():
         assert L.b200sr_disc_plan_create(C.byref(bad), C.byref(h)) < 0 and L.b200sr_last_error()
 
 
+@pytest.mark.usefixtures("golden_threads")
 @pytest.mark.parametrize("path", GOLDEN, ids=[os.path.basename(p) for p in GOLDEN])
 def test_disc_oracle_matches_golden(path):
     """seed + drop-in constructor reproduces the reference's parameters; the oracle reproduces the reference's logits and gradients"""

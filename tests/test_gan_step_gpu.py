@@ -1,9 +1,11 @@
-"""BASELINE configs[4] harness check (1 GPU): one BSRGAN GAN iteration (``BSRGAN/train_bsrgan.py:412-470``) with the reference's
-own ``DiscriminatorUNet`` and ``ContentLoss`` (seeded random-init VGG19 patched into torchvision: no ImageNet weights offline),
+"""BASELINE configs[4] harness check (1 GPU): one BSRGAN GAN iteration (``BSRGAN/train_bsrgan.py:412-470``) with a
+``DiscriminatorUNet`` and a ``ContentLoss`` (seeded random-init VGG19 patched into torchvision: no ImageNet weights offline),
 a discriminator optimizer step BETWEEN the generator's forward and backward, and the generator backward under the summed
 (20 x L1 + 1 x content + 0.5 x adversarial) x 65536 upstream gradient.  The generator's parameter gradients must match the fp32
-oracle driven by the SAME upstream gradient.  Needs the reference tree for the critics (/root/reference, or the staged copy under baseline/_ref on the GPU box; a log of a run
-on a B200 with a staged copy is kept in profiles/r2_gan_step.log)."""
+oracle driven by the SAME upstream gradient.  The critics are the reference's own classes where its tree is present
+($SRGANFD_REFERENCE), else the drop-in critics through their stock torch paths -- the reference's op sequences (the
+discriminator's pinned against it by tests/golden/disc).  A log of a run on a B200 with the reference's critics is kept in
+profiles/r2_gan_step_test.log."""
 import os
 import sys
 
@@ -18,15 +20,15 @@ from sr_gan_fd_b200.compat._passthrough import reference_root
 # __graft_entry__.stage_reference() under baseline/_ref (git-ignored, travels with the snapshot)
 REF = reference_root()
 os.environ["SRGANFD_REFERENCE"] = REF
-pytestmark = [pytest.mark.gpu,
-              pytest.mark.skipif(not os.path.isfile(os.path.join(REF, "BSRGAN", "model.py")), reason="reference tree not present")]
+CRITICS = "reference" if os.path.isfile(os.path.join(REF, "BSRGAN", "model.py")) else "torch"
+pytestmark = pytest.mark.gpu
 
 
 def test_generator_gradients_inside_the_gan_step():
     sys.path.insert(0, os.path.join(ROOT, "tools"))
     import gan_step
     dev = torch.device("cuda", 0)
-    d_model, g_model, content = gan_step.build("b200", dev, seed=0)
+    d_model, g_model, content = gan_step.build("b200", dev, seed=0, content=CRITICS, disc=CRITICS)
     d_model.train(); g_model.train()
     params = {k: v.detach().cpu().clone() for k, v in g_model.state_dict().items()}
     params = orc.in_range_fixture(params)

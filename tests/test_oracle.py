@@ -8,10 +8,20 @@ import pytest
 import torch
 import torch.nn.functional as F
 
+from oracle import make_golden
 from oracle import reference_loader as rl
 from oracle import rrdbnet_oracle as orc
 
 GOLDEN = sorted(glob.glob(os.path.join(os.path.dirname(__file__), "golden", "*.pt")))
+
+
+@pytest.fixture
+def golden_threads():
+    """the thread count the fixtures were computed with (bit equality depends on it), whatever the host or an earlier test set"""
+    n = torch.get_num_threads()
+    torch.set_num_threads(make_golden.THREADS)
+    yield
+    torch.set_num_threads(n)
 
 
 def _drop_in(fix):
@@ -29,6 +39,7 @@ def _drop_in(fix):
     return net, params
 
 
+@pytest.mark.usefixtures("golden_threads")
 @pytest.mark.parametrize("path", GOLDEN, ids=[os.path.basename(p) for p in GOLDEN])
 def test_oracle_matches_golden(path):
     """seed + drop-in constructor reproduces the reference weights; oracle forward/backward reproduce the reference
