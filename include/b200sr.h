@@ -204,6 +204,12 @@ void b200sr_debug_set(int flags);
 /* bit 6 (64) of the debug flags makes the chain kernel record, per CTA, the cycles each warp role waited on each barrier
  * kind (12 counters per CTA, see conv_kernel.cuh); this copies the first n counters of the last launch to the host. */
 int b200sr_debug_read_profile(unsigned long long* out_host, int n);
+/* byte offset and size of a named workspace tensor of a plan (test / debugging use); B200SR_ERR_INVALID for a name the plan
+ * does not have.  Discriminator plans name every tensor they keep: the ingested input "xin", the forward activations
+ * "T0u" "T1u" "T2u" "T3" "B1" "A1" "B2" "A2" "B3" "A3" "S3" "A4" "A5" and, in training plans, the backward gradients "DYP" "G5"
+ * "G4" "GS3" "G3" "GB3" "GS2" "GA2" "GB2" "GS1" "GA1" "GB1" "GT3" "GT2" "GT1" "G0" (build_disc_plan in b200sr.cu says what each
+ * holds); generator and VGG plans name none. */
+int b200sr_debug_buffer(const b200sr_plan* plan, const char* name, int64_t* offset_bytes, int64_t* bytes);
 
 #ifdef __cplusplus
 }

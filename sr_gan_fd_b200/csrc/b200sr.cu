@@ -194,6 +194,8 @@ struct b200sr_plan {
   std::vector<long long> gw_off;      // float offsets per conv into the staging buffer
   std::vector<UnpackOp> unpack_ops;   // one per conv, conv order
   UnpackOp* d_unpack_ops = nullptr;
+  struct NamedBuf { std::string name; long long off, bytes; };
+  std::vector<NamedBuf> named_bufs;   // workspace tensors by name (b200sr_debug_buffer)
   // device-side tables + descriptor cache
   PackOp* d_pack_ops = nullptr;
   BiasOp* d_bias_ops = nullptr;
@@ -235,6 +237,12 @@ struct Builder {
   long long alloc(long long bytes) {
     long long o = cursor;
     cursor = align_up(cursor + bytes, 1024);
+    return o;
+  }
+  // the same, and the tensor can be looked up by name (b200sr_debug_buffer)
+  long long alloc(const char* name, long long bytes) {
+    const long long o = alloc(bytes);
+    P.named_bufs.push_back({name, o, bytes});
     return o;
   }
   int add_map(long long off, int c_valid, int c_pix, int n, int h, int w, int box_rows, int box_w = -1) {
@@ -1689,20 +1697,26 @@ static int build_disc_plan(b200sr_plan& P) {
   auto npx = [&](int lvl) { return (long long)N * lh(lvl) * lw(lvl); };
   Builder B(P);
   P.xin_stride = 64;
-  P.o_xin = B.alloc(npx(0) * 64 * 2);
+  P.o_xin = B.alloc("xin", npx(0) * 64 * 2);
   // forward activations (all kept: the backward pass reads every one of them)
-  const long long T0u = B.alloc(npx(0) * 64 * 2), T1u = B.alloc(npx(1) * 128 * 2), T2u = B.alloc(npx(2) * 256 * 2), T3 = B.alloc(npx(3) * 512 * 2);
-  const long long B1 = B.alloc(npx(2) * 512 * 2), A1 = B.alloc(npx(2) * 256 * 2), B2 = B.alloc(npx(1) * 256 * 2), A2 = B.alloc(npx(1) * 128 * 2);
-  const long long B3 = B.alloc(npx(0) * 128 * 2), A3 = B.alloc(npx(0) * 64 * 2), S3 = B.alloc(npx(0) * 64 * 2), A4 = B.alloc(npx(0) * 64 * 2), A5 = B.alloc(npx(0) * 64 * 2);
+  const long long T0u = B.alloc("T0u", npx(0) * 64 * 2), T1u = B.alloc("T1u", npx(1) * 128 * 2), T2u = B.alloc("T2u", npx(2) * 256 * 2),
+                  T3 = B.alloc("T3", npx(3) * 512 * 2);
+  const long long B1 = B.alloc("B1", npx(2) * 512 * 2), A1 = B.alloc("A1", npx(2) * 256 * 2), B2 = B.alloc("B2", npx(1) * 256 * 2),
+                  A2 = B.alloc("A2", npx(1) * 128 * 2);
+  const long long B3 = B.alloc("B3", npx(0) * 128 * 2), A3 = B.alloc("A3", npx(0) * 64 * 2), S3 = B.alloc("S3", npx(0) * 64 * 2),
+                  A4 = B.alloc("A4", npx(0) * 64 * 2), A5 = B.alloc("A5", npx(0) * 64 * 2);
   long long DYP = 0, G5 = 0, G4 = 0, GS3 = 0, G3 = 0, GB3 = 0, GS2 = 0, GA2 = 0, GB2 = 0, GS1 = 0, GA1 = 0, GB1 = 0, GT3 = 0, GT2 = 0, GT1 = 0, G0 = 0;
   // effective (as computed) input channels / staged output channels of every conv's weight gradient
   int eI[10], coPad[10];
   for (int c = 0; c < nconv; ++c) { eI[c] = (cK[c] == 4) ? 4 * cI[c] : cI[c]; coPad[c] = (int)align_up(cO[c], 4); }
   if (train) {
-    DYP = B.alloc(npx(0) * 64 * 2); G5 = B.alloc(npx(0) * 64 * 2); G4 = B.alloc(npx(0) * 64 * 2); GS3 = B.alloc(npx(0) * 64 * 2); G3 = B.alloc(npx(0) * 64 * 2);
-    GB3 = B.alloc(npx(0) * 128 * 2); GS2 = B.alloc(npx(1) * 128 * 2); GA2 = B.alloc(npx(1) * 128 * 2); GB2 = B.alloc(npx(1) * 256 * 2);
-    GS1 = B.alloc(npx(2) * 256 * 2); GA1 = B.alloc(npx(2) * 256 * 2); GB1 = B.alloc(npx(2) * 512 * 2); GT3 = B.alloc(npx(3) * 512 * 2);
-    GT2 = B.alloc(npx(2) * 256 * 2); GT1 = B.alloc(npx(1) * 128 * 2); G0 = B.alloc(npx(0) * 64 * 2);
+    DYP = B.alloc("DYP", npx(0) * 64 * 2); G5 = B.alloc("G5", npx(0) * 64 * 2); G4 = B.alloc("G4", npx(0) * 64 * 2);
+    GS3 = B.alloc("GS3", npx(0) * 64 * 2); G3 = B.alloc("G3", npx(0) * 64 * 2);
+    GB3 = B.alloc("GB3", npx(0) * 128 * 2); GS2 = B.alloc("GS2", npx(1) * 128 * 2); GA2 = B.alloc("GA2", npx(1) * 128 * 2);
+    GB2 = B.alloc("GB2", npx(1) * 256 * 2);
+    GS1 = B.alloc("GS1", npx(2) * 256 * 2); GA1 = B.alloc("GA1", npx(2) * 256 * 2); GB1 = B.alloc("GB1", npx(2) * 512 * 2);
+    GT3 = B.alloc("GT3", npx(3) * 512 * 2);
+    GT2 = B.alloc("GT2", npx(2) * 256 * 2); GT1 = B.alloc("GT1", npx(1) * 128 * 2); G0 = B.alloc("G0", npx(0) * 64 * 2);
     long long off = 0;
     int blocks = 0;
     P.gw_off.assign(nconv, 0);
@@ -1958,6 +1972,13 @@ void b200sr_debug_set(int flags) { g_debug = flags; }
 int b200sr_debug_read_profile(unsigned long long* out_host, int n) {
   CUDA_TRY(cudaMemcpyFromSymbol(out_host, g_conv_prof, sizeof(unsigned long long) * (size_t)n));
   return 0;
+}
+int b200sr_debug_buffer(const b200sr_plan* p, const char* name, int64_t* offset_bytes, int64_t* bytes) {
+  if (!p || !name || !offset_bytes || !bytes) return fail(B200SR_ERR_INVALID, "null argument");
+  for (const b200sr_plan::NamedBuf& nb : p->named_bufs) {
+    if (nb.name == name) { *offset_bytes = nb.off; *bytes = nb.bytes; return 0; }
+  }
+  return fail(B200SR_ERR_INVALID, "the plan has no workspace tensor named '%s'", name);
 }
 
 int b200sr_plan_create(const b200sr_net_desc* desc, b200sr_plan** out) {

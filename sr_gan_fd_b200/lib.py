@@ -71,6 +71,7 @@ SIGNATURES = {
     "b200sr_version": (C.c_int, []),
     "b200sr_debug_set": (None, [C.c_int]),
     "b200sr_debug_read_profile": (C.c_int, [C.c_void_p, C.c_int]),
+    "b200sr_debug_buffer": (C.c_int, [C.c_void_p, C.c_char_p, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
 }
 
 

@@ -222,11 +222,11 @@ def _settle_power_iteration(module, x, iters=5):
     return module
 
 
-def _record(tag, payload):
+def _record(tag, payload, fname="disc_parity.jsonl"):
     out = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "gpurun_out")
     if os.path.isdir(out):
         import json
-        with open(os.path.join(out, "disc_parity.jsonl"), "a") as fh:
+        with open(os.path.join(out, fname), "a") as fh:
             fh.write(json.dumps({"case": tag, **payload}) + "\n")
 
 
