@@ -138,7 +138,7 @@ struct Step {
   int xmap = -1, dymap = -1;
   WgradBatch wb;
   Ref seg_out[5];                 // bias-grad kernel outputs
-  Ref wseg_out[kWgMaxProblems][5];  // wgrad batch outputs
+  Ref wseg_out[kWgMaxProblems][kWgMaxSeg];  // wgrad batch outputs
   // bias grad
   BiasGradParams bp;
   Ref bg_g;
@@ -636,15 +636,23 @@ static int build_plan(b200sr_plan& P) {
     };
     auto add_problem = [&](Step& s, int a_c0, int b_c0, int n_cols, int bias_mode, int a_blocks = 2) {
       WgradParams& wp = s.wb.prob[s.wb.num_problems++];
-      wp.a_c0 = a_c0; wp.b_c0 = b_c0; wp.n_cols = n_cols; wp.n_blocks = (n_cols + 63) / 64; wp.bias_mode = bias_mode;
-      wp.a_blocks = a_blocks;
+      wp.b_c0 = b_c0; wp.n_cols = n_cols; wp.n_blocks = (n_cols + 63) / 64; wp.bias_mode = bias_mode;
+      wgrad_set_a(wp, a_c0, a_blocks);
       return s.wb.num_problems - 1;
     };
-    auto add_seg = [&](Step& s, int cb, int ce, Ref out, int ci_total, int ci0, int co_pad) {  // to the LAST problem added
+    // packed problem: M block 0 = X channels [c0, c0 + 64) at tap dx0, block 1 = the same channels at tap dx1 (>= 0) or all ones (-1)
+    auto add_packed = [&](Step& s, int c0, int dx0, int dx1, int b_c0, int n_cols) {
+      WgradParams& wp = s.wb.prob[s.wb.num_problems++];
+      wp.b_c0 = b_c0; wp.n_cols = n_cols; wp.n_blocks = (n_cols + 63) / 64; wp.bias_mode = 0;
+      wp.blk[0].kind = kWgBlkX; wp.blk[0].c0 = c0; wp.blk[0].dx = dx0;
+      wp.blk[1].kind = dx1 >= 0 ? kWgBlkX : kWgBlkOnes; wp.blk[1].c0 = c0; wp.blk[1].dx = dx1 >= 0 ? dx1 : 0;
+      return s.wb.num_problems - 1;
+    };
+    auto add_seg = [&](Step& s, int cb, int ce, Ref out, int ci_total, int ci0, int co_pad, int blk_mask = 0) {  // to the LAST problem added
       const int pj = s.wb.num_problems - 1;
       WgradParams& wp = s.wb.prob[pj];
       WgradSegment& g = wp.seg[wp.num_seg];
-      g.col_begin = cb; g.col_end = ce; g.out = nullptr; g.ci_total = ci_total; g.ci0 = ci0; g.co_pad = co_pad;
+      g.col_begin = cb; g.col_end = ce; g.out = nullptr; g.ci_total = ci_total; g.ci0 = ci0; g.co_pad = co_pad; g.blk_mask = blk_mask;
       s.wseg_out[pj][wp.num_seg] = out;
       wp.num_seg++;
     };
@@ -872,7 +880,37 @@ static int build_plan(b200sr_plan& P) {
         emit(s);
       }
       // weight gradients of the five convs, re-associated by input slice
-      {
+      static const bool wgrad_pack = [] { const char* e = getenv("B200SR_WGRAD_PACK"); return e ? atoi(e) != 0 : true; }();
+      if (wgrad_pack) {
+        // ONE launch per dense block, five problems, no idle accumulator rows: the 64-channel slices (x for conv1, o3|o4 for
+        // conv4 / conv5) put two horizontal taps into one CTA's M = 128, and the third tap shares its CTA with an all-ones block
+        // whose column sums are the bias gradients of all five convs.  Per 128-pixel tile: 7 CTA-units of (M = 128) x N x 24
+        // MMAs (3 x 160 + 160 + 96 + 32 + 32 = 800 columns) where the unpacked list below has 9 + 1/3 (928 columns).
+        const int c5 = conv_index_rdb(r, 5), c4 = conv_index_rdb(r, 4), c3 = conv_index_rdb(r, 3), c2 = conv_index_rdb(r, 2),
+                  c1 = conv_index_rdb(r, 1);
+        Step wg = wgrad_batch(D, 192, 192, DYc, 192, 192, N, H, W);
+        add_problem(wg, 0, 0, 160, 0);          // x, o1, o2 rows at the CTA's tap x [dY5|dY4|dY3|dY2]
+        add_seg(wg, 0, 64, wref(c5), 192, 0, 64);
+        add_seg(wg, 64, 96, wref(c4), 160, 0, 32);
+        add_seg(wg, 96, 128, wref(c3), 128, 0, 32);
+        add_seg(wg, 128, 160, wref(c2), 96, 0, 32);
+        add_packed(wg, 128, 2, -1, 0, 160);     // (o3|o4 at dx 2 | ones) x [dY5|dY4|dY3|dY2]
+        add_seg(wg, 0, 64, wref(c5), 192, 128, 64, 1);
+        add_seg(wg, 64, 96, wref(c4), 160, 128, 32, 1);
+        add_seg(wg, 0, 64, bref(c5), 1, 0, 64, 2);
+        add_seg(wg, 64, 96, bref(c4), 1, 0, 32, 2);
+        add_seg(wg, 96, 128, bref(c3), 1, 0, 32, 2);
+        add_seg(wg, 128, 160, bref(c2), 1, 0, 32, 2);
+        add_packed(wg, 128, 0, 1, 0, 96);       // (o3|o4 at dx 0 | o3|o4 at dx 1) x [dY5|dY4]
+        add_seg(wg, 0, 64, wref(c5), 192, 128, 64);
+        add_seg(wg, 64, 96, wref(c4), 160, 128, 32);
+        add_packed(wg, 0, 0, 1, 160, 32);       // (x at dx 0 | x at dx 1) x dY1
+        add_seg(wg, 0, 32, wref(c1), 64, 0, 32);
+        add_packed(wg, 0, 2, -1, 160, 32);      // (x at dx 2 | ones) x dY1
+        add_seg(wg, 0, 32, wref(c1), 64, 0, 32, 1);
+        add_seg(wg, 0, 32, bref(c1), 1, 0, 32, 2);
+        emit(wg);
+      } else {
         // ONE launch per dense block: three channel-block problems + the bias gradients (all-ones A operand)
         Step wg = wgrad_batch(D, 192, 192, DYc, 192, 192, N, H, W);
         add_problem(wg, 0, 0, 160, 0);   // x, o1, o2 rows x [dY5|dY4|dY3|dY2]
@@ -892,15 +930,15 @@ static int build_plan(b200sr_plan& P) {
         add_seg(wg, 128, 160, bref(conv_index_rdb(r, 2)), 1, 0, 32);
         add_seg(wg, 160, 192, bref(conv_index_rdb(r, 1)), 1, 0, 32);
         emit(wg);
-        if (j == 0) {
-          // gradient buckets: G RRDBs each (their convs are contiguous in the flat buffer); the LAST trunk bucket is at most two
-          // RRDBs so that little communication is left after the final kernels
-          const int blk = r / 3;
-          const int G = d.grad_bucket_rrdbs > 0 ? d.grad_bucket_rrdbs : 1;
-          if (blk % G == 0 || (G > 2 && blk == 2)) {
-            emit(unpack_step(conv_index_rdb(r, 1), bucket_hi));
-            bucket_hi = conv_index_rdb(r, 1);
-          }
+      }
+      if (j == 0) {
+        // gradient buckets: G RRDBs each (their convs are contiguous in the flat buffer); the LAST trunk bucket is at most two
+        // RRDBs so that little communication is left after the final kernels
+        const int blk = r / 3;
+        const int G = d.grad_bucket_rrdbs > 0 ? d.grad_bucket_rrdbs : 1;
+        if (blk % G == 0 || (G > 2 && blk == 2)) {
+          emit(unpack_step(conv_index_rdb(r, 1), bucket_hi));
+          bucket_hi = conv_index_rdb(r, 1);
         }
       }
     }
@@ -1222,15 +1260,14 @@ static int launch_wgrad(const Step& s, const CUtensorMap& tmX, const CUtensorMap
     for (int i = 0; i < wp.num_seg; ++i) wp.seg[i].out = (float*)resolve(s.wseg_out[j][i], b);
     const int nacc = wp.bias_mode ? 1 : (wp.dy_mask ? __builtin_popcount(wp.dy_mask) : 3);
     const double mma = nacc * 8.0 * (wp.n_cols / 2.0);
-    const double ld = wgrad_stage_bytes(wp) / 42.0;
-    const int ntx = wp.bias_mode ? 1 : (wp.dx_mask ? __builtin_popcount(wp.dx_mask) : 3);
-    work[j] = (mma > ld ? mma : ld) * ntx;
+    const double ld = wgrad_load_bytes(wp) / 42.0;
+    work[j] = (mma > ld ? mma : ld) * wgrad_ntap(wp);
     total += work[j];
   }
   int ctas = 0;
   for (int j = 0; j < wb.num_problems; ++j) {
     WgradParams& wp = wb.prob[j];
-    const int ntap = wp.bias_mode ? 1 : (wp.dx_mask ? __builtin_popcount(wp.dx_mask) : 3);
+    const int ntap = wgrad_ntap(wp);
     int splits = (int)(sms * work[j] / total / ntap + 0.5);
     if (splits < 1) splits = 1;
     if (splits > wb.num_tiles) splits = wb.num_tiles;
@@ -1886,8 +1923,8 @@ static int build_disc_plan(b200sr_plan& P) {
           const int ncols = std::min(128, ncols_all - cob);
           const int pj = cur.wb.num_problems++;
           WgradParams& wp = cur.wb.prob[pj];
-          wp.a_c0 = cib; wp.b_c0 = cob; wp.n_cols = ncols; wp.n_blocks = (ncols + 63) / 64; wp.bias_mode = 0;
-          wp.a_blocks = (x_cvalid - cib > 64) ? 2 : 1;
+          wp.b_c0 = cob; wp.n_cols = ncols; wp.n_blocks = (ncols + 63) / 64; wp.bias_mode = 0;
+          wgrad_set_a(wp, cib, (x_cvalid - cib > 64) ? 2 : 1);
           WgradSegment& g = wp.seg[0];
           g.col_begin = 0; g.col_end = ncols; g.out = nullptr; g.ci_total = ci_total; g.ci0 = cib; g.co_pad = coPad[c];
           if (cK[c] == 4 && g_down4) {
@@ -1901,7 +1938,7 @@ static int build_disc_plan(b200sr_plan& P) {
           }
           cur.wseg_out[pj][0] = wref(c, (long long)(cob / 4) * ci_total * 4);
           wp.num_seg = 1;
-          if (cur.wb.num_problems == kWgMaxProblems) { P.bwd.push_back(cur); open = false; }
+          if (cur.wb.num_problems == 4) { P.bwd.push_back(cur); open = false; }
         }
       }
       if (open) P.bwd.push_back(cur);
@@ -2244,7 +2281,7 @@ int b200sr_conv3x3_wgrad(const void* x, int n, int h, int w_, int cin, int x_str
   wb.tiles_x = (w_ + kTileW - 1) / kTileW; wb.tiles_y = (h + kWgTileH - 1) / kWgTileH; wb.num_tiles = n * wb.tiles_x * wb.tiles_y;
   wb.num_problems = 1;
   WgradParams& wp = wb.prob[0];
-  wp.a_c0 = 0; wp.b_c0 = 0; wp.n_cols = cout; wp.n_blocks = (cout + 63) / 64; wp.a_blocks = (cin > 64) ? 2 : 1;
+  wp.b_c0 = 0; wp.n_cols = cout; wp.n_blocks = (cout + 63) / 64; wgrad_set_a(wp, 0, (cin > 64) ? 2 : 1);
   wp.num_seg = 1;
   wp.seg[0].col_begin = 0; wp.seg[0].col_end = cout; wp.seg[0].out = staging; wp.seg[0].ci_total = cin; wp.seg[0].ci0 = 0; wp.seg[0].co_pad = cout;
   int splits = g_num_sms / 3;

@@ -12,10 +12,15 @@
 // pixel loop and are flushed once with 16-byte vector reductions (red.global.add.v4.f32) into a [tap][co/4][ci][4]
 // fp32 staging tensor; a small unpack kernel transposes that to the OIHW gradient layout per gradient bucket.
 //
-// One launch carries a BATCH of up to four such problems over the same two tensor maps (the three channel-block
-// problems of a dense block + its bias gradients), with the CTAs dealt out in proportion to each problem's cost so
-// the whole dense block is one balanced wave.  The bias gradient is the same GEMM with an all-ones A operand
-// (column sums of dY), so it rides the same pipeline and flush.
+// One launch carries a BATCH of up to five such problems over the same two tensor maps (the channel-block problems of a
+// dense block + its bias gradients), with the CTAs dealt out in proportion to each problem's cost so the whole dense
+// block is one balanced wave.  The bias gradient is the same GEMM with an all-ones A operand (column sums of dY), so it
+// rides the same pipeline and flush.
+//
+// The two 64-row M blocks of a problem are described independently (WgradMBlock): each is X channels [c0, c0 + 64) at
+// its own horizontal tap, an all-ones block, or idle.  A CTA that needs only 64 input channels therefore fills its
+// other half with useful rows -- the same channels at another tap, or ones whose products are the bias gradients --
+// instead of multiplying rows that are never flushed (every tcgen05 MMA costs the same for M = 64 real rows as for 128).
 #pragma once
 #include "conv_kernel.cuh"
 
@@ -29,8 +34,8 @@ constexpr int kWgXRows = kWgTileH + 2;
 constexpr int kWgXBytes = kWgXRows * kTileW * 128;   // 18432 B per 64-channel haloed X tile
 constexpr int kWgBBytes = kWgTileH * kTileW * 128;   // 16384 B per 64-channel dY tile
 constexpr int kWgThreads = 192;
-constexpr int kWgMaxSeg = 5;
-constexpr int kWgMaxProblems = 4;
+constexpr int kWgMaxSeg = 6;
+constexpr int kWgMaxProblems = 5;
 constexpr int kWgOnesBytes = 4096;  // two 64-channel M blocks x 16 pixels x 128 B of bf16 1.0 (A operand of the bias-gradient problem)
 
 struct WgradSegment {
@@ -40,16 +45,28 @@ struct WgradSegment {
   int ci_total;            // input channels of that conv
   int ci0;                 // conv input channel of accumulator row 0
   int co_pad;              // output channels rounded up to a multiple of 4
+  int blk_mask;            // M blocks whose rows this segment flushes (bit b = block b; 0 = both)
+};
+
+enum : int { kWgBlkIdle = 0, kWgBlkX = 1, kWgBlkOnes = 2 };
+// One 64-row half of the UMMA's M = 128, at stage offset b * kWgXBytes (the A descriptor's LBO).
+//   kWgBlkX:    haloed X tile of channels [c0, c0 + 64) at horizontal tap dx; rows map to (tap, channel) in the flush.
+//   kWgBlkOnes: bf16 1.0 (written once per ring stage, never loaded): every row and every vertical-tap accumulator holds the column
+//               sums of dY, so ONE row of ONE accumulator is flushed -- the bias gradients of the problem's columns.
+//   kWgBlkIdle: block 1 only: nothing loaded (the MMA reads whatever follows in the stage, finite data), nothing flushed.
+struct WgradMBlock {
+  int kind;
+  int c0;
+  int dx;  // 0..2, or -1: the CTA's own tap (the problem's dx_mask deals one tap per CTA).  Either both X blocks use -1 or neither.
 };
 
 struct WgradParams {
-  int a_c0;      // first X channel (accumulator row 0); two 64-channel boxes are loaded
+  WgradMBlock blk[2];
   int b_c0;      // first dY channel (accumulator column 0)
   int n_cols;    // UMMA N (multiple of 16, <= 160; bias problem: <= 256)
   int n_blocks;  // ceil(n_cols / 64) dY boxes per tile
-  int a_blocks;  // X boxes loaded per tile: 2 (128 input channels) or 1 (only accumulator rows 0..63 are kept)
-  int bias_mode; // 1: A = all ones, one accumulator, no X loads, no taps: column sums of dY
-  int splits;    // pixel-tile splits of this problem (CTAs = splits * taps_x, taps_x = 1 in bias mode, else popcount(dx_mask))
+  int bias_mode; // 1: A = all ones, one accumulator, no X loads, no taps: column sums of dY (blk[] unused)
+  int splits;    // pixel-tile splits of this problem (CTAs = splits * wgrad_ntap)
   int num_seg;
   int dx_mask, dy_mask;  // horizontal taps that get a CTA / vertical taps that get an accumulator (0 = all three).  The 4x4 stride-2
                          // convs of the U-Net discriminator, computed as 3x3 convs over the pixel-unshuffled input, only have a
@@ -66,8 +83,23 @@ struct WgradBatch {
   WgradParams prob[kWgMaxProblems];
 };
 
+// ring-stage footprint (an all-ones block keeps its slot) and the bytes TMA brings in per stage
 __host__ __device__ inline int wgrad_stage_bytes(const WgradParams& p) {
-  return (p.bias_mode ? 0 : p.a_blocks * kWgXBytes) + p.n_blocks * kWgBBytes;
+  return (p.bias_mode ? 0 : (p.blk[1].kind == kWgBlkIdle ? 1 : 2) * kWgXBytes) + p.n_blocks * kWgBBytes;
+}
+__host__ __device__ inline int wgrad_load_bytes(const WgradParams& p) {
+  return (p.bias_mode ? 0 : ((p.blk[0].kind == kWgBlkX) + (p.blk[1].kind == kWgBlkX)) * kWgXBytes) + p.n_blocks * kWgBBytes;
+}
+// CTAs per pixel split: one per horizontal tap of dx_mask when the X blocks follow the CTA's tap, else one
+__host__ __device__ inline int wgrad_ntap(const WgradParams& p) {
+  if (p.bias_mode || p.blk[0].dx >= 0) return 1;
+  const int m = p.dx_mask ? p.dx_mask : 7;
+  return (m & 1) + ((m >> 1) & 1) + ((m >> 2) & 1);
+}
+// legacy A operand: X channels [a_c0, a_c0 + 64 * a_blocks) at the CTA's tap (a_blocks = 1: block 1 idle)
+__host__ inline void wgrad_set_a(WgradParams& p, int a_c0, int a_blocks) {
+  p.blk[0].kind = kWgBlkX; p.blk[0].c0 = a_c0; p.blk[0].dx = -1;
+  p.blk[1].kind = a_blocks == 2 ? kWgBlkX : kWgBlkIdle; p.blk[1].c0 = a_c0 + 64; p.blk[1].dx = -1;
 }
 constexpr int kWgSmemBytes = 227 * 1024;
 
@@ -92,19 +124,20 @@ wgrad3x3_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
   const WgradParams& p = batch.prob[pj];
   const int local = blockIdx.x - batch.cta_begin[pj];
   const int dxm = p.dx_mask ? p.dx_mask : 7, dym = p.dy_mask ? p.dy_mask : 7;
-  const int ntap = p.bias_mode ? 1 : __popc(dxm);
+  const int ntap = wgrad_ntap(p);
   int dxi = 1;  // horizontal tap owned by this CTA: the (local % ntap)-th set bit of the mask
-  if (!p.bias_mode) {
+  if (!p.bias_mode && p.blk[0].dx < 0) {
     int k = local % ntap;
     dxi = 0;
     while (!((dxm >> dxi) & 1) || k-- > 0) ++dxi;
   }
   const int split = local / ntap;
-  const int nacc = p.bias_mode ? 1 : 3;
   const int stage_bytes = wgrad_stage_bytes(p);
   int S = kRing / stage_bytes;
   if (S > 4) S = 4;
-  const int b_off = p.bias_mode ? 0 : p.a_blocks * kWgXBytes;
+  const int b_off = stage_bytes - p.n_blocks * kWgBBytes;
+  const int bdx0 = p.blk[0].dx >= 0 ? p.blk[0].dx : dxi, bdx1 = p.blk[1].dx >= 0 ? p.blk[1].dx : dxi;
+  const bool ones_blk = !p.bias_mode && p.blk[1].kind == kWgBlkOnes;
 
   if (warp == 0 && lane == 0) {
     prefetch_tensormap(&tmX);
@@ -119,6 +152,15 @@ wgrad3x3_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
   if (warp == 1) tmem_alloc_imm<512>(tmem_slot);
   if (p.bias_mode) {
     for (int i = threadIdx.x; i < kWgOnesBytes / 4; i += kWgThreads) reinterpret_cast<uint32_t*>(ones)[i] = batch.a_f16 ? 0x3C003C00u : 0x3F803F80u;  // 1.0 x2
+    fence_proxy_async_smem();
+  } else if (ones_blk) {
+    // all-ones M block 1: its slot of every ring stage, written once (the producer never loads into it)
+    constexpr int kVec = kWgXBytes / 16;
+    const uint32_t one2 = batch.a_f16 ? 0x3C003C00u : 0x3F803F80u;
+    for (int i = threadIdx.x; i < S * kVec; i += kWgThreads) {
+      const int s = i / kVec;
+      *reinterpret_cast<uint4*>(smem + s * stage_bytes + kWgXBytes + (i - s * kVec) * 16) = make_uint4(one2, one2, one2, one2);
+    }
     fence_proxy_async_smem();
   }
   tcgen05_fence_before();
@@ -140,12 +182,10 @@ wgrad3x3_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
       mbar_wait(&empty[s], ph ^ 1);
       if (elect_one_sync()) {
         uint8_t* st = smem + s * stage_bytes;
-        mbar_arrive_expect_tx(&full[s], stage_bytes);
+        mbar_arrive_expect_tx(&full[s], wgrad_load_bytes(p));
         if (!p.bias_mode) {
-          tma_load_4d(st, &tmX, &full[s], p.a_c0, x0 + dxi - 1, y0 - 1, n);
-          // with one X box the MMA's rows 64..127 read whatever follows in the stage (finite bf16 data); those accumulator
-          // rows are never flushed
-          if (p.a_blocks == 2) tma_load_4d(st + kWgXBytes, &tmX, &full[s], p.a_c0 + 64, x0 + dxi - 1, y0 - 1, n);
+          if (p.blk[0].kind == kWgBlkX) tma_load_4d(st, &tmX, &full[s], p.blk[0].c0, x0 + bdx0 - 1, y0 - 1, n);
+          if (p.blk[1].kind == kWgBlkX) tma_load_4d(st + kWgXBytes, &tmX, &full[s], p.blk[1].c0, x0 + bdx1 - 1, y0 - 1, n);
         }
         for (int j = 0; j < p.n_blocks; ++j)
           tma_load_4d(st + b_off + j * kWgBBytes, &tmDY, &full[s], p.b_c0 + 64 * j, x0, y0, n);
@@ -188,25 +228,31 @@ wgrad3x3_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
     }
     if (elect_one_sync()) umma_commit(done);
     __syncwarp();
-  } else if (has_work) {
-    // epilogue: flush the accumulators with 16-byte fp32 vector reductions into [tap][ci][co] staging tensors
+  } else if (has_work && (p.bias_mode || p.blk[(warp & 3) >> 1].kind != kWgBlkIdle)) {
+    // epilogue: flush the accumulators with 16-byte fp32 vector reductions into [tap][ci][co] staging tensors.  Warps 2 + q
+    // hold accumulator rows 32q .. 32q + 31: rows 0..63 are M block 0, rows 64..127 block 1.
     const int q = warp & 3;
-    const int m = q * 32 + lane;  // accumulator row = input channel a_c0 + m
+    const int b = q >> 1;
+    const bool ones = p.bias_mode || p.blk[b].kind == kWgBlkOnes;
+    // conv input channel = sg.ci0 + m: m counts X channels from block 0's first one (bias mode / ones block: row 0 of the block)
+    const int m = p.bias_mode ? q * 32 + lane : (ones ? 0 : p.blk[b].c0 - p.blk[0].c0) + (q & 1) * 32 + lane;
+    const int bdx = b ? bdx1 : bdx0;
+    const int nacc = ones ? 1 : 3;  // the vertical-tap accumulators of a ones block all hold the same column sums
     mbar_wait(done, 0);
     tcgen05_fence_after();
     for (int dyi = 0; dyi < nacc; ++dyi) {
-      if (!p.bias_mode && !((dym >> dyi) & 1)) continue;
-      const int tap = p.bias_mode ? 0 : dyi * 3 + dxi;
+      if (!ones && !((dym >> dyi) & 1)) continue;
+      const int tap = ones ? 0 : dyi * 3 + bdx;
       for (int c0 = 0; c0 < p.n_cols; c0 += 16) {
         uint32_t r[16];
         tmem_ld_32x32b_x16(tmem_base + (static_cast<uint32_t>(q * 32) << 16) + dyi * p.n_cols + c0, r);
         tmem_ld_wait();
         int sgi = 0;
-        while (sgi < p.num_seg - 1 && c0 >= p.seg[sgi].col_end) ++sgi;
+        while (sgi < p.num_seg - 1 && (c0 >= p.seg[sgi].col_end || (p.seg[sgi].blk_mask && !((p.seg[sgi].blk_mask >> b) & 1)))) ++sgi;
         const WgradSegment& sg = p.seg[sgi];
         const int co = c0 - sg.col_begin;
         const int ci = sg.ci0 + m;
-        if (c0 >= sg.col_begin && c0 < sg.col_end && ci < sg.ci_total) {
+        if (c0 >= sg.col_begin && c0 < sg.col_end && ci < sg.ci_total && (!sg.blk_mask || ((sg.blk_mask >> b) & 1))) {
           float* dst = sg.out + ((static_cast<long long>(tap) * (sg.co_pad >> 2) + (co >> 2)) * sg.ci_total + ci) * 4;
 #pragma unroll
           for (int j = 0; j < 4; ++j)
