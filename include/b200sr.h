@@ -208,7 +208,10 @@ int b200sr_debug_read_profile(unsigned long long* out_host, int n);
  * does not have.  Discriminator plans name every tensor they keep: the ingested input "xin", the forward activations
  * "T0u" "T1u" "T2u" "T3" "B1" "A1" "B2" "A2" "B3" "A3" "S3" "A4" "A5" and, in training plans, the backward gradients "DYP" "G5"
  * "G4" "GS3" "G3" "GB3" "GS2" "GA2" "GB2" "GS1" "GA1" "GB1" "GT3" "GT2" "GT1" "G0" (build_disc_plan in b200sr.cu says what each
- * holds); generator and VGG plans name none. */
+ * holds).  Generator plans name theirs too (build_plan in b200sr.cu): "xin", the fp32 carriers "T0" "TR" "C1" "C2" (tile-blocked),
+ * the dense-block buffers "D0" ... "D{R-1}" (R = 3 * num_blocks; inference plans keep only the ping-pong pair "D0" "D1"), the
+ * tail activations "SPLT" "SPL0" ... "SPL{n_up}" "SPLC" and, in training plans, "CMASK" "DYP" "G3" "GU1" ... "GU{n_up}" "GT" "GTB"
+ * "GR" "GC1" "GC2" "GO1" "DYB0" ... "DYB{R-1}".  VGG plans name none. */
 int b200sr_debug_buffer(const b200sr_plan* plan, const char* name, int64_t* offset_bytes, int64_t* bytes);
 
 #ifdef __cplusplus

@@ -240,7 +240,7 @@ struct Builder {
     return o;
   }
   // the same, and the tensor can be looked up by name (b200sr_debug_buffer)
-  long long alloc(const char* name, long long bytes) {
+  long long alloc(const std::string& name, long long bytes) {
     const long long o = alloc(bytes);
     P.named_bufs.push_back({name, o, bytes});
     return o;
@@ -377,30 +377,30 @@ static int build_plan(b200sr_plan& P) {
   Builder B(P);
   P.xin_stride = (int)align_up(3 * d.in_channels, 64);
   // ---- workspace layout
-  P.o_xin = B.alloc(Ppix * P.xin_stride * 2);
+  P.o_xin = B.alloc("xin", Ppix * P.xin_stride * 2);
   // fp32 carriers: tile-blocked layout over the LR lattice's 8 x 32 tiles (padded to whole tiles)
   const long long carrier_bytes = (long long)N * ((W + kTileW - 1) / kTileW) * ((H + kTileH - 1) / kTileH) * kCarrierBytesPerTile;
-  P.o_t0 = B.alloc(carrier_bytes);
-  P.o_tr = B.alloc(carrier_bytes);
-  P.o_c1 = B.alloc(carrier_bytes);
-  P.o_c2 = B.alloc(carrier_bytes);
+  P.o_t0 = B.alloc("T0", carrier_bytes);
+  P.o_tr = B.alloc("TR", carrier_bytes);
+  P.o_c1 = B.alloc("C1", carrier_bytes);
+  P.o_c2 = B.alloc("C2", carrier_bytes);
   const int ndense = train ? R : 2;
-  for (int i = 0; i < ndense; ++i) P.o_dense.push_back(B.alloc(Ppix * 192 * 2));
+  for (int i = 0; i < ndense; ++i) P.o_dense.push_back(B.alloc("D" + std::to_string(i), Ppix * 192 * 2));
   // tail activations: fp16 [pixels][64] (one fp16 product per conv), or the [hi | lo] bf16 pairs of the split-precision form
   // (training keeps a bf16 twin of every fp16 tail activation next to it, channels [64, 128): the weight-gradient GEMM pairs it with
   // the bf16 output gradients -- tcgen05 kind::f16 takes ONE 16-bit format for both operands, and the gradients stay bf16 for range)
   const bool tf16 = P.tail_f16;
   const int ts = (tf16 && !train) ? 64 : 128;  // channels per pixel of the tail activation buffers
-  P.o_splt = B.alloc(Ppix * ts * 2);
-  for (int l = 0; l <= L; ++l) P.o_spl.push_back(B.alloc((Ppix << (2 * l)) * ts * 2));
-  P.o_splc = B.alloc((Ppix << (2 * L)) * ts * 2);
+  P.o_splt = B.alloc("SPLT", Ppix * ts * 2);
+  for (int l = 0; l <= L; ++l) P.o_spl.push_back(B.alloc("SPL" + std::to_string(l), (Ppix << (2 * l)) * ts * 2));
+  P.o_splc = B.alloc("SPLC", (Ppix << (2 * L)) * ts * 2);
   const long long HRpix = Ppix << (2 * L);
   if (train) {
-    P.o_cmask = B.alloc(HRpix * d.out_channels);
-    P.o_dyp = B.alloc(HRpix * 64 * 2);
-    P.o_g3 = B.alloc(HRpix * 64 * 2);
+    P.o_cmask = B.alloc("CMASK", HRpix * d.out_channels);
+    P.o_dyp = B.alloc("DYP", HRpix * 64 * 2);
+    P.o_g3 = B.alloc("G3", HRpix * 64 * 2);
     P.o_gu.assign(L + 1, 0);
-    for (int l = 1; l <= L; ++l) P.o_gu[l] = B.alloc((Ppix << (2 * (l - 1))) * 256 * 2);
+    for (int l = 1; l <= L; ++l) P.o_gu[l] = B.alloc("GU" + std::to_string(l), (Ppix << (2 * (l - 1))) * 256 * 2);
     {
       // weight-gradient staging: per conv [9][ci][co_pad] fp32 (upsample convs: the four phase kernels, co = 256)
       long long off = 0;
@@ -422,14 +422,14 @@ static int build_plan(b200sr_plan& P) {
       P.o_gw = B.alloc(off * 4);
       P.gw_bytes = off * 4;
     }
-    P.o_gt = B.alloc(carrier_bytes);
-    P.o_gtb = B.alloc(Ppix * 64 * 2);
-    P.o_gr = B.alloc(carrier_bytes);
-    P.o_gc1 = B.alloc(carrier_bytes);
-    P.o_gc2 = B.alloc(carrier_bytes);
-    P.o_go1 = B.alloc(Ppix * 64 * 2);
+    P.o_gt = B.alloc("GT", carrier_bytes);
+    P.o_gtb = B.alloc("GTB", Ppix * 64 * 2);
+    P.o_gr = B.alloc("GR", carrier_bytes);
+    P.o_gc1 = B.alloc("GC1", carrier_bytes);
+    P.o_gc2 = B.alloc("GC2", carrier_bytes);
+    P.o_go1 = B.alloc("GO1", Ppix * 64 * 2);
     P.o_dyb.assign(R, 0);
-    for (size_t i = 0; i < P.o_dyb.size(); ++i) P.o_dyb[i] = B.alloc(Ppix * 192 * 2);
+    for (size_t i = 0; i < P.o_dyb.size(); ++i) P.o_dyb[i] = B.alloc("DYB" + std::to_string(i), Ppix * 192 * 2);
   }
   P.ws_bytes = B.cursor;
 

@@ -95,7 +95,7 @@ def test_debug_buffer_regions_match_the_layout_table(L, geom, training):
             assert _lookup(L, plan.handle, name)[0] == -1, name  # B200SR_ERR_INVALID: an inference plan keeps no gradients
 
 
-def test_debug_buffer_rejects_unknown_names_and_other_plans(L):
+def test_debug_buffer_rejects_unknown_and_foreign_names(L):
     plan = _disc_plan(3, 1, 2, 64, 64, True)
     for name in ("nope", "", "t0u", "G6", "xin "):
         rc, _, _ = _lookup(L, plan.handle, name)
@@ -105,8 +105,13 @@ def test_debug_buffer_rejects_unknown_names_and_other_plans(L):
     handle = C.c_void_p()
     assert L.b200sr_plan_create(C.byref(nd), C.byref(handle)) == 0
     try:
-        for name in ("xin", "T0u", "DYP", "G0"):
-            assert _lookup(L, handle, name)[0] == -1, name
+        # a generator plan names its own tensors (test_gen_stages_gpu.py): the names it shares with the discriminator resolve to the
+        # generator's regions, every discriminator-only name is rejected
+        for name in set(FWD_LAYOUT) | set(BWD_LAYOUT):
+            if name not in ("xin", "DYP", "G3"):
+                assert _lookup(L, handle, name)[0] == -1, name
+        assert _lookup(L, handle, "xin")[2] == 2 * 32 * 32 * 64 * 2    # conv1 input [hi | lo | hi | 0], 64 channels
+        assert _lookup(L, handle, "DYP")[2] == 2 * 128 * 128 * 64 * 2  # x4 output gradient, 64 channels
     finally:
         L.b200sr_plan_destroy(handle)
     vd = _lib.VggDesc(2, 32, 32, 15, 1 << 15, -1, 0, (C.c_float * 3)(0.5, 0.5, 0.5), (C.c_float * 3)(0.25, 0.25, 0.25))
