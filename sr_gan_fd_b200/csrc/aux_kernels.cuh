@@ -206,62 +206,14 @@ __global__ void ingest_grad_kernel(const float* __restrict__ dy, const unsigned 
 }
 
 // ------------------------------------------------------------------------------------------------ bias gradients
-// db[c] += sum over pixels of g[pixel][c0 + c] for c in [0, ncols).  g is bf16 [P][stride]; ncols is even.
-// Thread layout: (ncols/2) channel-pair lanes x PL pixel lanes, so a warp reads consecutive channels of one pixel row
-// (coalesced); pixel lanes are reduced through shared memory, one atomicAdd per channel and block.
+// db[c] += sum over pixels of g[pixel][c0 + c] for c in [0, ncols).  g is bf16 (or fp16) [P][stride]; ncols, c0 and stride are
+// multiples of 8 and g is 16-byte aligned.  Each thread owns EIGHT consecutive channels of a pixel row (one 16-byte load, four of
+// them in flight); pixel lanes are reduced through shared memory, one atomicAdd per channel and block.  The launch uses at most two
+// blocks per SM: those final atomics all hit the SAME few addresses and cost ~45 ns each once a thousand blocks queue up on one.
 struct BiasGradSeg { int col_begin, col_end; float* out; int n_valid; };
 struct BiasGradParams { const __nv_bfloat16* g; long long P; int stride; int c0; int ncols; int nseg; BiasGradSeg seg[5]; int f16; };
-__device__ __forceinline__ float2 ld16x2_f32(const __nv_bfloat162* p, bool f16) {
-  return f16 ? __half22float2(*reinterpret_cast<const __half2*>(p)) : __bfloat1622float2(*p);
-}
 constexpr int kBiasGradThreads = 256;
 
-__global__ void __launch_bounds__(kBiasGradThreads) bias_grad_kernel(const BiasGradParams p) {
-  __shared__ float2 red[kBiasGradThreads];
-  const int half = p.ncols >> 1;              // channel pairs
-  const int PL = kBiasGradThreads / half;     // pixel lanes per block
-  const int cp = threadIdx.x % half;
-  const int pl = threadIdx.x / half;
-  float2 acc = make_float2(0.f, 0.f);
-  if (pl < PL) {
-    const __nv_bfloat162* base = reinterpret_cast<const __nv_bfloat162*>(p.g + p.c0) + cp;
-    const long long step = static_cast<long long>(gridDim.x) * PL;
-    const long long sp = p.stride >> 1;
-    long long px = static_cast<long long>(blockIdx.x) * PL + pl;
-    // four independent loads in flight per thread (the loop is latency-bound otherwise)
-    float2 a1 = make_float2(0.f, 0.f), a2 = a1, a3 = a1;
-    for (; px + 3 * step < p.P; px += 4 * step) {
-      const bool hf = p.f16 != 0;
-      const float2 v0 = ld16x2_f32(base + px * sp, hf);
-      const float2 v1 = ld16x2_f32(base + (px + step) * sp, hf);
-      const float2 v2 = ld16x2_f32(base + (px + 2 * step) * sp, hf);
-      const float2 v3 = ld16x2_f32(base + (px + 3 * step) * sp, hf);
-      acc.x += v0.x; acc.y += v0.y; a1.x += v1.x; a1.y += v1.y; a2.x += v2.x; a2.y += v2.y; a3.x += v3.x; a3.y += v3.y;
-    }
-    for (; px < p.P; px += step) {
-      const float2 v = ld16x2_f32(base + px * sp, p.f16 != 0);
-      acc.x += v.x; acc.y += v.y;
-    }
-    acc.x += a1.x + a2.x + a3.x; acc.y += a1.y + a2.y + a3.y;
-  }
-  red[threadIdx.x] = acc;
-  __syncthreads();
-  if (pl == 0) {
-    for (int i = 1; i < PL; ++i) { acc.x += red[i * half + cp].x; acc.y += red[i * half + cp].y; }
-    for (int k = 0; k < 2; ++k) {
-      const int c = 2 * cp + k;
-      const float s = k ? acc.y : acc.x;
-      for (int sgi = 0; sgi < p.nseg; ++sgi) {
-        const BiasGradSeg& sg = p.seg[sgi];
-        if (c >= sg.col_begin && c < sg.col_end && (c - sg.col_begin) < sg.n_valid) atomicAdd(sg.out + (c - sg.col_begin), s);
-      }
-    }
-  }
-}
-
-// Vector form (ncols, c0 and stride multiples of 8): each thread owns EIGHT consecutive channels of a pixel row (one 16-byte load, four of
-// them in flight) and the launch uses at most two blocks per SM -- the scalar form above spends its time in the final atomics (one per
-// channel and block onto the SAME few addresses: ~45 ns each once a thousand blocks queue up on one address), not in the loads.
 __global__ void __launch_bounds__(kBiasGradThreads) bias_grad_vec_kernel(const BiasGradParams p) {
   __shared__ float red[8 * kBiasGradThreads];
   const int L = p.ncols >> 3;                 // 8-channel lanes per pixel row

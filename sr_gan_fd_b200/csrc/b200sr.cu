@@ -222,8 +222,6 @@ struct b200sr_plan {
   size_t counters_bytes = 0;          // 16 KB of counters + the largest chain's (entries x items) flag matrix
 };
 
-// K = 32 pass layers carry 64-byte weight rows (B200SR_K32=0: padded 128-byte rows as for every other layer)
-static const bool g_k32 = [] { const char* e = getenv("B200SR_K32"); return !(e && atoi(e) == 0); }();
 static int wmap_index(int n_cols) { return n_cols == 16 ? 0 : n_cols == 32 ? 1 : n_cols == 64 ? 2 : 3; }
 static const int kWmapCols[4] = {16, 32, 64, 128};
 
@@ -519,7 +517,7 @@ static int build_plan(b200sr_plan& P) {
         const int col_lo = 32 * q, ncols = 128 - col_lo;
         PackOp op; memset(&op, 0, sizeof(op));
         op.n_total = ncols; op.n_cols = ncols; op.n_valid = ncols; op.num_chunks = 1; op.mode = kPackFwd; op.nseg = 0;
-        op.k32 = (klen == 32 && g_k32) ? 1 : 0;
+        op.k32 = (klen == 32) ? 1 : 0;  // K = 32 pass layers carry 64-byte weight rows
         for (int k = q + 1; k <= 4; ++k)
           op.seg[op.nseg++] = nseg(32 * (k - 1) - col_lo, 32, 0, klen, 2 * conv_index_rdb(r, k), 32, 64 + 32 * (k - 1), 0, c_q);
         const int row0 = B.add_pack(op);
@@ -634,16 +632,16 @@ static int build_plan(b200sr_plan& P) {
       wb.tiles_x = (w + kTileW - 1) / kTileW; wb.tiles_y = (h + kWgTileH - 1) / kWgTileH; wb.num_tiles = n * wb.tiles_x * wb.tiles_y;
       return s;
     };
-    auto add_problem = [&](Step& s, int a_c0, int b_c0, int n_cols, int bias_mode, int a_blocks = 2) {
+    auto add_problem = [&](Step& s, int a_c0, int b_c0, int n_cols, int a_blocks = 2) {
       WgradParams& wp = s.wb.prob[s.wb.num_problems++];
-      wp.b_c0 = b_c0; wp.n_cols = n_cols; wp.n_blocks = (n_cols + 63) / 64; wp.bias_mode = bias_mode;
+      wp.b_c0 = b_c0; wp.n_cols = n_cols; wp.n_blocks = (n_cols + 63) / 64;
       wgrad_set_a(wp, a_c0, a_blocks);
       return s.wb.num_problems - 1;
     };
     // packed problem: M block 0 = X channels [c0, c0 + 64) at tap dx0, block 1 = the same channels at tap dx1 (>= 0) or all ones (-1)
     auto add_packed = [&](Step& s, int c0, int dx0, int dx1, int b_c0, int n_cols) {
       WgradParams& wp = s.wb.prob[s.wb.num_problems++];
-      wp.b_c0 = b_c0; wp.n_cols = n_cols; wp.n_blocks = (n_cols + 63) / 64; wp.bias_mode = 0;
+      wp.b_c0 = b_c0; wp.n_cols = n_cols; wp.n_blocks = (n_cols + 63) / 64;
       wp.blk[0].kind = kWgBlkX; wp.blk[0].c0 = c0; wp.blk[0].dx = dx0;
       wp.blk[1].kind = dx1 >= 0 ? kWgBlkX : kWgBlkOnes; wp.blk[1].c0 = c0; wp.blk[1].dx = dx1 >= 0 ? dx1 : 0;
       return s.wb.num_problems - 1;
@@ -659,7 +657,7 @@ static int build_plan(b200sr_plan& P) {
     auto wgrad_step = [&](long long x_off, int x_cvalid, int x_cpix, long long dy_off, int dy_cvalid, int dy_cpix, int n, int h, int w,
                           int a_c0, int b_c0, int n_cols) {  // single-problem launch
       Step s = wgrad_batch(x_off, x_cvalid, x_cpix, dy_off, dy_cvalid, dy_cpix, n, h, w);
-      add_problem(s, a_c0, b_c0, n_cols, 0, (x_cvalid - a_c0 > 64) ? 2 : 1);
+      add_problem(s, a_c0, b_c0, n_cols, (x_cvalid - a_c0 > 64) ? 2 : 1);
       return s;
     };
     auto biasgrad_step = [&](long long g_off, long long npix, int stride, int c0, int ncols) {
@@ -787,9 +785,7 @@ static int build_plan(b200sr_plan& P) {
     // The data-gradient chain is cut ONCE, behind the HR tail: the tail's weight / bias gradients (HR-sized, L2-heavy, 8 % of the
     // weight-gradient FLOPs but 12 % of their time) then run on the side streams WHILE the trunk chain -- latency-bound, launched on one
     // CTA per work item of an image group (128 of 148 SMs at config 2) -- walks the 69 dense blocks (run_steps defers them behind it).
-    static const bool bwd_split = [] { const char* e = getenv("B200SR_BWD_SPLIT"); return e ? atoi(e) != 0 : true; }();
-    const bool split_here = bwd_split && P.reassoc && P.groups >= 2;
-    if (split_here) {
+    if (P.reassoc && P.groups >= 2) {
       for (const Step& c : seg_convs) P.bwd.push_back(c);
       for (const Step& o : seg_others) P.bwd.push_back(o);
       seg_convs.clear(); seg_others.clear();
@@ -838,7 +834,7 @@ static int build_plan(b200sr_plan& P) {
           const int col_lo = 32 * q, ncols = 128 - col_lo;
           PackOp op; memset(&op, 0, sizeof(op));
           op.n_total = ncols; op.n_cols = ncols; op.n_valid = ncols; op.num_chunks = 1; op.mode = kPackDgrad; op.nseg = 0;
-          op.k32 = (klen == 32 && g_k32) ? 1 : 0;
+          op.k32 = (klen == 32) ? 1 : 0;
           for (int sidx = 4 - q; sidx >= 1; --sidx)
             op.seg[op.nseg++] = nseg(32 * (4 - sidx) - col_lo, 32, 0, klen, 2 * ci, klen, 64 + 32 * (kk - 1), 0, 64 + 32 * (sidx - 1));
           const int row0 = B.add_pack(op);
@@ -879,58 +875,36 @@ static int build_plan(b200sr_plan& P) {
         }
         emit(s);
       }
-      // weight gradients of the five convs, re-associated by input slice
-      static const bool wgrad_pack = [] { const char* e = getenv("B200SR_WGRAD_PACK"); return e ? atoi(e) != 0 : true; }();
-      if (wgrad_pack) {
-        // ONE launch per dense block, five problems, no idle accumulator rows: the 64-channel slices (x for conv1, o3|o4 for
-        // conv4 / conv5) put two horizontal taps into one CTA's M = 128, and the third tap shares its CTA with an all-ones block
-        // whose column sums are the bias gradients of all five convs.  Per 128-pixel tile: 7 CTA-units of (M = 128) x N x 24
-        // MMAs (3 x 160 + 160 + 96 + 32 + 32 = 800 columns) where the unpacked list below has 9 + 1/3 (928 columns).
-        const int c5 = conv_index_rdb(r, 5), c4 = conv_index_rdb(r, 4), c3 = conv_index_rdb(r, 3), c2 = conv_index_rdb(r, 2),
-                  c1 = conv_index_rdb(r, 1);
-        Step wg = wgrad_batch(D, 192, 192, DYc, 192, 192, N, H, W);
-        add_problem(wg, 0, 0, 160, 0);          // x, o1, o2 rows at the CTA's tap x [dY5|dY4|dY3|dY2]
-        add_seg(wg, 0, 64, wref(c5), 192, 0, 64);
-        add_seg(wg, 64, 96, wref(c4), 160, 0, 32);
-        add_seg(wg, 96, 128, wref(c3), 128, 0, 32);
-        add_seg(wg, 128, 160, wref(c2), 96, 0, 32);
-        add_packed(wg, 128, 2, -1, 0, 160);     // (o3|o4 at dx 2 | ones) x [dY5|dY4|dY3|dY2]
-        add_seg(wg, 0, 64, wref(c5), 192, 128, 64, 1);
-        add_seg(wg, 64, 96, wref(c4), 160, 128, 32, 1);
-        add_seg(wg, 0, 64, bref(c5), 1, 0, 64, 2);
-        add_seg(wg, 64, 96, bref(c4), 1, 0, 32, 2);
-        add_seg(wg, 96, 128, bref(c3), 1, 0, 32, 2);
-        add_seg(wg, 128, 160, bref(c2), 1, 0, 32, 2);
-        add_packed(wg, 128, 0, 1, 0, 96);       // (o3|o4 at dx 0 | o3|o4 at dx 1) x [dY5|dY4]
-        add_seg(wg, 0, 64, wref(c5), 192, 128, 64);
-        add_seg(wg, 64, 96, wref(c4), 160, 128, 32);
-        add_packed(wg, 0, 0, 1, 160, 32);       // (x at dx 0 | x at dx 1) x dY1
-        add_seg(wg, 0, 32, wref(c1), 64, 0, 32);
-        add_packed(wg, 0, 2, -1, 160, 32);      // (x at dx 2 | ones) x dY1
-        add_seg(wg, 0, 32, wref(c1), 64, 0, 32, 1);
-        add_seg(wg, 0, 32, bref(c1), 1, 0, 32, 2);
-        emit(wg);
-      } else {
-        // ONE launch per dense block: three channel-block problems + the bias gradients (all-ones A operand)
-        Step wg = wgrad_batch(D, 192, 192, DYc, 192, 192, N, H, W);
-        add_problem(wg, 0, 0, 160, 0);   // x, o1, o2 rows x [dY5|dY4|dY3|dY2]
-        add_seg(wg, 0, 64, wref(conv_index_rdb(r, 5)), 192, 0, 64);
-        add_seg(wg, 64, 96, wref(conv_index_rdb(r, 4)), 160, 0, 32);
-        add_seg(wg, 96, 128, wref(conv_index_rdb(r, 3)), 128, 0, 32);
-        add_seg(wg, 128, 160, wref(conv_index_rdb(r, 2)), 96, 0, 32);
-        add_problem(wg, 128, 0, 96, 0, 1);  // o3, o4 rows (64 channels: one X box) x [dY5|dY4]
-        add_seg(wg, 0, 64, wref(conv_index_rdb(r, 5)), 192, 128, 64);
-        add_seg(wg, 64, 96, wref(conv_index_rdb(r, 4)), 160, 128, 32);
-        add_problem(wg, 0, 160, 32, 0, 1);  // x rows (one X box) x dY1 (conv1)
-        add_seg(wg, 0, 32, wref(conv_index_rdb(r, 1)), 64, 0, 32);
-        add_problem(wg, 0, 0, 192, 1);   // bias gradients: column sums of [dY5|dY4|dY3|dY2|dY1]
-        add_seg(wg, 0, 64, bref(conv_index_rdb(r, 5)), 1, 0, 64);
-        add_seg(wg, 64, 96, bref(conv_index_rdb(r, 4)), 1, 0, 32);
-        add_seg(wg, 96, 128, bref(conv_index_rdb(r, 3)), 1, 0, 32);
-        add_seg(wg, 128, 160, bref(conv_index_rdb(r, 2)), 1, 0, 32);
-        add_seg(wg, 160, 192, bref(conv_index_rdb(r, 1)), 1, 0, 32);
-        emit(wg);
-      }
+      // weight gradients of the five convs, re-associated by input slice.
+      // ONE launch per dense block, five problems, no idle accumulator rows: the 64-channel slices (x for conv1, o3|o4 for
+      // conv4 / conv5) put two horizontal taps into one CTA's M = 128, and the third tap shares its CTA with an all-ones block
+      // whose column sums are the bias gradients of all five convs.  Per 128-pixel tile: 7 CTA-units of (M = 128) x N x 24
+      // MMAs (3 x 160 + 160 + 96 + 32 + 32 = 800 columns); three channel-block problems with idle M rows and a separate bias
+      // problem would take 9 + 1/3 (928 columns).
+      const int c5 = conv_index_rdb(r, 5), c4 = conv_index_rdb(r, 4), c3 = conv_index_rdb(r, 3), c2 = conv_index_rdb(r, 2),
+                c1 = conv_index_rdb(r, 1);
+      Step wg = wgrad_batch(D, 192, 192, DYc, 192, 192, N, H, W);
+      add_problem(wg, 0, 0, 160);             // x, o1, o2 rows at the CTA's tap x [dY5|dY4|dY3|dY2]
+      add_seg(wg, 0, 64, wref(c5), 192, 0, 64);
+      add_seg(wg, 64, 96, wref(c4), 160, 0, 32);
+      add_seg(wg, 96, 128, wref(c3), 128, 0, 32);
+      add_seg(wg, 128, 160, wref(c2), 96, 0, 32);
+      add_packed(wg, 128, 2, -1, 0, 160);     // (o3|o4 at dx 2 | ones) x [dY5|dY4|dY3|dY2]
+      add_seg(wg, 0, 64, wref(c5), 192, 128, 64, 1);
+      add_seg(wg, 64, 96, wref(c4), 160, 128, 32, 1);
+      add_seg(wg, 0, 64, bref(c5), 1, 0, 64, 2);
+      add_seg(wg, 64, 96, bref(c4), 1, 0, 32, 2);
+      add_seg(wg, 96, 128, bref(c3), 1, 0, 32, 2);
+      add_seg(wg, 128, 160, bref(c2), 1, 0, 32, 2);
+      add_packed(wg, 128, 0, 1, 0, 96);       // (o3|o4 at dx 0 | o3|o4 at dx 1) x [dY5|dY4]
+      add_seg(wg, 0, 64, wref(c5), 192, 128, 64);
+      add_seg(wg, 64, 96, wref(c4), 160, 128, 32);
+      add_packed(wg, 0, 0, 1, 160, 32);       // (x at dx 0 | x at dx 1) x dY1
+      add_seg(wg, 0, 32, wref(c1), 64, 0, 32);
+      add_packed(wg, 0, 2, -1, 160, 32);      // (x at dx 2 | ones) x dY1
+      add_seg(wg, 0, 32, wref(c1), 64, 0, 32, 1);
+      add_seg(wg, 0, 32, bref(c1), 1, 0, 32, 2);
+      emit(wg);
       if (j == 0) {
         // gradient buckets: G RRDBs each (their convs are contiguous in the flat buffer); the LAST trunk bucket is at most two
         // RRDBs so that little communication is left after the final kernels
@@ -1153,24 +1127,21 @@ static int ensure_maps(b200sr_plan& P, void* wsp, void* packed, cudaStream_t st)
         // and everything older is covered transitively (release / acquire chains stay inside the image's CTAs, which have
         // themselves seen every earlier whole-entry announcement).  Images then drift apart instead of meeting at a 128-CTA
         // rendezvous after every layer.
-        static const bool img_deps = [] { const char* e = getenv("B200SR_IMG_DEPS"); return e ? atoi(e) != 0 : true; }();
-        if (img_deps) {
-          std::vector<int> ok((size_t)s.nentries, -1);  // -1: no consumer yet, 1: all consumers eligible so far, 0: not eligible
-          for (int i = 0; i < s.nentries; ++i) {
-            const EntryDesc& e = P.h_entries[s.entry0 + i];
-            if (e.dep < 0) continue;
-            const EntryDesc& dpe = P.h_entries[s.entry0 + e.dep];
-            const ConvParams& ce = P.layer_steps[e.layer].cp;
-            const ConvParams& cd = P.layer_steps[dpe.layer].cp;
-            const int tpi = ce.tiles_x * ce.tiles_y, ntiles = e.tile_hi - e.tile_lo;
-            const bool same = ce.col_groups == 1 && cd.col_groups == 1 && e.tile_lo == dpe.tile_lo && e.tile_hi == dpe.tile_hi && e.rot == dpe.rot &&
-                              ce.tiles_x == cd.tiles_x && ce.tiles_y == cd.tiles_y && ntiles <= grid && tpi >= 2 && ntiles / tpi <= kCtrStride - 1;
-            if (!same) ok[e.dep] = 0;
-            else if (ok[e.dep] < 0) ok[e.dep] = 1;
-          }
-          for (int i = 0; i < s.nentries; ++i)
-            if (ok[i] == 1) P.h_entries[s.entry0 + i].pad[0] = 1;
+        std::vector<int> ok((size_t)s.nentries, -1);  // -1: no consumer yet, 1: all consumers eligible so far, 0: not eligible
+        for (int i = 0; i < s.nentries; ++i) {
+          const EntryDesc& e = P.h_entries[s.entry0 + i];
+          if (e.dep < 0) continue;
+          const EntryDesc& dpe = P.h_entries[s.entry0 + e.dep];
+          const ConvParams& ce = P.layer_steps[e.layer].cp;
+          const ConvParams& cd = P.layer_steps[dpe.layer].cp;
+          const int tpi = ce.tiles_x * ce.tiles_y, ntiles = e.tile_hi - e.tile_lo;
+          const bool same = ce.col_groups == 1 && cd.col_groups == 1 && e.tile_lo == dpe.tile_lo && e.tile_hi == dpe.tile_hi && e.rot == dpe.rot &&
+                            ce.tiles_x == cd.tiles_x && ce.tiles_y == cd.tiles_y && ntiles <= grid && tpi >= 2 && ntiles / tpi <= kCtrStride - 1;
+          if (!same) ok[e.dep] = 0;
+          else if (ok[e.dep] < 0) ok[e.dep] = 1;
         }
+        for (int i = 0; i < s.nentries; ++i)
+          if (ok[i] == 1) P.h_entries[s.entry0 + i].pad[0] = 1;
       }
     };
     build_entries(P.fwd);
@@ -1247,18 +1218,16 @@ static int launch_chain(b200sr_plan& P, const Step& s, const Bases& b, cudaStrea
   return 0;
 }
 
-// SMs one wgrad wave may use (B200SR_WGRAD_SMS, experiment: leave room for concurrently running NCCL kernels)
-static const int g_wgrad_sms_cap = [] { const char* e = getenv("B200SR_WGRAD_SMS"); return e ? atoi(e) : 0; }();
-static int launch_wgrad(const Step& s, const CUtensorMap& tmX, const CUtensorMap& tmDY, const Bases& b, cudaStream_t st, int default_cap = 0) {
+// sms_cap: SMs one wgrad wave may use (0: all)
+static int launch_wgrad(const Step& s, const CUtensorMap& tmX, const CUtensorMap& tmDY, const Bases& b, cudaStream_t st, int sms_cap) {
   WgradBatch wb = s.wb;
-  const int cap = g_wgrad_sms_cap > 0 ? g_wgrad_sms_cap : default_cap;
-  const int sms = (cap > 0 && cap < g_num_sms) ? cap : g_num_sms;
+  const int sms = (sms_cap > 0 && sms_cap < g_num_sms) ? sms_cap : g_num_sms;
   // deal the CTAs of one wave out in proportion to each problem's cost (max of tensor cycles and L2->SM bytes / 42 B per clock)
   double work[kWgMaxProblems], total = 0;
   for (int j = 0; j < wb.num_problems; ++j) {
     WgradParams& wp = wb.prob[j];
     for (int i = 0; i < wp.num_seg; ++i) wp.seg[i].out = (float*)resolve(s.wseg_out[j][i], b);
-    const int nacc = wp.bias_mode ? 1 : (wp.dy_mask ? __builtin_popcount(wp.dy_mask) : 3);
+    const int nacc = wp.dy_mask ? __builtin_popcount(wp.dy_mask) : 3;
     const double mma = nacc * 8.0 * (wp.n_cols / 2.0);
     const double ld = wgrad_load_bytes(wp) / 42.0;
     work[j] = (mma > ld ? mma : ld) * wgrad_ntap(wp);
@@ -1290,12 +1259,11 @@ static int run_steps(b200sr_plan& P, std::vector<Step>& steps, const Bases& b, c
   // Generator plans (round 2, same-box scans over streams x CTAs per launch): FOUR streams with HALF of the SMs per launch
   // -- fewer pixel splits per dense block = fewer partial sums flushed with red.global.add into the same addresses, and the launches
   // of neighbouring blocks run side by side -- 11.93 -> 11.73 ms/step (2 streams x all SMs: the round-1 setting, kept for the
-  // discriminator / VGG plans).  B200SR_WGRAD_STREAMS / B200SR_WGRAD_SMS override both.
-  static const int env_streams = [] { const char* e = getenv("B200SR_WGRAD_STREAMS"); int v = e ? atoi(e) : 0; return v < 0 ? 0 : (v > 4 ? 4 : v); }();
+  // discriminator / VGG plans).
   const bool gen_plan = !P.is_disc && !P.is_vgg;
-  const int nstreams = env_streams > 0 ? env_streams : (gen_plan ? 4 : 2);
+  const int nstreams = gen_plan ? 4 : 2;
   const int wgrad_cap = gen_plan ? g_num_sms / 2 : 0;  // two launches exactly side by side (74 + 74 on 148 SMs)
-  const bool alternate = nstreams > 1 && (&steps == &P.bwd);
+  const bool alternate = &steps == &P.bwd;
   bool forked = false, side_dirty = false;
   int wcount = 0;
   auto join = [&]() -> int {
@@ -1322,26 +1290,21 @@ static int run_steps(b200sr_plan& P, std::vector<Step>& steps, const Bases& b, c
     BiasGradParams bp = s.bp;
     bp.g = (const __nv_bfloat16*)resolve(s.bg_g, b);
     for (int i = 0; i < bp.nseg; ++i) bp.seg[i].out = (float*)resolve(s.seg_out[i], b);
-    static const bool vec_ok = [] { const char* e = getenv("B200SR_BIASGRAD_VEC"); return e ? atoi(e) != 0 : true; }();
-    if (vec_ok && bp.ncols % 8 == 0 && bp.ncols / 8 <= kBiasGradThreads && bp.c0 % 8 == 0 && bp.stride % 8 == 0 &&
-        (reinterpret_cast<uintptr_t>(bp.g) & 15) == 0) {
-      const int plv = kBiasGradThreads / (bp.ncols / 8);
-      long long blocks = (bp.P + plv * 8 - 1) / (plv * 8);
-      if (blocks > 2 * g_num_sms) blocks = 2 * g_num_sms;
-      bias_grad_vec_kernel<<<(int)blocks, kBiasGradThreads, 0, bs>>>(bp);
-      CUDA_TRY(cudaGetLastError());
-      return 0;
-    }
-    const int pl = kBiasGradThreads / (bp.ncols / 2);
-    long long blocks = (bp.P + pl * 16 - 1) / (pl * 16);
-    if (blocks > 8 * g_num_sms) blocks = 8 * g_num_sms;
-    bias_grad_kernel<<<(int)blocks, kBiasGradThreads, 0, bs>>>(bp);
+    // every plan's bias-gradient steps satisfy this (ncols 16 / 64 / 256, c0 = 0, stride 64 / 256, 1024-aligned buffers)
+    if (bp.ncols % 8 != 0 || bp.ncols / 8 > kBiasGradThreads || bp.c0 % 8 != 0 || bp.stride % 8 != 0 ||
+        (reinterpret_cast<uintptr_t>(bp.g) & 15) != 0)
+      return fail(B200SR_ERR_INVALID, "internal: bias-gradient step with ncols %d, c0 %d, stride %d is not 16-byte vectorisable",
+                  bp.ncols, bp.c0, bp.stride);
+    const int plv = kBiasGradThreads / (bp.ncols / 8);
+    long long blocks = (bp.P + plv * 8 - 1) / (plv * 8);
+    if (blocks > 2 * g_num_sms) blocks = 2 * g_num_sms;
+    bias_grad_vec_kernel<<<(int)blocks, kBiasGradThreads, 0, bs>>>(bp);
     CUDA_TRY(cudaGetLastError());
     return 0;
   };
   // Weight / bias gradients that sit between two data-gradient chains (the HR tail's, see build_plan) are DEFERRED behind the launch of
   // the second chain and go to the side streams only: the trunk chain, enqueued first, takes its SMs, they fill the rest and run beside it.
-  const int overlap_chain = (alternate && !cb && nstreams > 1 && b.grads) ? P.bwd_overlap_chain : -1;
+  const int overlap_chain = (alternate && !cb && b.grads) ? P.bwd_overlap_chain : -1;
   std::vector<int> deferred;
   for (size_t si = 0; si < steps.size(); ++si) {
     Step& s = steps[si];
@@ -1547,8 +1510,6 @@ static const int kVggCin[16] = {3, 64, 64, 128, 128, 256, 256, 256, 256, 512, 51
 static const int kVggCout[16] = {64, 64, 128, 128, 256, 256, 256, 256, 512, 512, 512, 512, 512, 512, 512, 512};
 static const bool kVggPoolAfter[16] = {false, true, false, true, false, false, false, true, false, false, false, true, false, false, false, false};
 
-// B200SR_N128=0: column groups of 64 everywhere in the discriminator / VGG plans (A/B switch)
-static const bool g_n128 = [] { const char* e = getenv("B200SR_N128"); return !(e && atoi(e) == 0); }();
 static int build_vgg_plan(b200sr_plan& P) {
   const b200sr_vgg_desc& v = P.vd;
   if (v.batch < 1 || v.height < 1 || v.width < 1) return fail(B200SR_ERR_INVALID, "bad geometry");
@@ -1603,7 +1564,7 @@ static int build_vgg_plan(b200sr_plan& P) {
   { Step s; s.type = ST_VGG_INGEST; P.fwd.push_back(s); }
   for (int l = 0; l < NL; ++l) {
     const int cin = kVggCin[l], cout = kVggCout[l], hh = P.vgg_h[l], ww = P.vgg_w[l];
-    const int n_cols = (g_n128 && cout % 128 == 0) ? 128 : 64;  // column groups of 128 for the wide layers, else 64
+    const int n_cols = (cout % 128 == 0) ? 128 : 64;  // column groups of 128 for the wide layers, else 64
     PackOp op; memset(&op, 0, sizeof(op));
     op.n_total = cout; op.n_cols = n_cols; op.n_valid = cout; op.mode = kPackFwd;
     int amap, chunks, ksl;
@@ -1640,7 +1601,7 @@ static int build_vgg_plan(b200sr_plan& P) {
     for (int l = v.grad_conv; l >= 0; --l) {
       const int cin = kVggCin[l], cout = kVggCout[l], hh = P.vgg_h[l], ww = P.vgg_w[l];
       const int nin = (l == 0) ? 16 : cin;  // dgrad output channels (conv 0: 3 padded to 16, stored NCHW fp32 to dx)
-      const int n_cols = (l == 0) ? 16 : ((g_n128 && cin % 128 == 0) ? 128 : 64);
+      const int n_cols = (l == 0) ? 16 : ((cin % 128 == 0) ? 128 : 64);
       PackOp op; memset(&op, 0, sizeof(op));
       op.n_total = nin; op.n_cols = n_cols; op.n_valid = (l == 0) ? 3 : cin; op.num_chunks = cout / 64; op.mode = kPackDgrad; op.nseg = 1;
       op.seg[0] = seg(0, cout, 2 * l, cout, cin, 0, 0, 0);
@@ -1697,8 +1658,6 @@ static int build_vgg_plan(b200sr_plan& P) {
 // stride-2 conv is then an ordinary 3x3 conv over 4C channels (weights packed with structural zeros, kPackDownFwd), its data
 // gradient an ordinary 3x3 dgrad whose 4C output columns are pixel-shuffled back to the plain layout on store, and its weight
 // gradient the ordinary 3x3 wgrad over the U-layout input, gathered to [co][c][4][4] by unpack_wgrad_down_kernel.
-// B200SR_DOWN4=0: the stride-2 convs run all nine taps of the unshuffled 3x3 form (structural zeros included) -- A/B switch
-static const bool g_down4 = [] { const char* e = getenv("B200SR_DOWN4"); return !(e && atoi(e) == 0); }();
 static int build_disc_plan(b200sr_plan& P) {
   const b200sr_disc_desc& v = P.dd;
   if (v.channels != 64) return fail(B200SR_ERR_INVALID, "only channels=64 is supported (got %d)", v.channels);
@@ -1781,11 +1740,11 @@ static int build_disc_plan(b200sr_plan& P) {
     const int lvl = cLvl[c], cout = cO[c];
     // column groups of 128 for the wide stride-1 layers (an N = 128 tcgen05.mma does twice the work of an N = 64 one in 4/3 of the
     // time, and the activation tile is re-read half as often); the 4-tap stride-2 stages stay at 64 columns (32 KB per stage)
-    const int n_total = (c == 9) ? 16 : cout, n_cols = (c == 9) ? 16 : ((g_n128 && mode == kPackFwd && cout % 128 == 0) ? 128 : 64);
+    const int n_total = (c == 9) ? 16 : cout, n_cols = (c == 9) ? 16 : ((mode == kPackFwd && cout % 128 == 0) ? 128 : 64);
     PackOp op; memset(&op, 0, sizeof(op));
     op.n_total = n_total; op.n_cols = n_cols; op.n_valid = cout; op.mode = mode; op.num_chunks = c_in / 64; op.nseg = 1;
     op.seg[0] = seg(0, c_in, 2 * c, cout, cI[c], 0, 0, 0);
-    if (mode == kPackDownFwd && g_down4) op.down_c = cI[c];
+    if (mode == kPackDownFwd) op.down_c = cI[c];
     const int row0 = B.add_pack(op);
     ConvParams cp = base_conv_params(N, lh(lvl), lw(lvl), op.num_chunks, 4, 0, 1 << 20, row0, n_cols, n_total);
     if (op.down_c > 0) { cp.w_taps = 4; cp.down_mode = 1; cp.down_c64 = cI[c] / 64; }
@@ -1845,7 +1804,7 @@ static int build_disc_plan(b200sr_plan& P) {
       PackOp op; memset(&op, 0, sizeof(op));
       op.n_total = n_total; op.n_cols = n_cols; op.n_valid = n_valid; op.mode = mode; op.num_chunks = (k_in + 63) / 64; op.nseg = 1;
       op.seg[0] = seg(0, cO[c], 2 * c, cO[c], cI[c], 0, 0, 0);
-      if (mode == kPackDownDgrad && g_down4) op.down_c = cI[c];
+      if (mode == kPackDownDgrad) op.down_c = cI[c];
       const int row0 = B.add_pack(op);
       const int kl = k_in - 64 * (op.num_chunks - 1);
       ConvParams cp = base_conv_params(N, lh(lvl), lw(lvl), op.num_chunks, (kl + 15) / 16, 0, 1 << 20, row0, n_cols, n_total);
@@ -1871,11 +1830,11 @@ static int build_disc_plan(b200sr_plan& P) {
     { Step s = dgrad_conv(8, G5, 64, 64, kPackDgrad, 64, 64, 64); mask_by(s, A4, 64); out_to(s, G4, 64); P.bwd.push_back(s); }
     { Step s = dgrad_conv(7, G4, 64, 64, kPackDgrad, 64, 64, 64); out_to(s, GS3, 64); P.bwd.push_back(s); }   // gradient of (up3 + out1)
     { Step s; s.type = ST_DISC_MASK; s.a = ws(GS3); s.b = ws(A3); s.c = ws(G3); s.pn = N; s.ph = H; s.pw = W; s.pc = 64; P.bwd.push_back(s); }
-    { Step s = dgrad_conv(6, G3, 64, 64, kPackDgrad, 128, g_n128 ? 128 : 64, 128); out_to(s, GB3, 128); P.bwd.push_back(s); }
+    { Step s = dgrad_conv(6, G3, 64, 64, kPackDgrad, 128, 128, 128); out_to(s, GB3, 128); P.bwd.push_back(s); }
     P.bwd.push_back(up_bwd(GB3, A2, GS2, GA2, 1, 128));
-    { Step s = dgrad_conv(5, GA2, 128, 128, kPackDgrad, 256, g_n128 ? 128 : 64, 256); out_to(s, GB2, 256); P.bwd.push_back(s); }
+    { Step s = dgrad_conv(5, GA2, 128, 128, kPackDgrad, 256, 128, 256); out_to(s, GB2, 256); P.bwd.push_back(s); }
     P.bwd.push_back(up_bwd(GB2, A1, GS1, GA1, 2, 256));
-    { Step s = dgrad_conv(4, GA1, 256, 256, kPackDgrad, 512, g_n128 ? 128 : 64, 512); out_to(s, GB1, 512); P.bwd.push_back(s); }
+    { Step s = dgrad_conv(4, GA1, 256, 256, kPackDgrad, 512, 128, 512); out_to(s, GB1, 512); P.bwd.push_back(s); }
     P.bwd.push_back(up_bwd(GB1, T3, -1, GT3, 3, 512));
     // stride-2 convs: 4C output columns on the conv's own lattice, pixel-shuffled to the plain layout of the finer lattice; the
     // skip connection's gradient (plain layout, finer lattice) joins before the LeakyReLU derivative of the U-layout activation
@@ -1923,11 +1882,11 @@ static int build_disc_plan(b200sr_plan& P) {
           const int ncols = std::min(128, ncols_all - cob);
           const int pj = cur.wb.num_problems++;
           WgradParams& wp = cur.wb.prob[pj];
-          wp.b_c0 = cob; wp.n_cols = ncols; wp.n_blocks = (ncols + 63) / 64; wp.bias_mode = 0;
+          wp.b_c0 = cob; wp.n_cols = ncols; wp.n_blocks = (ncols + 63) / 64;
           wgrad_set_a(wp, cib, (x_cvalid - cib > 64) ? 2 : 1);
           WgradSegment& g = wp.seg[0];
           g.col_begin = 0; g.col_end = ncols; g.out = nullptr; g.ci_total = ci_total; g.ci0 = cib; g.co_pad = coPad[c];
-          if (cK[c] == 4 && g_down4) {
+          if (cK[c] == 4) {
             // U-layout input channels [cib, cib + 128): phases of the first and the last channel of the block (equal when a phase
             // is >= 128 channels wide); a phase (py, px) keeps tap rows {1,2} / {0,1} for py = 0 / 1, columns alike
             const int hi = std::min(cib + 128, x_cvalid) - 1;

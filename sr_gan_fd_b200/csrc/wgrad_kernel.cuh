@@ -12,31 +12,26 @@
 // pixel loop and are flushed once with 16-byte vector reductions (red.global.add.v4.f32) into a [tap][co/4][ci][4]
 // fp32 staging tensor; a small unpack kernel transposes that to the OIHW gradient layout per gradient bucket.
 //
-// One launch carries a BATCH of up to five such problems over the same two tensor maps (the channel-block problems of a
-// dense block + its bias gradients), with the CTAs dealt out in proportion to each problem's cost so the whole dense
-// block is one balanced wave.  The bias gradient is the same GEMM with an all-ones A operand (column sums of dY), so it
-// rides the same pipeline and flush.
+// One launch carries a BATCH of up to five such problems over the same two tensor maps (the five problems of a dense
+// block), with the CTAs dealt out in proportion to each problem's cost so the whole dense block is one balanced wave.
 //
 // The two 64-row M blocks of a problem are described independently (WgradMBlock): each is X channels [c0, c0 + 64) at
 // its own horizontal tap, an all-ones block, or idle.  A CTA that needs only 64 input channels therefore fills its
-// other half with useful rows -- the same channels at another tap, or ones whose products are the bias gradients --
-// instead of multiplying rows that are never flushed (every tcgen05 MMA costs the same for M = 64 real rows as for 128).
+// other half with useful rows -- the same channels at another tap, or ones whose products are the bias gradients
+// (column sums of dY) -- instead of multiplying rows that are never flushed (every tcgen05 MMA costs the same for
+// M = 64 real rows as for 128).
 #pragma once
 #include "conv_kernel.cuh"
 
 namespace b200sr {
 
-#ifndef B200SR_WG_TILEH
-#define B200SR_WG_TILEH 16
-#endif
-constexpr int kWgTileH = B200SR_WG_TILEH;             // wgrad K-tile: 8 x 16 pixels
+constexpr int kWgTileH = 16;                         // wgrad K-tile: 8 x 16 pixels
 constexpr int kWgXRows = kWgTileH + 2;
 constexpr int kWgXBytes = kWgXRows * kTileW * 128;   // 18432 B per 64-channel haloed X tile
 constexpr int kWgBBytes = kWgTileH * kTileW * 128;   // 16384 B per 64-channel dY tile
 constexpr int kWgThreads = 192;
 constexpr int kWgMaxSeg = 6;
 constexpr int kWgMaxProblems = 5;
-constexpr int kWgOnesBytes = 4096;  // two 64-channel M blocks x 16 pixels x 128 B of bf16 1.0 (A operand of the bias-gradient problem)
 
 struct WgradSegment {
   int col_begin, col_end;  // accumulator columns of this conv's output channels (multiples of 16)
@@ -63,9 +58,8 @@ struct WgradMBlock {
 struct WgradParams {
   WgradMBlock blk[2];
   int b_c0;      // first dY channel (accumulator column 0)
-  int n_cols;    // UMMA N (multiple of 16, <= 160; bias problem: <= 256)
+  int n_cols;    // UMMA N (multiple of 16, <= 160)
   int n_blocks;  // ceil(n_cols / 64) dY boxes per tile
-  int bias_mode; // 1: A = all ones, one accumulator, no X loads, no taps: column sums of dY (blk[] unused)
   int splits;    // pixel-tile splits of this problem (CTAs = splits * wgrad_ntap)
   int num_seg;
   int dx_mask, dy_mask;  // horizontal taps that get a CTA / vertical taps that get an accumulator (0 = all three).  The 4x4 stride-2
@@ -85,18 +79,18 @@ struct WgradBatch {
 
 // ring-stage footprint (an all-ones block keeps its slot) and the bytes TMA brings in per stage
 __host__ __device__ inline int wgrad_stage_bytes(const WgradParams& p) {
-  return (p.bias_mode ? 0 : (p.blk[1].kind == kWgBlkIdle ? 1 : 2) * kWgXBytes) + p.n_blocks * kWgBBytes;
+  return (p.blk[1].kind == kWgBlkIdle ? 1 : 2) * kWgXBytes + p.n_blocks * kWgBBytes;
 }
 __host__ __device__ inline int wgrad_load_bytes(const WgradParams& p) {
-  return (p.bias_mode ? 0 : ((p.blk[0].kind == kWgBlkX) + (p.blk[1].kind == kWgBlkX)) * kWgXBytes) + p.n_blocks * kWgBBytes;
+  return ((p.blk[0].kind == kWgBlkX) + (p.blk[1].kind == kWgBlkX)) * kWgXBytes + p.n_blocks * kWgBBytes;
 }
 // CTAs per pixel split: one per horizontal tap of dx_mask when the X blocks follow the CTA's tap, else one
 __host__ __device__ inline int wgrad_ntap(const WgradParams& p) {
-  if (p.bias_mode || p.blk[0].dx >= 0) return 1;
+  if (p.blk[0].dx >= 0) return 1;
   const int m = p.dx_mask ? p.dx_mask : 7;
   return (m & 1) + ((m >> 1) & 1) + ((m >> 2) & 1);
 }
-// legacy A operand: X channels [a_c0, a_c0 + 64 * a_blocks) at the CTA's tap (a_blocks = 1: block 1 idle)
+// plain A operand: X channels [a_c0, a_c0 + 64 * a_blocks) at the CTA's tap (a_blocks = 1: block 1 idle)
 __host__ inline void wgrad_set_a(WgradParams& p, int a_c0, int a_blocks) {
   p.blk[0].kind = kWgBlkX; p.blk[0].c0 = a_c0; p.blk[0].dx = -1;
   p.blk[1].kind = a_blocks == 2 ? kWgBlkX : kWgBlkIdle; p.blk[1].c0 = a_c0 + 64; p.blk[1].dx = -1;
@@ -108,9 +102,8 @@ wgrad3x3_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
                 const __grid_constant__ WgradBatch batch) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  constexpr int kRing = kWgSmemBytes - 1024 - kWgOnesBytes - 1024;
-  uint8_t* ones = smem + kRing;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kRing + kWgOnesBytes);
+  constexpr int kRing = kWgSmemBytes - 1024 - 1024;
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + kRing);
   uint64_t* full = bars;
   uint64_t* empty = bars + 4;
   uint64_t* done = bars + 8;
@@ -126,7 +119,7 @@ wgrad3x3_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
   const int dxm = p.dx_mask ? p.dx_mask : 7, dym = p.dy_mask ? p.dy_mask : 7;
   const int ntap = wgrad_ntap(p);
   int dxi = 1;  // horizontal tap owned by this CTA: the (local % ntap)-th set bit of the mask
-  if (!p.bias_mode && p.blk[0].dx < 0) {
+  if (p.blk[0].dx < 0) {
     int k = local % ntap;
     dxi = 0;
     while (!((dxm >> dxi) & 1) || k-- > 0) ++dxi;
@@ -137,7 +130,7 @@ wgrad3x3_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
   if (S > 4) S = 4;
   const int b_off = stage_bytes - p.n_blocks * kWgBBytes;
   const int bdx0 = p.blk[0].dx >= 0 ? p.blk[0].dx : dxi, bdx1 = p.blk[1].dx >= 0 ? p.blk[1].dx : dxi;
-  const bool ones_blk = !p.bias_mode && p.blk[1].kind == kWgBlkOnes;
+  const bool ones_blk = p.blk[1].kind == kWgBlkOnes;
 
   if (warp == 0 && lane == 0) {
     prefetch_tensormap(&tmX);
@@ -150,10 +143,7 @@ wgrad3x3_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
     fence_barrier_init();
   }
   if (warp == 1) tmem_alloc_imm<512>(tmem_slot);
-  if (p.bias_mode) {
-    for (int i = threadIdx.x; i < kWgOnesBytes / 4; i += kWgThreads) reinterpret_cast<uint32_t*>(ones)[i] = batch.a_f16 ? 0x3C003C00u : 0x3F803F80u;  // 1.0 x2
-    fence_proxy_async_smem();
-  } else if (ones_blk) {
+  if (ones_blk) {
     // all-ones M block 1: its slot of every ring stage, written once (the producer never loads into it)
     constexpr int kVec = kWgXBytes / 16;
     const uint32_t one2 = batch.a_f16 ? 0x3C003C00u : 0x3F803F80u;
@@ -183,10 +173,8 @@ wgrad3x3_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
       if (elect_one_sync()) {
         uint8_t* st = smem + s * stage_bytes;
         mbar_arrive_expect_tx(&full[s], wgrad_load_bytes(p));
-        if (!p.bias_mode) {
-          if (p.blk[0].kind == kWgBlkX) tma_load_4d(st, &tmX, &full[s], p.blk[0].c0, x0 + bdx0 - 1, y0 - 1, n);
-          if (p.blk[1].kind == kWgBlkX) tma_load_4d(st + kWgXBytes, &tmX, &full[s], p.blk[1].c0, x0 + bdx1 - 1, y0 - 1, n);
-        }
+        if (p.blk[0].kind == kWgBlkX) tma_load_4d(st, &tmX, &full[s], p.blk[0].c0, x0 + bdx0 - 1, y0 - 1, n);
+        if (p.blk[1].kind == kWgBlkX) tma_load_4d(st + kWgXBytes, &tmX, &full[s], p.blk[1].c0, x0 + bdx1 - 1, y0 - 1, n);
         for (int j = 0; j < p.n_blocks; ++j)
           tma_load_4d(st + b_off + j * kWgBBytes, &tmDY, &full[s], p.b_c0 + 64 * j, x0, y0, n);
       }
@@ -205,20 +193,14 @@ wgrad3x3_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
       if (elect_one_sync()) {
         const uint32_t a0 = smem_u32(smem + s * stage_bytes);
         const uint32_t b_lo = smem_desc_lo(a0 + b_off, kWgBBytes);  // LBO = stride between 64-ch N blocks
-        if (p.bias_mode) {
-          const uint32_t o_lo = smem_desc_lo(smem_u32(ones), 2048);  // every K step reads the same all-ones tile
+        const uint32_t a_lo = smem_desc_lo(a0, kWgXBytes);          // LBO = stride between the two 64-ch M blocks
 #pragma unroll
-          for (int ks = 0; ks < kWgTileH / 2; ++ks) umma_bf16_ss_lohi(tmem_base, o_lo, b_lo + ks * 128, kHi, idesc, (ks == 0) ? acc : 1u);
-        } else {
-          const uint32_t a_lo = smem_desc_lo(a0, kWgXBytes);  // LBO = stride between the two 64-ch M blocks
+        for (int dyi = 0; dyi < 3; ++dyi) {
+          if (!((dym >> dyi) & 1)) continue;
 #pragma unroll
-          for (int dyi = 0; dyi < 3; ++dyi) {
-            if (!((dym >> dyi) & 1)) continue;
-#pragma unroll
-            for (int ks = 0; ks < kWgTileH / 2; ++ks)  // 16 pixels (two 8-pixel patch rows) per UMMA
-              umma_bf16_ss_lohi(tmem_base + dyi * p.n_cols, a_lo + dyi * 64 + ks * 128, b_lo + ks * 128, kHi, idesc,
-                                (ks == 0) ? acc : 1u);
-          }
+          for (int ks = 0; ks < kWgTileH / 2; ++ks)  // 16 pixels (two 8-pixel patch rows) per UMMA
+            umma_bf16_ss_lohi(tmem_base + dyi * p.n_cols, a_lo + dyi * 64 + ks * 128, b_lo + ks * 128, kHi, idesc,
+                              (ks == 0) ? acc : 1u);
         }
         umma_commit(&empty[s]);
       }
@@ -228,14 +210,14 @@ wgrad3x3_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
     }
     if (elect_one_sync()) umma_commit(done);
     __syncwarp();
-  } else if (has_work && (p.bias_mode || p.blk[(warp & 3) >> 1].kind != kWgBlkIdle)) {
+  } else if (has_work && p.blk[(warp & 3) >> 1].kind != kWgBlkIdle) {
     // epilogue: flush the accumulators with 16-byte fp32 vector reductions into [tap][ci][co] staging tensors.  Warps 2 + q
     // hold accumulator rows 32q .. 32q + 31: rows 0..63 are M block 0, rows 64..127 block 1.
     const int q = warp & 3;
     const int b = q >> 1;
-    const bool ones = p.bias_mode || p.blk[b].kind == kWgBlkOnes;
-    // conv input channel = sg.ci0 + m: m counts X channels from block 0's first one (bias mode / ones block: row 0 of the block)
-    const int m = p.bias_mode ? q * 32 + lane : (ones ? 0 : p.blk[b].c0 - p.blk[0].c0) + (q & 1) * 32 + lane;
+    const bool ones = p.blk[b].kind == kWgBlkOnes;
+    // conv input channel = sg.ci0 + m: m counts X channels from block 0's first one (ones block: row 0 of the block)
+    const int m = (ones ? 0 : p.blk[b].c0 - p.blk[0].c0) + (q & 1) * 32 + lane;
     const int bdx = b ? bdx1 : bdx0;
     const int nacc = ones ? 1 : 3;  // the vertical-tap accumulators of a ones block all hold the same column sums
     mbar_wait(done, 0);

@@ -10,9 +10,9 @@ Per profiled step it takes the kernel trace and reports
   * tail_ms: wall time from the end of the trunk data-gradient chain (the third chain launch of a step) to the end of the last
     wgrad3x3_kernel of the step.
 Run it in a process of its own: tracing slows the host, so end-to-end step times come from bench.py, not from here.  B200SR_LIB
-selects another build of the library (same-box A/B), B200SR_WGRAD_PACK=0 the unpacked dense-block problem list.
+selects another build of the library (same-box A/B).
 
---flops-only restates the dense-block problem lists of build_plan (b200sr.cu) and prints the MMA work they execute against the work
+--flops-only restates the dense-block problem list of build_plan (b200sr.cu) and prints the MMA work it executes against the work
 the five convs' weight and bias gradients need, per dense block at config 2 (16 x 64 x 64 pixels).
 """
 import argparse
@@ -26,26 +26,23 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
 # (CTA-units per pixel tile, N) of every problem; one unit runs M = 128 rows x N columns x 16 pixels per MMA, 3 vertical-tap
-# accumulators (1 for the legacy bias problem).  A unit is one CTA's share of one pixel split.
-UNPACKED = [("x,o1,o2 x [dY5..dY2], 3 taps", 3, 3, 160), ("o3,o4 (+64 idle rows) x [dY5|dY4], 3 taps", 3, 3, 96),
-            ("x (+64 idle rows) x dY1, 3 taps", 3, 3, 32), ("bias: ones x [dY5..dY1]", 1, 1, 192)]
+# accumulators.  A unit is one CTA's share of one pixel split.
 PACKED = [("x,o1,o2 x [dY5..dY2], 3 taps", 3, 3, 160), ("(o3,o4 @dx2 | ones) x [dY5..dY2]", 1, 3, 160),
           ("(o3,o4 @dx0 | o3,o4 @dx1) x [dY5|dY4]", 1, 3, 96), ("(x @dx0 | x @dx1) x dY1", 1, 3, 32),
           ("(x @dx2 | ones) x dY1", 1, 3, 32)]
 
 
 def dense_block_flops(pixels):
-    """GFLOP (2 per multiply-add) per dense block: executed by each problem list, and needed by the gradients themselves."""
+    """GFLOP (2 per multiply-add) per dense block: executed by the problem list, and needed by the gradients themselves."""
     useful = 0
     for k in range(1, 6):
         cin, cout = 64 + 32 * (k - 1), (64 if k == 5 else 32)
         useful += 9 * cin * cout + cout  # weight gradient (9 taps) + bias gradient, multiply-adds per pixel
     out = {"useful_gflop": 2 * useful * pixels / 1e9}
-    for tag, plist in (("unpacked", UNPACKED), ("packed", PACKED)):
-        macs = sum(units * nacc * 128 * n for _, units, nacc, n in plist)
-        out[tag + "_gflop"] = 2 * macs * pixels / 1e9
-        out[tag + "_ratio"] = macs / useful
-        out[tag + "_columns_per_tile"] = sum(units * nacc * n for _, units, nacc, n in plist) / 3
+    macs = sum(units * nacc * 128 * n for _, units, nacc, n in PACKED)
+    out["packed_gflop"] = 2 * macs * pixels / 1e9
+    out["packed_ratio"] = macs / useful
+    out["packed_columns_per_tile"] = sum(units * nacc * n for _, units, nacc, n in PACKED) / 3
     return out
 
 
@@ -96,8 +93,7 @@ def profile(args):
                          "dense_median_us": statistics.median(e["dur"] for e in after),
                          "tail_ms": (max(e["ts"] + e["dur"] for e in mine) - trunk_end) / 1e3})
     med = {k: statistics.median(s[k] for s in per_step) for k in ("wgrad_sum_ms", "dense_median_us", "tail_ms")}
-    return {"label": args.label, "steps": args.steps, "pack": os.environ.get("B200SR_WGRAD_PACK", "default"),
-            "lib": os.environ.get("B200SR_LIB", "in-tree"), "median": med, "per_step": per_step, "trace": trace}
+    return {"label": args.label, "steps": args.steps, "lib": os.environ.get("B200SR_LIB", "in-tree"), "median": med, "per_step": per_step, "trace": trace}
 
 
 def main():
