@@ -97,6 +97,25 @@ int b200sr_forward(b200sr_plan* plan, const void* x, int x_dtype, const int64_t*
 int b200sr_backward(b200sr_plan* plan, const float* dy, const void* packed, void* workspace, float* flat_grads,
                     float* dx_or_null, b200sr_bucket_cb cb, void* user, b200sr_stream stream);
 
+/* As b200sr_backward, restricted to what the caller wants (frozen and partially frozen generators).
+ * conv_wanted_or_null: host array of b200sr_num_params()/2 bytes in state_dict conv order (conv1, trunk.0.rdb1.conv1 ...
+ * conv2, upsampling*, conv3, conv4); 1 = this conv's weight and/or bias gradient is wanted.  NULL = all wanted.
+ * flat_grads_or_null: NULL = no parameter gradient at all (frozen generator); then conv_wanted must be NULL or all zero.
+ * Entries of flat_grads belonging to unwanted convs are zero.  Buckets (cb) are announced only for ranges that
+ * contain a wanted conv.
+ * The data-gradient walk reaches conv1 only when dx is wanted or conv1 is; otherwise it ends after the lowest dense block that
+ * holds a wanted conv (or after the HR tail, or is skipped).  A weight- or bias-gradient launch runs when one of the convs it
+ * writes is wanted: a dense block's five convs share one launch.  With nothing wanted (no dx, no wanted conv) the call only
+ * zeroes flat_grads_or_null.  b200sr_backward(...) is b200sr_backward_select(..., NULL, ...). */
+int b200sr_backward_select(b200sr_plan* plan, const float* dy, const void* packed, void* workspace,
+                           float* flat_grads_or_null, float* dx_or_null, const uint8_t* conv_wanted_or_null,
+                           b200sr_bucket_cb cb, void* user, b200sr_stream stream);
+/* kernel launches b200sr_backward_select enqueues for a mask (NULL = all wanted), counted as b200sr_num_launches counts them
+ * (memsets are not launches): with_dx = the input gradient is wanted, with_cb = a bucket callback is installed (one unpack
+ * launch per announced bucket instead of one merged unpack).  (plan, NULL, 0, 0) == b200sr_num_launches(plan, 1) and
+ * (plan, NULL, 0, 1) == b200sr_num_launches(plan, 2).  0 for plans without a generator backward. */
+int32_t b200sr_backward_launches(const b200sr_plan* plan, const uint8_t* conv_wanted_or_null, int with_dx, int with_cb);
+
 /* ---- single-layer entry points (used by the parity tests) ------------------------------------------------------
  * x: NHWC bf16 [n*h*w][x_stride], the conv reads channels [0, cin).  w: fp32 OIHW [cout][cin][3][3], bias [cout] or
  * NULL.  y: NHWC bf16 [n*h*w][y_stride], written at channel y_coff.  act = 1 applies LeakyReLU(0.2).
@@ -121,7 +140,8 @@ int b200sr_conv3x3_wgrad(const void* x, int n, int h, int w_, int cin, int x_str
  * block_tensor: DEVICE int32[total_blocks], block -> tensor index.  step: DEVICE float scalar, Adam steps taken so far
  * (advanced by the call unless skipped).  grad_scale / found_inf: device scalars or NULL (GradScaler protocol: gradients
  * are divided by *grad_scale; when *found_inf > 0 the Adam update is skipped -- the EMA still updates, as the reference
- * calls update_parameters unconditionally). */
+ * calls update_parameters unconditionally).  A NULL g marks a frozen parameter: no Adam update (p, m, v keep their values, as
+ * torch.optim.Adam skips a parameter without a gradient), the EMA still averages it. */
 int b200sr_fused_adam_ema(const void* tensor_table, const int32_t* block_tensor, int n_tensors, int64_t total_blocks, float lr,
                           float beta1, float beta2, float eps, float weight_decay, float* step, float ema_decay, int ema_copy,
                           const float* grad_scale, const float* found_inf, b200sr_stream stream);

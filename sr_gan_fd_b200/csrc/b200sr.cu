@@ -150,6 +150,10 @@ struct Step {
   long long cb_off = 0, cb_count = 0;
   bool needs_dx = false;  // only launched when the caller asks for the gradient w.r.t. the LR input
   bool needs_wgrad = false;  // discriminator plans: only launched when the caller asks for the parameter gradients
+  // generator backward, for b200sr_backward_select: the dense block a data-gradient conv belongs to (R: the HR tail), and the
+  // convs [wc0, wc1) whose parameter gradients a weight- / bias-gradient / carrier-sum step serves
+  int blk = -1;
+  int wc0 = 0, wc1 = 0;
 };
 
 struct b200sr_plan {
@@ -695,11 +699,15 @@ static int build_plan(b200sr_plan& P) {
     // Launch order inside one gradient bucket: all data-gradient convs first (they form ONE chain launch), then the
     // weight/bias-gradient kernels that consume what the chain produced, then the unpack + bucket announcement.
     std::vector<Step> seg_convs, seg_others;
-    auto emit = [&](const Step& st) {
+    int cur_blk = R, cur_c0 = 0, cur_c1 = 0;  // what the steps emitted next belong to (set by serves())
+    auto serves = [&](int blk, int c0, int c1) { cur_blk = blk; cur_c0 = c0; cur_c1 = c1; };
+    auto emit = [&](Step st) {
+      st.blk = cur_blk; st.wc0 = cur_c0; st.wc1 = cur_c1;
       if (st.type == ST_CONV) seg_convs.push_back(st); else seg_others.push_back(st);
     };
     // conv4: wgrad, bias grad, dgrad (-> G3, masked by lrelu'(conv3 out))
     {
+      serves(R, ci_conv4, ci_conv4 + 1);
       Step w4 = wgrad_step(P.o_splc, wg_c0 + 64, ts, P.o_dyp, 16, 64, N, hH, hW, wg_c0, 0, 16);
       add_seg(w4, 0, 16, wref(ci_conv4), 64, 0, (int)align_up(d.out_channels, 4));
       emit(w4);
@@ -715,6 +723,7 @@ static int build_plan(b200sr_plan& P) {
     }
     // conv3
     {
+      serves(R, ci_conv3, ci_conv3 + 1);
       Step w3 = wgrad_step(P.o_spl[L], wg_c0 + 64, ts, P.o_g3, 64, 64, N, hH, hW, wg_c0, 0, 64);
       add_seg(w3, 0, 64, wref(ci_conv3), 64, 0, 64);
       emit(w3);
@@ -738,6 +747,7 @@ static int build_plan(b200sr_plan& P) {
       const int ci = ci_up1 + (l - 1);
       const int h = H << (l - 1), w = W << (l - 1);
       const long long npix = Ppix << (2 * (l - 1));
+      serves(R, ci, ci + 1);
       for (int half = 0; half < 2; ++half) {
         Step wu = wgrad_step(P.o_spl[l - 1], wg_c0 + 64, ts, P.o_gu[l], 256, 256, N, h, w, wg_c0, 128 * half, 128);
         Ref out = wref(ci);
@@ -767,6 +777,7 @@ static int build_plan(b200sr_plan& P) {
     }
     // conv2
     {
+      serves(R, ci_conv2, ci_conv2 + 1);
       Step w2 = wgrad_step(P.o_splt, wg_c0 + 64, ts, P.o_gtb, 64, 64, N, H, W, wg_c0, 0, 64);
       add_seg(w2, 0, 64, wref(ci_conv2), 64, 0, 64);
       emit(w2);
@@ -797,6 +808,7 @@ static int build_plan(b200sr_plan& P) {
       const long long D = P.o_dense[r];
       const long long DYc = P.o_dyb[r];
       const long long DYn = P.o_dyb[r > 0 ? r - 1 : 0];
+      serves(r, conv_index_rdb(r, 1), conv_index_rdb(r, 5) + 1);
       // epilogue of the block-input (x) slice: fp32 gradient carriers and the next block's dY5
       auto xslice_epilogue = [&](Step& s) {
         if (j == 2) { s.r1 = ws(P.o_gr); s.cp.epi.beta1 = 0.2f; s.of = ws(P.o_gc2); s.cp.epi.delta = 0.2f; }
@@ -918,6 +930,7 @@ static int build_plan(b200sr_plan& P) {
     }
     // conv1: gradient of its output = trunk path (GR) + long skip (GT)
     {
+      serves(-1, 0, 1);
       Step ad; ad.type = ST_ADD; ad.a = ws(P.o_gr); ad.b = ws(P.o_gt); ad.c = ws(P.o_go1); ad.count = Ppix * 64;
       emit(ad);
       Step w1 = wgrad_step(P.o_xin, P.xin_stride, P.xin_stride, P.o_go1, 64, 64, N, H, W, 0, 0, 64);
@@ -1250,8 +1263,86 @@ static int launch_wgrad(const Step& s, const CUtensorMap& tmX, const CUtensorMap
   return 0;
 }
 
+// What a selective generator backward (b200sr_backward_select) computes.  Chosen per call: the plan and its step list serve
+// every freeze pattern, and run_steps skips what nobody asked for.
+struct GradSelect {
+  std::vector<uint8_t> want;  // per conv: its weight and/or bias gradient is wanted
+  int stop_blk = -1;          // data-gradient layers of dense blocks below this one are not launched (R: tail only, R + 1: none)
+  int R = 0;
+  bool any(int c0, int c1) const {
+    for (int c = c0; c < c1; ++c)
+      if (want[c]) return true;
+    return false;
+  }
+  // the convs a launch wrote: a dense block's one weight-gradient launch writes all five of its convs if any is wanted
+  bool written(int c) const {
+    if (c < 1 || c > 5 * R) return want[c] != 0;
+    const int c0 = 1 + (c - 1) / 5 * 5;
+    return any(c0, c0 + 5);
+  }
+};
+
+// mask: per conv (NULL: all); grads: a flat gradient buffer is written; dx: the input gradient is wanted
+static GradSelect make_select(const b200sr_plan& P, const uint8_t* mask, bool grads, bool dx) {
+  const int nconv = ((int)P.param_off.size() - 1) / 2;
+  GradSelect g;
+  g.R = P.R;
+  g.want.assign(nconv, 0);
+  if (grads)
+    for (int c = 0; c < nconv; ++c) g.want[c] = mask ? (mask[c] != 0) : 1;
+  // conv1's output gradient GO1 = GR + GT needs the whole trunk; otherwise the walk ends after the lowest wanted dense block
+  if (dx || g.want[0]) {
+    g.stop_blk = -1;
+  } else {
+    g.stop_blk = P.R + 1;
+    for (int r = 0; r < P.R; ++r)
+      if (g.any(conv_index_rdb(r, 1), conv_index_rdb(r, 5) + 1)) { g.stop_blk = r; break; }
+    if (g.stop_blk > P.R && g.any(1 + 5 * P.R, nconv)) g.stop_blk = P.R;
+  }
+  return g;
+}
+
+// layers of data-gradient chain s that a selection launches: a prefix, the chain walks from the tail down to block 0
+static int chain_layers(const b200sr_plan& P, const Step& s, const GradSelect* g) {
+  if (!g || s.needs_dx) return s.nlayers;
+  int n = 0;
+  while (n < s.nlayers && P.layer_steps[s.layer0 + n].blk >= g->stop_blk) ++n;
+  return n;
+}
+
+// whether a non-chain step of the generator backward runs under a selection (grads / dx: the caller passed those buffers; cb: a
+// bucket callback is installed, otherwise one merged unpack covers every conv)
+static bool step_selected(const Step& s, const GradSelect* g, bool grads, bool dx, bool cb) {
+  if (!g) return true;
+  switch (s.type) {
+    case ST_MEMSET: return grads || s.a.kind != RK_GRADS;
+    case ST_WGRAD: case ST_BIASGRAD: return g->any(s.wc0, s.wc1);
+    case ST_ADD: return dx || g->want[0];  // GO1 feeds conv1's weight / bias gradients and the input gradient
+    case ST_UNPACK: return cb ? g->any(s.i0, s.i1) : g->any(0, (int)g->want.size());
+    default: return true;
+  }
+}
+
+static int launch_chain(b200sr_plan& P, const Step& s, const Bases& b, cudaStream_t st);
+
+// launches the first `nlayers` layers of chain s (all of them: the chain itself)
+static int launch_chain_prefix(b200sr_plan& P, const Step& s, int nlayers, const Bases& b, cudaStream_t st) {
+  if (nlayers == s.nlayers) return launch_chain(P, s, b, st);
+  // entries go layer block by layer block, so those of a layer prefix are a prefix of the entry list (their dependencies
+  // point backwards only)
+  Step c = s;
+  c.nlayers = nlayers;
+  c.nentries = 0;
+  for (int i = 0; i < s.nentries; ++i) {
+    if (P.h_entries[s.entry0 + i].layer >= s.layer0 + nlayers) continue;
+    if (i != c.nentries) return fail(B200SR_ERR_INVALID, "internal: the entries of a chain's layer prefix are not a prefix");
+    ++c.nentries;
+  }
+  return launch_chain(P, c, b, st);
+}
+
 static int run_steps(b200sr_plan& P, std::vector<Step>& steps, const Bases& b, const void* x, int x_dtype, const int64_t* xs,
-                     b200sr_bucket_cb cb, void* user, cudaStream_t st) {
+                     b200sr_bucket_cb cb, void* user, cudaStream_t st, const GradSelect* sel = nullptr) {
   const b200sr_net_desc& d = P.d;
   // Weight-gradient launches of different dense blocks are independent of one another: once the data-gradient chain is
   // done they alternate between the caller's stream and a side stream, so the flush tail of one launch overlaps the ramp-up
@@ -1309,6 +1400,7 @@ static int run_steps(b200sr_plan& P, std::vector<Step>& steps, const Bases& b, c
   for (size_t si = 0; si < steps.size(); ++si) {
     Step& s = steps[si];
     if (s.needs_wgrad && !b.grads) continue;  // discriminator backward for the generator update: data gradients only
+    if (!step_selected(s, sel, b.grads != nullptr, b.y != nullptr, cb != nullptr)) continue;
     if (overlap_chain >= 0 && (int)si < overlap_chain && (s.type == ST_WGRAD || s.type == ST_BIASGRAD)) {
       deferred.push_back((int)si);
       continue;
@@ -1316,7 +1408,8 @@ static int run_steps(b200sr_plan& P, std::vector<Step>& steps, const Bases& b, c
     if (overlap_chain >= 0 && (int)si == overlap_chain) {
       int rc = ensure_streams(); if (rc) return rc;
       CUDA_TRY(cudaEventRecord(P.ev_fork, st));  // everything the deferred kernels read exists once the FIRST chain is done
-      rc = launch_chain(P, s, b, st);
+      const int nl = chain_layers(P, s, sel);   // 0: only tail gradients wanted, the deferred kernels run alone
+      if (nl > 0) rc = launch_chain_prefix(P, s, nl, b, st);
       if (rc) return rc;
       for (int k = 0; k < nstreams - 1; ++k) CUDA_TRY(cudaStreamWaitEvent(P.side_stream[k], P.ev_fork, 0));
       int lane = 0;
@@ -1343,7 +1436,9 @@ static int run_steps(b200sr_plan& P, std::vector<Step>& steps, const Bases& b, c
         return fail(B200SR_ERR_INVALID, "internal: unchained conv step");
       case ST_CHAIN: {
         if (s.needs_dx && !b.y) break;  // nobody asked for the input gradient
-        int rc = launch_chain(P, s, b, st);
+        const int nl = chain_layers(P, s, sel);
+        if (nl == 0) break;
+        int rc = launch_chain_prefix(P, s, nl, b, st);
         if (rc) return rc;
         forked = false;  // weight gradients behind this chain read what it produces: the side streams fork again after it
         break;
@@ -1380,6 +1475,15 @@ static int run_steps(b200sr_plan& P, std::vector<Step>& steps, const Bases& b, c
         for (int c = c0; c < c1; ++c) blocks += P.unpack_ops[c].nblocks;
         unpack_wgrad_kernel<<<blocks, 256, 0, st>>>(P.d_unpack_ops, c0, c1, (const float*)((char*)b.ws + P.o_gw), (float*)b.grads);
         CUDA_TRY(cudaGetLastError());
+        if (sel) {  // unwanted convs of a wanted dense block got gradients from its one launch: their entries are zero again
+          for (int c = c0; c < c1;) {
+            int e = c;
+            while (e < c1 && !sel->want[e] && sel->written(e)) ++e;
+            if (e == c) { ++c; continue; }
+            CUDA_TRY(cudaMemsetAsync((float*)b.grads + P.param_off[2 * c], 0, (size_t)(P.param_off[2 * e] - P.param_off[2 * c]) * 4, st));
+            c = e;
+          }
+        }
         break;
       }
       case ST_ADD: {
@@ -2112,9 +2216,56 @@ int b200sr_forward(b200sr_plan* p, const void* x, int x_dtype, const int64_t* x_
 
 int b200sr_backward(b200sr_plan* p, const float* dy, const void* packed, void* workspace, float* flat_grads, float* dx_or_null,
                     b200sr_bucket_cb cb, void* user, b200sr_stream stream) {
-  if (!p || !dy || !packed || !workspace || !flat_grads) return fail(B200SR_ERR_INVALID, "null argument");
+  if (!flat_grads) return fail(B200SR_ERR_INVALID, "null argument");
+  return b200sr_backward_select(p, dy, packed, workspace, flat_grads, dx_or_null, nullptr, cb, user, stream);
+}
+
+// mask_or_null / grads / dx as in b200sr_backward_select; *out: nullptr when everything is wanted (the full backward)
+static int select_for(const b200sr_plan* p, const uint8_t* mask, bool grads, bool dx, GradSelect* g, const GradSelect** out) {
+  const int nconv = ((int)p->param_off.size() - 1) / 2;
+  if (!grads && mask)
+    for (int c = 0; c < nconv; ++c)
+      if (mask[c]) return fail(B200SR_ERR_INVALID, "conv %d is wanted but no gradient buffer was given", c);
+  *out = nullptr;
+  if (grads && !mask) return 0;
+  if (p->is_vgg || p->is_disc) return fail(B200SR_ERR_INVALID, "a gradient selection needs a generator plan");
+  *g = make_select(*p, mask, grads, dx);
+  if (grads && std::all_of(g->want.begin(), g->want.end(), [](uint8_t w) { return w != 0; })) return 0;  // all ones = full backward
+  *out = g;
+  return 0;
+}
+
+int32_t b200sr_backward_launches(const b200sr_plan* p, const uint8_t* conv_wanted_or_null, int with_dx, int with_cb) {
+  if (!p || !p->d.training || p->is_vgg || p->is_disc) return 0;
+  GradSelect g;
+  const GradSelect* sel = nullptr;
+  select_for(p, conv_wanted_or_null, true, with_dx != 0, &g, &sel);  // cannot fail for a generator plan with a gradient buffer
+  if (sel && !with_dx && !sel->any(0, (int)sel->want.size())) return 0;
+  // counted as b200sr_num_launches counts: memsets are not launches, the unpack steps merge into one without a callback
+  int n = 0;
+  for (const Step& s : p->bwd) {
+    if (s.type == ST_MEMSET) continue;
+    if (s.type == ST_CHAIN) { n += s.needs_dx ? (with_dx != 0) : (chain_layers(*p, s, sel) > 0); continue; }
+    if (s.type == ST_UNPACK && !with_cb && s.i0 != 0) continue;
+    n += step_selected(s, sel, true, with_dx != 0, with_cb != 0);
+  }
+  return n;
+}
+
+int b200sr_backward_select(b200sr_plan* p, const float* dy, const void* packed, void* workspace, float* flat_grads_or_null,
+                           float* dx_or_null, const uint8_t* conv_wanted_or_null, b200sr_bucket_cb cb, void* user,
+                           b200sr_stream stream) {
+  if (!p || !dy || !packed || !workspace) return fail(B200SR_ERR_INVALID, "null argument");
   if (!p->d.training) return fail(B200SR_ERR_INVALID, "plan was created with training=0");
-  int rc = runtime_init();
+  GradSelect g;
+  const GradSelect* sel = nullptr;
+  int rc = select_for(p, conv_wanted_or_null, flat_grads_or_null != nullptr, dx_or_null != nullptr, &g, &sel);
+  if (rc) return rc;
+  if (sel && !dx_or_null && !sel->any(0, (int)sel->want.size())) {  // nothing to compute: every wanted entry is zero
+    if (flat_grads_or_null) CUDA_TRY(cudaMemsetAsync(flat_grads_or_null, 0, (size_t)p->param_off.back() * 4, (cudaStream_t)stream));
+    return 0;
+  }
+  rc = runtime_init();
   if (rc) return rc;
   rc = ensure_maps(*p, workspace, (void*)packed, (cudaStream_t)stream);
   if (rc) return rc;
@@ -2123,8 +2274,8 @@ int b200sr_backward(b200sr_plan* p, const float* dy, const void* packed, void* w
     CUDA_TRY(cudaMemcpyAsync(p->d_unpack_ops, p->unpack_ops.data(), p->unpack_ops.size() * sizeof(UnpackOp), cudaMemcpyHostToDevice,
                              (cudaStream_t)stream));
   }
-  Bases b{workspace, (void*)packed, dx_or_null, dy, flat_grads};
-  return run_steps(*p, p->bwd, b, nullptr, 0, nullptr, cb, user, (cudaStream_t)stream);
+  Bases b{workspace, (void*)packed, dx_or_null, dy, flat_grads_or_null};
+  return run_steps(*p, p->bwd, b, nullptr, 0, nullptr, cb, user, (cudaStream_t)stream, sel);
 }
 
 // ------------------------------------------------------------------------------------------ single-layer helpers

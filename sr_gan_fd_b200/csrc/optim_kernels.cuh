@@ -10,7 +10,7 @@ namespace b200sr {
 
 struct OptTensor {       // one parameter tensor
   float* p;
-  const float* g;
+  const float* g;         // nullptr: a frozen parameter (no gradient) -- no Adam update, the EMA still averages it
   float* m;
   float* v;
   float* ema;            // may be nullptr
@@ -36,7 +36,8 @@ __global__ void __launch_bounds__(kOptBlock) fused_adam_ema_kernel(const OptTens
   const bool skip = h.found_inf && *h.found_inf > 0.f;
   const long long b = blockIdx.x;
   const OptTensor t = tensors[h.block_tensor[b]];
-  if (skip && !t.ema) return;
+  const bool no_adam = skip || !t.g;
+  if (no_adam && !t.ema) return;
   const float tstep = *h.step + 1.f;
   const float bias_corr1 = 1.f - powf(h.beta1, tstep);
   const float bias_corr2_sqrt = sqrtf(1.f - powf(h.beta2, tstep));
@@ -44,7 +45,7 @@ __global__ void __launch_bounds__(kOptBlock) fused_adam_ema_kernel(const OptTens
   const long long base = (b - t.block0) * kOptElemsPerBlock;
   const float step_size = h.lr / bias_corr1;
   auto upd = [&](float& p, float g, float& m, float& v, float& e) {
-    if (!skip) {
+    if (!no_adam) {
       g *= inv_scale;
       if (h.weight_decay != 0.f) g = fmaf(h.weight_decay, p, g);
       m = fmaf(h.beta1, m, (1.f - h.beta1) * g);
@@ -58,7 +59,7 @@ __global__ void __launch_bounds__(kOptBlock) fused_adam_ema_kernel(const OptTens
                      reinterpret_cast<uintptr_t>(t.v) | reinterpret_cast<uintptr_t>(t.ema)) & 15) == 0;
   if (vec && i0 + 3 < t.numel) {
     float4 p = *reinterpret_cast<const float4*>(t.p + i0);
-    const float4 g = *reinterpret_cast<const float4*>(t.g + i0);
+    const float4 g = t.g ? *reinterpret_cast<const float4*>(t.g + i0) : make_float4(0.f, 0.f, 0.f, 0.f);
     float4 m = *reinterpret_cast<const float4*>(t.m + i0);
     float4 v = *reinterpret_cast<const float4*>(t.v + i0);
     float4 e = t.ema ? *reinterpret_cast<const float4*>(t.ema + i0) : make_float4(0.f, 0.f, 0.f, 0.f);
@@ -70,7 +71,7 @@ __global__ void __launch_bounds__(kOptBlock) fused_adam_ema_kernel(const OptTens
   } else {
     for (long long i = i0; i < i0 + 4 && i < t.numel; ++i) {
       float p = t.p[i], m = t.m[i], v = t.v[i], e = t.ema ? t.ema[i] : 0.f;
-      upd(p, t.g[i], m, v, e);
+      upd(p, t.g ? t.g[i] : 0.f, m, v, e);
       t.p[i] = p; t.m[i] = m; t.v[i] = v;
       if (t.ema) t.ema[i] = e;
     }

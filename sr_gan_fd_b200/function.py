@@ -43,6 +43,12 @@ class _Plan:
         self.launches_bwd = int(lib.b200sr_num_launches(handle, 1)) if training else 0
         self.launches_bwd_bucketed = int(lib.b200sr_num_launches(handle, 2)) if training else 0
 
+    def backward_launches(self, need_params=None, with_dx: bool = False, with_cb: bool = False) -> int:
+        """Kernel launches of one backward that computes the gradients of the parameters flagged in ``need_params``
+        (state_dict order; None: all of them), the input gradient if ``with_dx``, with a bucket callback if ``with_cb``."""
+        mask = conv_mask(need_params) if need_params is not None else None
+        return int(_lib.load().b200sr_backward_launches(self.handle, mask, int(with_dx), int(with_cb)))
+
     def __del__(self):
         try:
             if self.handle:
@@ -167,31 +173,48 @@ class _RRDBNetFn(torch.autograd.Function):
         if rt.pack_serial.get(ctx.pack_slot) != ctx.pack_serial:
             raise RuntimeError("generator weights were re-packed between this forward and its backward")
         dy = dy.contiguous().float()
+        need = ctx.needs_input_grad
+        need_params = need[2:]
+        all_params = all(need_params)
+        any_params = all_params or any(need_params)
         with torch.cuda.device(dy.device):
             stream = torch.cuda.current_stream().cuda_stream
-            flat = torch.empty(plan.param_numel, dtype=torch.float32, device=dy.device)  # fresh per backward
+            flat = None
+            if any_params:
+                flat = torch.empty(plan.param_numel, dtype=torch.float32, device=dy.device)  # fresh per backward
             hook = rt.grad_bucket_hook
-            if hook is not None:
+            if hook is not None and flat is not None:
                 cb = _lib.BUCKET_CB(lambda user, off, cnt: hook(flat, int(off), int(cnt)))
             else:
                 cb = _lib.BUCKET_CB()
-            need = ctx.needs_input_grad
             dx = None
             if need[1]:  # gradient w.r.t. the LR input: conv1's data gradient, fp32 NCHW (only when x.requires_grad)
                 dx = torch.empty(ctx.x_meta[0], dtype=torch.float32, device=dy.device)
-            _lib.check(lib.b200sr_backward(plan.handle, C.c_void_p(dy.data_ptr()), C.c_void_p(ctx.packed.data_ptr()),
-                                           C.c_void_p(ctx.workspace.data_ptr()), C.c_void_p(flat.data_ptr()),
-                                           C.c_void_p(dx.data_ptr()) if dx is not None else None, cb, None,
-                                           C.c_void_p(stream)))
-            if rt.grad_done_hook is not None:
+            args = (plan.handle, C.c_void_p(dy.data_ptr()), C.c_void_p(ctx.packed.data_ptr()), C.c_void_p(ctx.workspace.data_ptr()),
+                    C.c_void_p(flat.data_ptr()) if flat is not None else None, C.c_void_p(dx.data_ptr()) if dx is not None else None)
+            if all_params:
+                _lib.check(lib.b200sr_backward(*args, cb, None, C.c_void_p(stream)))
+            else:  # frozen or partially frozen generator: only what autograd asks for is computed
+                mask = conv_mask(need_params) if any_params else None
+                _lib.check(lib.b200sr_backward_select(*args, mask, cb, None, C.c_void_p(stream)))
+            if rt.grad_done_hook is not None and flat is not None:
                 rt.grad_done_hook(flat)
         ctx.workspace = None
         ctx.x_keepalive = None
         if dx is not None and ctx.x_meta[1] != torch.float32:
             dx = dx.to(ctx.x_meta[1])
+        if flat is None:
+            return (None, dx, *([None] * len(need_params)))
         pieces = flat.split(rt.param_numels)  # one call: 702 views of the flat gradient buffer, state_dict order
-        grads = [t.view(shp) if need[2 + i] else None for i, (t, shp) in enumerate(zip(pieces, rt.param_shapes))]
+        grads = [t.view(shp) if need_params[i] else None for i, (t, shp) in enumerate(zip(pieces, rt.param_shapes))]
         return (None, dx, *grads)
+
+
+def conv_mask(need_params) -> "C.Array":
+    """Per-conv byte mask of ``b200sr_backward_select`` from per-parameter flags (weight, bias pairs in state_dict order):
+    a conv is wanted when its weight or its bias is."""
+    flags = [bool(need_params[i] or need_params[i + 1]) for i in range(0, len(need_params), 2)]
+    return (C.c_uint8 * len(flags))(*flags)
 
 
 def generator_forward(module, x: torch.Tensor) -> torch.Tensor:

@@ -47,6 +47,9 @@ SIGNATURES = {
                                  C.c_void_p, C.c_void_p]),
     "b200sr_backward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, BUCKET_CB,
                                   C.c_void_p, C.c_void_p]),
+    "b200sr_backward_select": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                         C.POINTER(C.c_uint8), BUCKET_CB, C.c_void_p, C.c_void_p]),
+    "b200sr_backward_launches": (C.c_int32, [C.c_void_p, C.POINTER(C.c_uint8), C.c_int, C.c_int]),
     "b200sr_conv3x3_scratch_bytes": (C.c_size_t, [C.c_int, C.c_int]),
     "b200sr_conv3x3_fwd": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p,
                                      C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),

@@ -9,6 +9,11 @@ the EMA copy the scripts maintain with ``AveragedModel(model, avg_fn=...)`` + ``
 and cooperates with ``torch.cuda.amp.GradScaler`` (``_step_supports_amp_scaling``): unscale, non-finite skip, Adam and
 EMA are ONE kernel launch over all 702 tensors (libb200sr ``b200sr_fused_adam_ema``) instead of the foreach Adam
 kernels plus a 702-iteration Python EMA loop (~3k launches).  CUDA fp32 parameters only; no CPU fallback.
+
+Frozen parameters: a parameter whose ``.grad`` is None gets no Adam update (parameter and moments untouched, as
+``torch.optim.Adam`` skips it) and is still averaged into the EMA copy (``AveragedModel.update_parameters`` averages every
+parameter).  One limit: the Adam step counter is shared by all parameters, so a parameter that is unfrozen later takes its
+bias correction from the shared count, not from the steps it took itself.  A fixed freeze pattern matches torch exactly.
 """
 from __future__ import annotations
 
@@ -127,8 +132,9 @@ class FusedAdamEMA(torch.optim.Optimizer):
         tbl = self._tables_host[slot].numpy()
         for i, p in enumerate(self._params):
             g = p.grad
-            if g is None:
-                raise RuntimeError("FusedAdamEMA.step(): every parameter needs a gradient")
+            if g is None:  # frozen: no Adam update (null gradient pointer), the EMA still averages it
+                tbl[i, 1] = 0
+                continue
             if g.dtype != torch.float32 or not g.is_contiguous():
                 g = g.float().contiguous()
                 p.grad = g
