@@ -56,7 +56,17 @@ typedef struct b200sr_net_desc {
   int32_t grad_bucket_rrdbs; /* gradient buckets announced through b200sr_bucket_cb: RRDBs per bucket (0 = 1; the tail convs and
                               * conv1 are buckets of their own, the last trunk bucket holds at most two RRDBs so that little
                               * communication is left exposed after the last kernel) */
+  int32_t deterministic; /* 1: bit-reproducible backward (see "Deterministic plans" below); 0: the default, atomic reductions */
 } b200sr_net_desc;
+
+/* Deterministic plans (the `deterministic` member of the net, VGG and discriminator descriptors; torch.use_deterministic_algorithms).
+ * A default plan sums weight and bias gradients (and the VGG loss value) with atomics, so their order -- and the last bits --
+ * depend on CTA scheduling.  A deterministic plan gives bit-identical outputs for bit-identical inputs, for one GPU model,
+ * one library build and one plan geometry: its reductions store per-split / per-block partials into a workspace area that
+ * only deterministic plans have, and one ordered-sum launch behind each weight- or bias-gradient launch adds them in index
+ * order (b200sr_num_launches / b200sr_backward_launches count those launches).  The split counts are fixed when the plan is
+ * built.  Packing does not depend on the flag: b200sr_pack_layout_id is equal for the two modes, and one packed buffer serves both.
+ * The single-layer b200sr_conv3x3_wgrad keeps its atomic flush. */
 
 /* Called from inside b200sr_backward (on the calling host thread) each time every kernel that contributes to a
  * contiguous range [offset, offset+count) of the flat gradient buffer has been ENQUEUED on the stream: the callee
@@ -154,6 +164,11 @@ int b200sr_fused_adam_ema(const void* tensor_table, const int32_t* block_tensor,
  * ssim_map_sum[i]   = sum of the SSIM map over its (h - 2 crop - 10) x (w - 2 crop - 10) positions -> SSIM = sum / count */
 int b200sr_iqa_psnr_ssim_y(const float* raw, const float* dst, int n, int h, int w, int crop_border, const double* window11,
                            double* psnr_sqerr_sum, double* ssim_map_sum, b200sr_stream stream);
+/* The same sums, bit-reproducible: per-block partials go to scratch (device, >= b200sr_iqa_det_scratch_bytes(n, h, w) bytes for
+ * an n x h x w batch; a crop never needs more) and are added in block order. */
+size_t b200sr_iqa_det_scratch_bytes(int n, int h, int w);
+int b200sr_iqa_psnr_ssim_y_det(const float* raw, const float* dst, int n, int h, int w, int crop_border, const double* window11,
+                               double* psnr_sqerr_sum, double* ssim_map_sum, double* scratch, b200sr_stream stream);
 /* ESRGAN/imgproc.py:160-183 tensor_to_image: x [c, h, w] fp32 -> out_hwc [h, w, c] uint8 = trunc(clamp(255 x, 0, 255));
  * range_norm: x <- (x + 1) / 2 first; half: round to fp16 and multiply in fp16 as the reference does with half=True */
 int b200sr_tensor_to_image_u8(const float* x, int c, int h, int w, int range_norm, int half, uint8_t* out_hwc, b200sr_stream stream);
@@ -173,6 +188,7 @@ typedef struct b200sr_vgg_desc {
   int32_t grad_conv;            /* -1, or the conv whose L1 feature loss is differentiated w.r.t. the input images */
   int32_t grad_images;          /* images (from 0) that receive a gradient: the sr half */
   float mean[3], std[3];        /* transforms.Normalize of the input */
+  int32_t deterministic;        /* 1: b200sr_vgg_feature_l1 sums per-block partials in block order (bit-reproducible) */
 } b200sr_vgg_desc;
 int b200sr_vgg_plan_create(const b200sr_vgg_desc* desc, b200sr_plan** out);
 /* x: [batch, 3, height, width] fp32 in [0, 1] with element strides x_strides[4] */
@@ -201,6 +217,7 @@ typedef struct b200sr_disc_desc {
   int32_t training;     /* 1: build the backward schedule */
   int32_t fp16;         /* 16-bit format of the activations / packed weights / gradients: 1 = fp16 (what the reference's autocast runs
                          * this network in; needs in_channels == 3, other widths fall back to bf16), 0 = bf16 (wider range) */
+  int32_t deterministic; /* 1: bit-reproducible weight and bias gradients (see "Deterministic plans" above) */
 } b200sr_disc_desc;
 int b200sr_disc_plan_create(const b200sr_disc_desc* desc, b200sr_plan** out);
 /* x: [batch, in_channels, height, width], element strides x_strides[4], dtype per b200sr_dtype;

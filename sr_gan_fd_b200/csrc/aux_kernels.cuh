@@ -210,10 +210,13 @@ __global__ void ingest_grad_kernel(const float* __restrict__ dy, const unsigned 
 // multiples of 8 and g is 16-byte aligned.  Each thread owns EIGHT consecutive channels of a pixel row (one 16-byte load, four of
 // them in flight); pixel lanes are reduced through shared memory, one atomicAdd per channel and block.  The launch uses at most two
 // blocks per SM: those final atomics all hit the SAME few addresses and cost ~45 ns each once a thousand blocks queue up on one.
+// kDet (deterministic plans): seg[0].out is a [gridDim.x][ncols] partial-sum matrix instead; every block stores its row and
+// ordered_sum_kernel adds the rows in block order.
 struct BiasGradSeg { int col_begin, col_end; float* out; int n_valid; };
 struct BiasGradParams { const __nv_bfloat16* g; long long P; int stride; int c0; int ncols; int nseg; BiasGradSeg seg[5]; int f16; };
 constexpr int kBiasGradThreads = 256;
 
+template <bool kDet>
 __global__ void __launch_bounds__(kBiasGradThreads) bias_grad_vec_kernel(const BiasGradParams p) {
   __shared__ float red[8 * kBiasGradThreads];
   const int L = p.ncols >> 3;                 // 8-channel lanes per pixel row
@@ -261,11 +264,56 @@ __global__ void __launch_bounds__(kBiasGradThreads) bias_grad_vec_kernel(const B
 #pragma unroll
     for (int k = 0; k < 8; ++k) {
       const int c = 8 * cl + k;
-      for (int sgi = 0; sgi < p.nseg; ++sgi) {
-        const BiasGradSeg& sg = p.seg[sgi];
-        if (c >= sg.col_begin && c < sg.col_end && (c - sg.col_begin) < sg.n_valid) atomicAdd(sg.out + (c - sg.col_begin), acc[k]);
+      if constexpr (kDet) {
+        p.seg[0].out[static_cast<long long>(blockIdx.x) * p.ncols + c] = acc[k];
+      } else {
+        for (int sgi = 0; sgi < p.nseg; ++sgi) {
+          const BiasGradSeg& sg = p.seg[sgi];
+          if (c >= sg.col_begin && c < sg.col_end && (c - sg.col_begin) < sg.n_valid) atomicAdd(sg.out + (c - sg.col_begin), acc[k]);
+        }
       }
     }
+  }
+}
+
+// ------------------------------------------------------------------------------------ ordered sums (deterministic plans)
+// Every per-split / per-block partial a deterministic plan's reductions leave behind is summed here, in index order, so the
+// result does not depend on which CTA finished first.  One job, over a box of elements (i0 < n0, i1 < n1, i2 < n2, i3 < n3):
+//   dst[i0 + i1 d1 + i2 d2 + i3 d3] = sum over s < S, in order, of src[s * stride + i0 + i1 s1 + i2 s2 + i3 s3]
+// The weight-gradient jobs are boxes of [tap][co/4][ci][4] staging tensors (src: the compact copies of a pixel split); bias,
+// VGG and IQA partials are rows (n0 only).
+template <typename T>
+struct SumJob {
+  T* dst;
+  const T* src;
+  long long stride;  // between the S partials of an element
+  int S, n0, n1, n2, n3;
+  long long d1, d2, d3, s1, s2, s3;
+};
+constexpr int kMaxSumJobs = 24;
+template <typename T>
+struct SumJobs {
+  int n;
+  int block0[kMaxSumJobs + 1];  // blocks of job j: [block0[j], block0[j + 1])
+  SumJob<T> job[kMaxSumJobs];
+};
+
+template <typename T>
+__global__ void __launch_bounds__(256) ordered_sum_kernel(const __grid_constant__ SumJobs<T> J) {
+  int j = 0;
+  while (j + 1 < J.n && static_cast<int>(blockIdx.x) >= J.block0[j + 1]) ++j;
+  const SumJob<T>& b = J.job[j];
+  const unsigned total = static_cast<unsigned>(b.n0) * b.n1 * b.n2 * b.n3;
+  const unsigned step = static_cast<unsigned>(J.block0[j + 1] - J.block0[j]) * blockDim.x;
+  for (unsigned e = (blockIdx.x - J.block0[j]) * blockDim.x + threadIdx.x; e < total; e += step) {
+    unsigned r = e;
+    const unsigned i0 = r % b.n0; r /= b.n0;
+    const unsigned i1 = r % b.n1; r /= b.n1;
+    const unsigned i2 = r % b.n2, i3 = r / b.n2;
+    const long long o = i0 + i1 * b.s1 + i2 * b.s2 + i3 * b.s3;
+    T acc = b.src[o];
+    for (int s = 1; s < b.S; ++s) acc += b.src[o + s * b.stride];
+    b.dst[i0 + i1 * b.d1 + i2 * b.d2 + i3 * b.d3] = acc;
   }
 }
 

@@ -77,7 +77,8 @@ static int runtime_init() {
     CUDA_TRY(cudaFuncSetAttribute(conv3x3_chain_kernel<0, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, conv_smem_bytes(1)));
     CUDA_TRY(cudaFuncSetAttribute(conv3x3_chain_kernel<1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, conv_smem_bytes(1)));
     CUDA_TRY(cudaFuncSetAttribute(conv3x3_chain_kernel<0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, conv_smem_bytes(1)));
-    CUDA_TRY(cudaFuncSetAttribute(wgrad3x3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kWgSmemBytes));
+    CUDA_TRY(cudaFuncSetAttribute(wgrad3x3_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kWgSmemBytes));
+    CUDA_TRY(cudaFuncSetAttribute(wgrad3x3_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kWgSmemBytes));
     g_dev_attr_set[di] = true;
   }
   return 0;
@@ -142,6 +143,7 @@ struct Step {
   // bias grad
   BiasGradParams bp;
   Ref bg_g;
+  int det_blocks = 0;  // deterministic plans: blocks (= partial-sum rows) of the bias-gradient launch, fixed at plan build
   // fold / add / memset / ingest
   Ref a, b, c, d2;
   long long count = 0;
@@ -185,6 +187,8 @@ struct b200sr_plan {
                                       // per image than SMs: plain per-conv schedule
   int groups = 1;                     // image groups that flow through a chain independently
   int plan_sms = 148;                 // SM count the schedule was laid out for
+  bool det = false;                   // deterministic plan: ordered partial sums instead of atomics (b200sr.h "Deterministic plans")
+  long long o_det = 0, det_lane_bytes = 0;  // its partial-sum area: one lane of det_lane_bytes per weight-gradient stream
   // VGG19 feature plans (b200sr_vgg_plan_create): the same step / chain machinery over another layer list
   bool is_vgg = false;
   b200sr_vgg_desc vd;
@@ -326,6 +330,20 @@ static void conv_dims(const b200sr_plan& P, int ci, int* O, int* I) {
   *O = (t == P.L + 2) ? d.out_channels : d.channels;
 }
 
+// SM count of the current device, 0 without one (plans built on a machine without a GPU lay out for 148)
+static int device_sms() {
+  int dev_count = 0, sms = 0;
+  if (cudaGetDeviceCount(&dev_count) == cudaSuccess && dev_count > 0) {
+    int dev = 0;
+    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  } else {
+    cudaGetLastError();
+  }
+  return sms;
+}
+
+static void plan_deterministic(b200sr_plan& P, int lanes, int wgrad_sms);
+
 static int build_plan(b200sr_plan& P) {
   const b200sr_net_desc& d = P.d;
   if (d.channels != 64 || d.growth != 32) return fail(B200SR_ERR_INVALID, "only channels=64, growth=32 are supported (got %d, %d)", d.channels, d.growth);
@@ -338,13 +356,7 @@ static int build_plan(b200sr_plan& P) {
   {
     // Image groups: >= 2 whenever the batch allows (latency hiding between groups).  The re-associated dense block keeps
     // one work item's partial sums in a CTA's TMEM across five passes, so every group must fit one item per CTA.
-    int dev_count = 0, sms = 0;
-    if (cudaGetDeviceCount(&dev_count) == cudaSuccess && dev_count > 0) {
-      int dev = 0;
-      if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    } else {
-      cudaGetLastError();
-    }
+    const int sms = device_sms();
     if (sms > 0) P.plan_sms = sms;
     const int tpi = ((d.width + kTileW - 1) / kTileW) * ((d.height + kTileH - 1) / kTileH);  // resident 8 x 32 items per image
     P.groups = d.batch >= 2 ? 2 : 1;
@@ -1015,6 +1027,7 @@ static int build_plan(b200sr_plan& P) {
       P.bwd_overlap_chain = last;
     }
   }
+  if (P.det && train) plan_deterministic(P, 4, P.plan_sms / 2);  // run_steps: four weight-gradient streams on half the SMs each
   return 0;
 }
 
@@ -1231,15 +1244,12 @@ static int launch_chain(b200sr_plan& P, const Step& s, const Bases& b, cudaStrea
   return 0;
 }
 
-// sms_cap: SMs one wgrad wave may use (0: all)
-static int launch_wgrad(const Step& s, const CUtensorMap& tmX, const CUtensorMap& tmDY, const Bases& b, cudaStream_t st, int sms_cap) {
-  WgradBatch wb = s.wb;
-  const int sms = (sms_cap > 0 && sms_cap < g_num_sms) ? sms_cap : g_num_sms;
-  // deal the CTAs of one wave out in proportion to each problem's cost (max of tensor cycles and L2->SM bytes / 42 B per clock)
+// deal the CTAs of one wave of `sms` SMs out in proportion to each problem's cost (max of tensor cycles and L2->SM bytes / 42 B
+// per clock): sets the problems' split counts and CTA ranges
+static void wgrad_deal(WgradBatch& wb, int sms) {
   double work[kWgMaxProblems], total = 0;
   for (int j = 0; j < wb.num_problems; ++j) {
     WgradParams& wp = wb.prob[j];
-    for (int i = 0; i < wp.num_seg; ++i) wp.seg[i].out = (float*)resolve(s.wseg_out[j][i], b);
     const int nacc = wp.dy_mask ? __builtin_popcount(wp.dy_mask) : 3;
     const double mma = nacc * 8.0 * (wp.n_cols / 2.0);
     const double ld = wgrad_load_bytes(wp) / 42.0;
@@ -1258,9 +1268,144 @@ static int launch_wgrad(const Step& s, const CUtensorMap& tmX, const CUtensorMap
     ctas += splits * ntap;
   }
   wb.cta_begin[wb.num_problems] = ctas;
-  wgrad3x3_kernel<<<dim3(ctas), kWgThreads, kWgSmemBytes, st>>>(tmX, tmDY, wb);
+}
+
+// ordered_sum_kernel over a list of jobs (at most kMaxSumJobs), about 1024 elements per block
+template <typename T>
+static int launch_ordered_sum(const SumJob<T>* jobs, int n, cudaStream_t st) {
+  if (n < 1 || n > kMaxSumJobs) return fail(B200SR_ERR_INVALID, "internal: %d ordered-sum jobs", n);
+  SumJobs<T> J;
+  memset(&J, 0, sizeof(J));
+  J.n = n;
+  int blocks = 0;
+  for (int j = 0; j < n; ++j) {
+    J.job[j] = jobs[j];
+    J.block0[j] = blocks;
+    const long long total = (long long)jobs[j].n0 * jobs[j].n1 * jobs[j].n2 * jobs[j].n3;
+    if (total < 1 || total >= (1LL << 31)) return fail(B200SR_ERR_INVALID, "internal: ordered-sum job of %lld elements", total);
+    blocks += (int)std::min<long long>((total + 1023) / 1024, 1024);
+  }
+  J.block0[n] = blocks;
+  ordered_sum_kernel<T><<<blocks, 256, 0, st>>>(J);
   CUDA_TRY(cudaGetLastError());
   return 0;
+}
+// a row job: dst[i] = sum over r < rows of src[r * stride + i], i < n
+template <typename T>
+static SumJob<T> sum_rows_t(T* dst, const T* src, int rows, long long stride, int n) {
+  SumJob<T> j;
+  memset(&j, 0, sizeof(j));
+  j.dst = dst; j.src = src; j.stride = stride; j.S = rows; j.n0 = n; j.n1 = j.n2 = j.n3 = 1;
+  return j;
+}
+static SumJob<double> sum_rows(double* dst, const double* src, int rows, long long stride, int n) { return sum_rows_t(dst, src, rows, stride, n); }
+
+// Deterministic launches: the segment a split flushes into -- the part of the staging tensor that `g` of problem `wp` writes
+// (input channels [ci0, ci_total) up to two 64-row M blocks, the output channels of its columns), as a compact tensor of its own
+static WgradSegment wgrad_det_segment(const WgradParams& wp, const WgradSegment& g) {
+  WgradSegment c = g;
+  c.ci0 = 0;
+  c.ci_total = std::max(1, std::min(g.ci0 + (wp.blk[1].kind == kWgBlkIdle ? 64 : 128), g.ci_total) - g.ci0);
+  c.co_pad = std::min(g.co_pad, std::min(g.col_end, wp.n_cols) - g.col_begin);
+  return c;
+}
+// floats of one split's copy of that segment
+static long long wgrad_det_region(const WgradParams& wp, const WgradSegment& g) {
+  const WgradSegment c = wgrad_det_segment(wp, g);
+  return 9LL * c.co_pad * c.ci_total;
+}
+// first bit and length of a contiguous tap mask (0 = all three); length 0 when the bits are not contiguous
+static int tap_range(int mask, int* lo) {
+  const int m = mask ? mask : 7;
+  *lo = __builtin_ctz(m);
+  const int n = __builtin_popcount(m);
+  return (m >> *lo) == (1 << n) - 1 ? n : 0;
+}
+// bias-gradient blocks of a launch (at most two per SM: see bias_grad_vec_kernel)
+static int bias_grad_blocks(const BiasGradParams& bp, int sms) {
+  const int plv = kBiasGradThreads / (bp.ncols / 8);
+  long long blocks = (bp.P + plv * 8 - 1) / (plv * 8);
+  if (blocks > 2 * sms) blocks = 2 * sms;
+  return (int)blocks;
+}
+
+// Deterministic plans: the split counts of every weight-gradient launch are dealt once, here, for `wgrad_sms` SMs (what
+// run_steps gives one launch), and the workspace gains one partial-sum lane per weight-gradient stream, sized for the largest
+// launch.  A launch and its ordered sum run on one stream, so the lane is reused in stream order.
+static void plan_deterministic(b200sr_plan& P, int lanes, int wgrad_sms) {
+  long long lane = 0;
+  for (Step& s : P.bwd) {
+    long long bytes = 0;
+    if (s.type == ST_WGRAD) {
+      wgrad_deal(s.wb, wgrad_sms);
+      for (int j = 0; j < s.wb.num_problems; ++j)
+        for (int i = 0; i < s.wb.prob[j].num_seg; ++i) bytes += 4LL * s.wb.prob[j].splits * wgrad_det_region(s.wb.prob[j], s.wb.prob[j].seg[i]);
+    } else if (s.type == ST_BIASGRAD) {
+      s.det_blocks = bias_grad_blocks(s.bp, P.plan_sms);
+      bytes = 4LL * s.det_blocks * s.bp.ncols;
+    }
+    lane = std::max(lane, bytes);
+  }
+  P.det_lane_bytes = align_up(lane, 1024);
+  P.o_det = align_up(P.ws_bytes, 1024);
+  P.ws_bytes = P.o_det + lanes * P.det_lane_bytes;
+}
+
+// sms_cap: SMs one wgrad wave may use (0: all).  slab: the partial-sum lane of the stream (deterministic plans), else nullptr
+static int launch_wgrad(const Step& s, const CUtensorMap& tmX, const CUtensorMap& tmDY, const Bases& b, cudaStream_t st, int sms_cap,
+                        char* slab = nullptr) {
+  WgradBatch wb = s.wb;
+  for (int j = 0; j < wb.num_problems; ++j)
+    for (int i = 0; i < wb.prob[j].num_seg; ++i) wb.prob[j].seg[i].out = (float*)resolve(s.wseg_out[j][i], b);
+  if (!slab) {
+    wgrad_deal(wb, (sms_cap > 0 && sms_cap < g_num_sms) ? sms_cap : g_num_sms);
+    wgrad3x3_kernel<false><<<dim3(wb.cta_begin[wb.num_problems]), kWgThreads, kWgSmemBytes, st>>>(tmX, tmDY, wb);
+    CUDA_TRY(cudaGetLastError());
+    return 0;
+  }
+  // deterministic: the splits dealt at plan build; every segment flushes into its own slab (one compact copy per split), and one job
+  // per M block adds the split copies over exactly the box of the staging tensor that block writes (taps x channel quads x channels)
+  SumJob<float> jobs[kMaxSumJobs];
+  int nj = 0;
+  long long off = 0;
+  for (int j = 0; j < wb.num_problems; ++j) {
+    WgradParams& wp = wb.prob[j];
+    for (int i = 0; i < wp.num_seg; ++i) {
+      const WgradSegment g = wp.seg[i];  // the staging tensor's view
+      WgradSegment& c = wp.seg[i];       // the slab's
+      c = wgrad_det_segment(wp, g);
+      c.out = (float*)slab + off;
+      off += wp.splits * wgrad_det_region(wp, g);
+      for (int bk = 0; bk < 2; ++bk) {
+        const int kind = wp.blk[bk].kind;
+        if (kind == kWgBlkIdle || (g.blk_mask && !((g.blk_mask >> bk) & 1))) continue;
+        const bool ones = kind == kWgBlkOnes;
+        const int ci_lo = g.ci0 + (ones ? 0 : wp.blk[bk].c0 - wp.blk[0].c0);
+        const int ci_hi = std::min(ci_lo + 64, g.ci_total);
+        const int ncq = std::min(std::min(g.col_end, wp.n_cols) - g.col_begin, g.co_pad) / 4;
+        if (ci_lo >= ci_hi || ncq < 1) continue;
+        int dy_lo = 0, dx_lo = 0, ndy = 1, ndx = 1;
+        if (!ones) {
+          ndy = tap_range(wp.dy_mask, &dy_lo);
+          if (wp.blk[bk].dx >= 0) dx_lo = wp.blk[bk].dx;
+          else ndx = tap_range(wp.dx_mask, &dx_lo);
+        }
+        if (!ndy || !ndx || nj == kMaxSumJobs) return fail(B200SR_ERR_INVALID, "internal: deterministic wgrad launch not expressible as boxes");
+        const long long tap_d = (long long)(g.co_pad / 4) * g.ci_total * 4, tap_s = (long long)(c.co_pad / 4) * c.ci_total * 4;
+        const int tap0 = dy_lo * 3 + dx_lo;
+        SumJob<float>& jb = jobs[nj++];
+        jb.dst = g.out + tap0 * tap_d + ci_lo * 4LL;
+        jb.src = c.out + tap0 * tap_s + (ci_lo - g.ci0) * 4LL;
+        jb.stride = 9LL * c.co_pad * c.ci_total; jb.S = wp.splits;
+        jb.n0 = (ci_hi - ci_lo) * 4; jb.n1 = ncq; jb.n2 = ndx; jb.n3 = ndy;
+        jb.d1 = g.ci_total * 4LL; jb.d2 = tap_d; jb.d3 = 3 * tap_d;
+        jb.s1 = c.ci_total * 4LL; jb.s2 = tap_s; jb.s3 = 3 * tap_s;
+      }
+    }
+  }
+  wgrad3x3_kernel<true><<<dim3(wb.cta_begin[wb.num_problems]), kWgThreads, kWgSmemBytes, st>>>(tmX, tmDY, wb);
+  CUDA_TRY(cudaGetLastError());
+  return launch_ordered_sum(jobs, nj, st);
 }
 
 // What a selective generator backward (b200sr_backward_select) computes.  Chosen per call: the plan and its step list serve
@@ -1377,7 +1522,9 @@ static int run_steps(b200sr_plan& P, std::vector<Step>& steps, const Bases& b, c
     }
     return 0;
   };
-  auto do_biasgrad = [&](const Step& s, cudaStream_t bs) -> int {
+  // deterministic plans: partial-sum lane k belongs to weight-gradient stream k (0: the caller's stream, k: side_stream[k - 1])
+  auto lane_of = [&](int k) -> char* { return P.det ? (char*)b.ws + P.o_det + k * P.det_lane_bytes : nullptr; };
+  auto do_biasgrad = [&](const Step& s, cudaStream_t bs, char* slab) -> int {
     BiasGradParams bp = s.bp;
     bp.g = (const __nv_bfloat16*)resolve(s.bg_g, b);
     for (int i = 0; i < bp.nseg; ++i) bp.seg[i].out = (float*)resolve(s.seg_out[i], b);
@@ -1386,12 +1533,25 @@ static int run_steps(b200sr_plan& P, std::vector<Step>& steps, const Bases& b, c
         (reinterpret_cast<uintptr_t>(bp.g) & 15) != 0)
       return fail(B200SR_ERR_INVALID, "internal: bias-gradient step with ncols %d, c0 %d, stride %d is not 16-byte vectorisable",
                   bp.ncols, bp.c0, bp.stride);
-    const int plv = kBiasGradThreads / (bp.ncols / 8);
-    long long blocks = (bp.P + plv * 8 - 1) / (plv * 8);
-    if (blocks > 2 * g_num_sms) blocks = 2 * g_num_sms;
-    bias_grad_vec_kernel<<<(int)blocks, kBiasGradThreads, 0, bs>>>(bp);
+    if (!slab) {
+      bias_grad_vec_kernel<false><<<bias_grad_blocks(bp, g_num_sms), kBiasGradThreads, 0, bs>>>(bp);
+      CUDA_TRY(cudaGetLastError());
+      return 0;
+    }
+    // deterministic: the block rows [block][ncols] are summed row by row; the segments must split the columns into equal parts
+    // that all go to one output (the four phases of an upsample conv's bias), so the rows are [block][segment][width]
+    const int wd = bp.seg[0].col_end - bp.seg[0].col_begin;
+    for (int i = 0; i < bp.nseg; ++i)
+      if (bp.seg[i].col_begin != i * wd || bp.seg[i].col_end != (i + 1) * wd || bp.seg[i].out != bp.seg[0].out ||
+          bp.seg[i].n_valid != bp.seg[0].n_valid)
+        return fail(B200SR_ERR_INVALID, "internal: bias-gradient segments are not equal column groups of one output");
+    if (bp.nseg * wd != bp.ncols) return fail(B200SR_ERR_INVALID, "internal: bias-gradient segments do not cover the columns");
+    float* out = bp.seg[0].out;
+    bp.seg[0].out = (float*)slab;
+    bias_grad_vec_kernel<true><<<s.det_blocks, kBiasGradThreads, 0, bs>>>(bp);
     CUDA_TRY(cudaGetLastError());
-    return 0;
+    const SumJob<float> j = sum_rows_t(out, (const float*)slab, s.det_blocks * bp.nseg, wd, bp.seg[0].n_valid);
+    return launch_ordered_sum(&j, 1, bs);
   };
   // Weight / bias gradients that sit between two data-gradient chains (the HR tail's, see build_plan) are DEFERRED behind the launch of
   // the second chain and go to the side streams only: the trunk chain, enqueued first, takes its SMs, they fill the rest and run beside it.
@@ -1414,9 +1574,11 @@ static int run_steps(b200sr_plan& P, std::vector<Step>& steps, const Bases& b, c
       for (int k = 0; k < nstreams - 1; ++k) CUDA_TRY(cudaStreamWaitEvent(P.side_stream[k], P.ev_fork, 0));
       int lane = 0;
       for (int di : deferred) {
-        cudaStream_t ds = P.side_stream[lane++ % (nstreams - 1)];
-        if (steps[di].type == ST_WGRAD) rc = launch_wgrad(steps[di], P.maps()[steps[di].xmap], P.maps()[steps[di].dymap], b, ds, wgrad_cap);
-        else rc = do_biasgrad(steps[di], ds);
+        const int k = lane++ % (nstreams - 1);
+        cudaStream_t ds = P.side_stream[k];
+        if (steps[di].type == ST_WGRAD)
+          rc = launch_wgrad(steps[di], P.maps()[steps[di].xmap], P.maps()[steps[di].dymap], b, ds, wgrad_cap, lane_of(k + 1));
+        else rc = do_biasgrad(steps[di], ds, lane_of(k + 1));
         if (rc) return rc;
       }
       side_dirty = true;
@@ -1445,6 +1607,7 @@ static int run_steps(b200sr_plan& P, std::vector<Step>& steps, const Bases& b, c
       }
       case ST_WGRAD: {
         cudaStream_t ws = st;
+        int lane_ = 0;
         if (alternate) {
           { int rc = ensure_streams(); if (rc) return rc; }
           if (!forked) {  // the side stream starts after everything enqueued so far (the data-gradient chain)
@@ -1452,15 +1615,15 @@ static int run_steps(b200sr_plan& P, std::vector<Step>& steps, const Bases& b, c
             for (int k = 0; k < nstreams - 1; ++k) CUDA_TRY(cudaStreamWaitEvent(P.side_stream[k], P.ev_fork, 0));
             forked = true;
           }
-          const int lane_ = wcount++ % nstreams;
+          lane_ = wcount++ % nstreams;
           if (lane_ > 0) { ws = P.side_stream[lane_ - 1]; side_dirty = true; }
         }
-        int rc = launch_wgrad(s, P.maps()[s.xmap], P.maps()[s.dymap], b, ws, wgrad_cap);
+        int rc = launch_wgrad(s, P.maps()[s.xmap], P.maps()[s.dymap], b, ws, wgrad_cap, lane_of(lane_));
         if (rc) return rc;
         break;
       }
       case ST_BIASGRAD: {
-        int rc = do_biasgrad(s, st);
+        int rc = do_biasgrad(s, st, lane_of(0));
         if (rc) return rc;
         break;
       }
@@ -1658,6 +1821,7 @@ static int build_vgg_plan(b200sr_plan& P) {
       if (kVggPoolAfter[l] && l + 1 <= v.grad_conv) o_gpool[l] = B.alloc((long long)NB * (P.vgg_h[l] >> 1) * (P.vgg_w[l] >> 1) * kVggCout[l] * 2);
     }
   }
+  if (P.det) P.o_det = B.alloc(kVggL1MaxBlocks * sizeof(double));  // per-block partials of b200sr_vgg_feature_l1
   P.ws_bytes = B.cursor;
   auto packed_bias = [&](long long off_floats) { Ref r; r.kind = RK_PACKED; r.off = -1 - off_floats; return r; };
   auto conv_step = [&](int amap, const ConvParams& cp) {
@@ -2060,6 +2224,11 @@ static int build_disc_plan(b200sr_plan& P) {
     vv.swap(out);
   };
   chainify(P.fwd); chainify(P.bwd);
+  if (P.det && train) {
+    const int sms = device_sms();
+    if (sms > 0) P.plan_sms = sms;
+    plan_deterministic(P, 2, P.plan_sms);  // run_steps: two weight-gradient streams on all SMs
+  }
   return 0;
 }
 
@@ -2067,7 +2236,7 @@ static int build_disc_plan(b200sr_plan& P) {
 extern "C" {
 
 const char* b200sr_last_error(void) { return g_err; }
-int b200sr_version(void) { return 100; }
+int b200sr_version(void) { return 101; }
 void b200sr_debug_set(int flags) { g_debug = flags; }
 int b200sr_debug_read_profile(unsigned long long* out_host, int n) {
   CUDA_TRY(cudaMemcpyFromSymbol(out_host, g_conv_prof, sizeof(unsigned long long) * (size_t)n));
@@ -2085,6 +2254,7 @@ int b200sr_plan_create(const b200sr_net_desc* desc, b200sr_plan** out) {
   if (!desc || !out) return fail(B200SR_ERR_INVALID, "null argument");
   b200sr_plan* p = new b200sr_plan();
   p->d = *desc;
+  p->det = desc->deterministic != 0;
   if (const char* e = getenv("B200SR_REASSOC")) p->reassoc = atoi(e) != 0;  // 0: per-conv schedule everywhere
   p->tail_f16 = desc->training == 0;  // training: the L1 loss' sign(sr - gt) amplifies the fp16 rounding of the tail past the 1e-2 gradient bar
   if (const char* e = getenv("B200SR_TAIL_FP16")) p->tail_f16 = atoi(e) != 0;  // 0: split-precision bf16 tail everywhere, 1: fp16 tail everywhere
@@ -2167,13 +2337,19 @@ double b200sr_flops(const b200sr_plan* p, int backward) {
   return total;
 }
 
+// ordered-sum launches behind a step (deterministic plans: one per weight- or bias-gradient launch)
+static int det_sums(const b200sr_plan& P, const Step& s) { return P.det && (s.type == ST_WGRAD || s.type == ST_BIASGRAD) ? 1 : 0; }
+
 int32_t b200sr_num_launches(const b200sr_plan* p, int backward) {
   if (!p) return 0;
   const std::vector<Step>& v = backward ? p->bwd : p->fwd;
   // kernel launches of one pass.  backward = 1: no gradient-bucket callback, the per-bucket unpack steps collapse into one
   // launch; backward = 2: with a callback (data-parallel training), one unpack launch per bucket.
   int n = 0, unpacks = 0;
-  for (const Step& s : v) { n += (s.type != ST_MEMSET && !s.needs_dx); unpacks += (s.type == ST_UNPACK); }
+  for (const Step& s : v) {
+    n += (s.type != ST_MEMSET && !s.needs_dx) + det_sums(*p, s);
+    unpacks += (s.type == ST_UNPACK);
+  }
   if (backward == 1 && unpacks > 1) n -= unpacks - 1;
   return n;
 }
@@ -2247,7 +2423,7 @@ int32_t b200sr_backward_launches(const b200sr_plan* p, const uint8_t* conv_wante
     if (s.type == ST_MEMSET) continue;
     if (s.type == ST_CHAIN) { n += s.needs_dx ? (with_dx != 0) : (chain_layers(*p, s, sel) > 0); continue; }
     if (s.type == ST_UNPACK && !with_cb && s.i0 != 0) continue;
-    n += step_selected(s, sel, true, with_dx != 0, with_cb != 0);
+    n += step_selected(s, sel, true, with_dx != 0, with_cb != 0) * (1 + det_sums(*p, s));
   }
   return n;
 }
@@ -2398,7 +2574,7 @@ int b200sr_conv3x3_wgrad(const void* x, int n, int h, int w_, int cin, int x_str
   if (splits > wb.num_tiles) splits = wb.num_tiles;
   wp.splits = splits;
   wb.cta_begin[0] = 0; wb.cta_begin[1] = splits * 3;
-  wgrad3x3_kernel<<<dim3(splits * 3), kWgThreads, kWgSmemBytes, st>>>(tmX, tmDY, wb);
+  wgrad3x3_kernel<false><<<dim3(splits * 3), kWgThreads, kWgSmemBytes, st>>>(tmX, tmDY, wb);
   CUDA_TRY(cudaGetLastError());
   UnpackOp u;
   u.src_off = 0; u.dst_off = 0; u.co = cout; u.ci = cin; u.co_pad = cout; u.fold = 0; u.block0 = 0;
@@ -2427,30 +2603,70 @@ int b200sr_fused_adam_ema(const void* tensor_table, const int32_t* block_tensor,
 }
 
 // ------------------------------------------------------------------------------------------------ evaluation epilogue
-int b200sr_iqa_psnr_ssim_y(const float* raw, const float* dst, int n, int h, int w, int crop_border, const double* window11,
-                           double* psnr_sqerr_sum, double* ssim_map_sum, b200sr_stream stream) {
+// blocks of the two IQA launches for an n x hc x wc cropped batch (fixed by the shape)
+static long long iqa_psnr_blocks(int hc, int wc) { return std::min<long long>(((long long)hc * wc + 255) / 256, 1024); }
+static dim3 iqa_ssim_grid(int n, int hc, int wc) { return dim3((unsigned)((wc - 10 + 15) / 16), (unsigned)((hc - 10 + 15) / 16), (unsigned)n); }
+
+static int iqa_sums(const float* raw, const float* dst, int n, int h, int w, int crop_border, const double* window11,
+                    double* psnr_sqerr_sum, double* ssim_map_sum, double* det_scratch, cudaStream_t st) {
   if (!raw || !dst || !window11 || (!psnr_sqerr_sum && !ssim_map_sum)) return fail(B200SR_ERR_INVALID, "null argument");
   if (n < 1 || crop_border < 0 || h - 2 * crop_border < 11 || w - 2 * crop_border < 11)
     return fail(B200SR_ERR_INVALID, "frame %dx%d with crop %d is smaller than the 11x11 SSIM window", h, w, crop_border);
-  cudaStream_t st = (cudaStream_t)stream;
   IqaParams p;
   p.raw = raw; p.dst = dst; p.N = n; p.H = h; p.W = w; p.crop = crop_border;
   for (int i = 0; i < 11; ++i) p.win[i] = window11[i];
   p.psnr_sum = psnr_sqerr_sum; p.ssim_sum = ssim_map_sum;
   const int hc = h - 2 * crop_border, wc = w - 2 * crop_border;
+  const long long pblocks = iqa_psnr_blocks(hc, wc);
+  const dim3 sgrid = iqa_ssim_grid(n, hc, wc);
+  if (det_scratch) {
+    // deterministic: [blocks][n] partial sums of each launch, then one ordered sum per metric
+    SumJob<double> jobs[2];
+    int nj = 0;
+    double* part = det_scratch;
+    if (psnr_sqerr_sum) {
+      p.psnr_sum = part;
+      iqa_psnr_y_kernel<true><<<dim3((unsigned)pblocks, (unsigned)n), 256, 0, st>>>(p);
+      CUDA_TRY(cudaGetLastError());
+      jobs[nj++] = sum_rows(psnr_sqerr_sum, part, (int)pblocks, n, n);
+      part += pblocks * n;
+    }
+    if (ssim_map_sum) {
+      p.ssim_sum = part;
+      iqa_ssim_y_kernel<true><<<sgrid, dim3(16, 16), 0, st>>>(p);
+      CUDA_TRY(cudaGetLastError());
+      jobs[nj++] = sum_rows(ssim_map_sum, part, (int)(sgrid.x * sgrid.y), n, n);
+    }
+    return launch_ordered_sum(jobs, nj, st);
+  }
   if (psnr_sqerr_sum) {
     CUDA_TRY(cudaMemsetAsync(psnr_sqerr_sum, 0, sizeof(double) * n, st));
-    long long blocks = ((long long)hc * wc + 255) / 256;
-    if (blocks > 1024) blocks = 1024;
-    iqa_psnr_y_kernel<<<dim3((unsigned)blocks, (unsigned)n), 256, 0, st>>>(p);
+    iqa_psnr_y_kernel<false><<<dim3((unsigned)pblocks, (unsigned)n), 256, 0, st>>>(p);
     CUDA_TRY(cudaGetLastError());
   }
   if (ssim_map_sum) {
     CUDA_TRY(cudaMemsetAsync(ssim_map_sum, 0, sizeof(double) * n, st));
-    iqa_ssim_y_kernel<<<dim3((unsigned)((wc - 10 + 15) / 16), (unsigned)((hc - 10 + 15) / 16), (unsigned)n), dim3(16, 16), 0, st>>>(p);
+    iqa_ssim_y_kernel<false><<<sgrid, dim3(16, 16), 0, st>>>(p);
     CUDA_TRY(cudaGetLastError());
   }
   return 0;
+}
+
+int b200sr_iqa_psnr_ssim_y(const float* raw, const float* dst, int n, int h, int w, int crop_border, const double* window11,
+                           double* psnr_sqerr_sum, double* ssim_map_sum, b200sr_stream stream) {
+  return iqa_sums(raw, dst, n, h, w, crop_border, window11, psnr_sqerr_sum, ssim_map_sum, nullptr, (cudaStream_t)stream);
+}
+
+size_t b200sr_iqa_det_scratch_bytes(int n, int h, int w) {
+  if (n < 1 || h < 11 || w < 11) return 0;
+  const dim3 g = iqa_ssim_grid(n, h, w);
+  return sizeof(double) * (size_t)n * (size_t)(iqa_psnr_blocks(h, w) + (long long)g.x * g.y);
+}
+
+int b200sr_iqa_psnr_ssim_y_det(const float* raw, const float* dst, int n, int h, int w, int crop_border, const double* window11,
+                               double* psnr_sqerr_sum, double* ssim_map_sum, double* scratch, b200sr_stream stream) {
+  if (!scratch) return fail(B200SR_ERR_INVALID, "null argument");
+  return iqa_sums(raw, dst, n, h, w, crop_border, window11, psnr_sqerr_sum, ssim_map_sum, scratch, (cudaStream_t)stream);
 }
 
 int b200sr_tensor_to_image_u8(const float* x, int c, int h, int w, int range_norm, int half, uint8_t* out_hwc, b200sr_stream stream) {
@@ -2467,6 +2683,7 @@ int b200sr_disc_plan_create(const b200sr_disc_desc* desc, b200sr_plan** out) {
   if (!desc || !out) return fail(B200SR_ERR_INVALID, "null argument");
   b200sr_plan* p = new b200sr_plan();
   p->dd = *desc;
+  p->det = desc->deterministic != 0;
   int rc = build_disc_plan(*p);
   if (rc) { delete p; return rc; }
   *out = p;
@@ -2506,6 +2723,7 @@ int b200sr_vgg_plan_create(const b200sr_vgg_desc* desc, b200sr_plan** out) {
   if (!desc || !out) return fail(B200SR_ERR_INVALID, "null argument");
   b200sr_plan* p = new b200sr_plan();
   p->vd = *desc;
+  p->det = desc->deterministic != 0;
   int rc = build_vgg_plan(*p);
   if (rc) { delete p; return rc; }
   *out = p;
@@ -2528,10 +2746,18 @@ int b200sr_vgg_feature_l1(b200sr_plan* p, const void* workspace, int conv_index,
   if (2 * pairs != p->vd.batch) return fail(B200SR_ERR_INVALID, "pairs must be half of the plan's batch");
   const long long half = (long long)pairs * p->vgg_h[conv_index] * p->vgg_w[conv_index] * kVggCout[conv_index];
   cudaStream_t st = (cudaStream_t)stream;
-  CUDA_TRY(cudaMemsetAsync(out_sum, 0, sizeof(double), st));
   long long blocks = (half / 4 + 255) / 256;
-  if (blocks > 8 * 148) blocks = 8 * 148;
-  vgg_l1_pair_sum_kernel<<<(unsigned)blocks, 256, 0, st>>>((const float*)((const char*)workspace + p->o_vgg_feat[conv_index] - 1), half, out_sum);
+  if (blocks > kVggL1MaxBlocks) blocks = kVggL1MaxBlocks;
+  const float* f = (const float*)((const char*)workspace + p->o_vgg_feat[conv_index] - 1);
+  if (p->det) {
+    double* partial = (double*)((char*)const_cast<void*>(workspace) + p->o_det);
+    vgg_l1_pair_sum_kernel<true><<<(unsigned)blocks, 256, 0, st>>>(f, half, partial);
+    CUDA_TRY(cudaGetLastError());
+    SumJob<double> j = sum_rows(out_sum, partial, (int)blocks, 1, 1);
+    return launch_ordered_sum(&j, 1, st);
+  }
+  CUDA_TRY(cudaMemsetAsync(out_sum, 0, sizeof(double), st));
+  vgg_l1_pair_sum_kernel<false><<<(unsigned)blocks, 256, 0, st>>>(f, half, out_sum);
   CUDA_TRY(cudaGetLastError());
   return 0;
 }

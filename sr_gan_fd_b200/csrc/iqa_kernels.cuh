@@ -38,7 +38,8 @@ __device__ __forceinline__ double iqa_block_sum(double v, double* red) {
   return s;  // valid in thread 0
 }
 
-// grid (blocks, N), block (256, 1)
+// grid (blocks, N), block (256, 1).  kDet: psnr_sum is a [blocks][N] partial-sum matrix (ordered_sum_kernel adds the rows)
+template <bool kDet>
 __global__ void __launch_bounds__(256) iqa_psnr_y_kernel(const IqaParams p) {
   __shared__ double red[8];
   const int n = blockIdx.y;
@@ -55,10 +56,15 @@ __global__ void __launch_bounds__(256) iqa_psnr_y_kernel(const IqaParams p) {
     acc += e * e;
   }
   const double s = iqa_block_sum(acc, red);
-  if (threadIdx.x == 0) atomicAdd(p.psnr_sum + n, s);
+  if (threadIdx.x == 0) {
+    if constexpr (kDet) p.psnr_sum[static_cast<long long>(blockIdx.x) * p.N + n] = s;
+    else atomicAdd(p.psnr_sum + n, s);
+  }
 }
 
-// grid (ceil(Wo / 16), ceil(Ho / 16), N), block (16, 16); Wo = W - 2 crop - 10
+// grid (ceil(Wo / 16), ceil(Ho / 16), N), block (16, 16); Wo = W - 2 crop - 10.  kDet: ssim_sum is a [blocks][N] partial-sum
+// matrix, block = blockIdx.y * gridDim.x + blockIdx.x
+template <bool kDet>
 __global__ void __launch_bounds__(256) iqa_ssim_y_kernel(const IqaParams p) {
   __shared__ double yr[26][26], yd[26][26];
   __shared__ double hq[5][26][16];
@@ -109,7 +115,10 @@ __global__ void __launch_bounds__(256) iqa_ssim_y_kernel(const IqaParams p) {
     val = ((2 * m_r * m_d + c1) * (2 * cov + c2)) / ((m_r * m_r + m_d * m_d + c1) * (v_r + v_d + c2));
   }
   const double s = iqa_block_sum(val, red);
-  if (t == 0) atomicAdd(p.ssim_sum + n, s);
+  if (t == 0) {
+    if constexpr (kDet) p.ssim_sum[(static_cast<long long>(blockIdx.y) * gridDim.x + blockIdx.x) * p.N + n] = s;
+    else atomicAdd(p.ssim_sum + n, s);
+  }
 }
 
 // x: [C, H, W] fp32 (C <= 4) -> out [H, W, C] uint8 = trunc(clamp(255 x, 0, 255)); half: round to fp16 and multiply in fp16 first

@@ -103,7 +103,11 @@ __global__ void vgg_maxpool_relu_bwd_kernel(const __nv_bfloat16* __restrict__ ac
   }
 }
 
-// sum over the first `half` elements of |f[i] - f[i + half]| (fp32 features of the sr images followed by those of the gt images)
+constexpr int kVggL1MaxBlocks = 8 * 148;  // grid cap of vgg_l1_pair_sum_kernel (a constant: the grid depends on the shape only)
+
+// sum over the first `half` elements of |f[i] - f[i + half]| (fp32 features of the sr images followed by those of the gt images).
+// kDet: out[blockIdx.x] = this block's partial sum (ordered_sum_kernel adds them) instead of an atomicAdd into out[0]
+template <bool kDet>
 __global__ void __launch_bounds__(256) vgg_l1_pair_sum_kernel(const float* __restrict__ f, long long half, double* __restrict__ out) {
   __shared__ double red[8];
   double acc = 0.0;
@@ -118,7 +122,10 @@ __global__ void __launch_bounds__(256) vgg_l1_pair_sum_kernel(const float* __res
   if (threadIdx.x < 8) {
     double s = red[threadIdx.x];
     for (int o = 4; o > 0; o >>= 1) s += __shfl_xor_sync(0xffu, s, o);
-    if (threadIdx.x == 0) atomicAdd(out, s);
+    if (threadIdx.x == 0) {
+      if constexpr (kDet) out[blockIdx.x] = s;
+      else atomicAdd(out, s);
+    }
   }
 }
 

@@ -11,6 +11,9 @@
 // ("re-associated by input slice").  The accumulators (3 x N <= 480 TMEM columns) live in TMEM for the whole
 // pixel loop and are flushed once with 16-byte vector reductions (red.global.add.v4.f32) into a [tap][co/4][ci][4]
 // fp32 staging tensor; a small unpack kernel transposes that to the OIHW gradient layout per gradient bucket.
+// kDet (deterministic plans): the flush stores instead, into one copy per pixel split of the part of the staging tensor the segment
+// writes (the host hands the kernel a segment that describes that compact [tap][co/4][ci][4] copy: `out` is the slab, split s at
+// s * 9 * co_pad * ci_total floats), and ordered_sum_kernel adds the copies in split order.
 //
 // One launch carries a BATCH of up to five such problems over the same two tensor maps (the five problems of a dense
 // block), with the CTAs dealt out in proportion to each problem's cost so the whole dense block is one balanced wave.
@@ -97,6 +100,7 @@ __host__ inline void wgrad_set_a(WgradParams& p, int a_c0, int a_blocks) {
 }
 constexpr int kWgSmemBytes = 227 * 1024;
 
+template <bool kDet>
 __global__ void __launch_bounds__(kWgThreads, 1)
 wgrad3x3_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmDY,
                 const __grid_constant__ WgradBatch batch) {
@@ -236,11 +240,17 @@ wgrad3x3_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
         const int ci = sg.ci0 + m;
         if (c0 >= sg.col_begin && c0 < sg.col_end && ci < sg.ci_total && (!sg.blk_mask || ((sg.blk_mask >> b) & 1))) {
           float* dst = sg.out + ((static_cast<long long>(tap) * (sg.co_pad >> 2) + (co >> 2)) * sg.ci_total + ci) * 4;
+          if constexpr (kDet) dst += static_cast<long long>(split) * 9 * sg.co_pad * sg.ci_total;
 #pragma unroll
           for (int j = 0; j < 4; ++j)
-            if (co + 4 * j < sg.co_pad)
-              red_add_v4_f32(dst + static_cast<long long>(j) * sg.ci_total * 4, __uint_as_float(r[4 * j]), __uint_as_float(r[4 * j + 1]),
-                             __uint_as_float(r[4 * j + 2]), __uint_as_float(r[4 * j + 3]));
+            if (co + 4 * j < sg.co_pad) {
+              if constexpr (kDet)
+                *reinterpret_cast<float4*>(dst + static_cast<long long>(j) * sg.ci_total * 4) =
+                    make_float4(__uint_as_float(r[4 * j]), __uint_as_float(r[4 * j + 1]), __uint_as_float(r[4 * j + 2]), __uint_as_float(r[4 * j + 3]));
+              else
+                red_add_v4_f32(dst + static_cast<long long>(j) * sg.ci_total * 4, __uint_as_float(r[4 * j]), __uint_as_float(r[4 * j + 1]),
+                               __uint_as_float(r[4 * j + 2]), __uint_as_float(r[4 * j + 3]));
+            }
         }
       }
     }

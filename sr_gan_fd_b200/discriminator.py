@@ -39,13 +39,15 @@ _MAX_PLANS = 6
 
 class _DiscPlan:
     def __init__(self, in_channels: int, out_channels: int, channels: int, batch: int, height: int, width: int, training: bool,
-                 fp16: bool = True) -> None:
+                 fp16: bool = True, deterministic: bool = False) -> None:
         lib = _lib.load()
-        d = _lib.DiscDesc(in_channels, out_channels, channels, batch, height, width, 1 if training else 0, 1 if fp16 else 0)
+        d = _lib.DiscDesc(in_channels, out_channels, channels, batch, height, width, 1 if training else 0, 1 if fp16 else 0,
+                          1 if deterministic else 0)
         handle = C.c_void_p()
         _lib.check(lib.b200sr_disc_plan_create(C.byref(d), C.byref(handle)))
         self.handle = handle
         self.training = training
+        self.deterministic = deterministic
         self.out_channels = out_channels
         self.workspace_bytes = int(lib.b200sr_workspace_bytes(handle))
         self.packed_bytes = int(lib.b200sr_packed_bytes(handle))
@@ -72,10 +74,11 @@ class _DiscRuntime:
 
     def plan(self, module, device, batch, height, width, training) -> _DiscPlan:
         fp16 = module.operand_dtype == "fp16"
-        key = (device.index, batch, height, width, training, fp16)
+        det = _lib.deterministic()  # the backward runs in the forward's mode
+        key = (device.index, batch, height, width, training, fp16, det)
         p = self.plans.get(key)
         if p is None:
-            p = _DiscPlan(module._in_channels, module._out_channels, module._channels, batch, height, width, training, fp16)
+            p = _DiscPlan(module._in_channels, module._out_channels, module._channels, batch, height, width, training, fp16, det)
             self.plans[key] = p
             while len(self.plans) > _MAX_PLANS:
                 self.plans.popitem(last=False)

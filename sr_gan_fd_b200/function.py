@@ -21,14 +21,17 @@ _MAX_PACKED = 4  # packed-weight buffers kept per module ((training, pack layout
 
 
 class _Plan:
-    def __init__(self, desc: dict, batch: int, height: int, width: int, training: bool, grad_bucket_rrdbs: int = 0) -> None:
+    def __init__(self, desc: dict, batch: int, height: int, width: int, training: bool, grad_bucket_rrdbs: int = 0,
+                 deterministic: bool = False) -> None:
         lib = _lib.load()
         nd = _lib.NetDesc(desc["in_channels"], desc["out_channels"], desc["channels"], desc["growth"],
-                          desc["num_blocks"], desc["n_up"], batch, height, width, 1 if training else 0, grad_bucket_rrdbs)
+                          desc["num_blocks"], desc["n_up"], batch, height, width, 1 if training else 0, grad_bucket_rrdbs,
+                          1 if deterministic else 0)
         handle = C.c_void_p()
         _lib.check(lib.b200sr_plan_create(C.byref(nd), C.byref(handle)))
         self.handle = handle
         self.training = training
+        self.deterministic = deterministic
         self.geometry = (batch, height, width)
         self.scale = 1 << desc["n_up"]
         self.out_channels = desc["out_channels"]
@@ -80,11 +83,12 @@ class GeneratorRuntime:
         self.param_numels = None
         self.cur_key = None
 
-    def plan(self, desc: dict, device: torch.device, batch: int, height: int, width: int, training: bool) -> _Plan:
-        key = (device.index, batch, height, width, training, self.grad_bucket_rrdbs)
+    def plan(self, desc: dict, device: torch.device, batch: int, height: int, width: int, training: bool,
+             deterministic: bool = False) -> _Plan:
+        key = (device.index, batch, height, width, training, self.grad_bucket_rrdbs, deterministic)
         p = self.plans.get(key)
         if p is None:
-            p = _Plan(desc, batch, height, width, training, self.grad_bucket_rrdbs)
+            p = _Plan(desc, batch, height, width, training, self.grad_bucket_rrdbs, deterministic)
             self.plans[key] = p
             while len(self.plans) > _MAX_PLANS:
                 self.plans.popitem(last=False)
@@ -134,7 +138,7 @@ def _launch_forward(module, rt: "GeneratorRuntime", x: torch.Tensor, training: b
     st = _Launched()
     with torch.cuda.device(x.device):
         stream = torch.cuda.current_stream().cuda_stream
-        plan = rt.plan(desc, x.device, n, h, w, training)
+        plan = rt.plan(desc, x.device, n, h, w, training, _lib.deterministic())  # the backward runs in the forward's mode
         packed = rt.packed_weights(plan, params, stream, rt.cur_key)
         workspace = torch.empty(plan.workspace_bytes, dtype=torch.uint8, device=x.device)
         y = torch.empty((n, plan.out_channels, h * plan.scale, w * plan.scale), dtype=torch.float32, device=x.device)

@@ -62,11 +62,16 @@ def _native_sums(raw, dst, crop_border, win, want_psnr, want_ssim):
     n, _, h, w = raw.shape
     out = torch.empty((2, n), dtype=torch.float64, device=raw.device)
     arr = (C.c_double * 11)(*[float(v) for v in win])
+    lib = _lib.load()
     with torch.cuda.device(raw.device):
         stream = torch.cuda.current_stream().cuda_stream
-        _lib.check(_lib.load().b200sr_iqa_psnr_ssim_y(
-            C.c_void_p(raw.data_ptr()), C.c_void_p(dst.data_ptr()), n, h, w, crop_border, arr,
-            C.c_void_p(out[0].data_ptr()) if want_psnr else None, C.c_void_p(out[1].data_ptr()) if want_ssim else None, C.c_void_p(stream)))
+        args = (C.c_void_p(raw.data_ptr()), C.c_void_p(dst.data_ptr()), n, h, w, crop_border, arr,
+                C.c_void_p(out[0].data_ptr()) if want_psnr else None, C.c_void_p(out[1].data_ptr()) if want_ssim else None)
+        if _lib.deterministic():  # per-block partials summed in block order instead of atomics
+            scratch = torch.empty(int(lib.b200sr_iqa_det_scratch_bytes(n, h, w)), dtype=torch.uint8, device=raw.device)
+            _lib.check(lib.b200sr_iqa_psnr_ssim_y_det(*args, C.c_void_p(scratch.data_ptr()), C.c_void_p(stream)))
+        else:
+            _lib.check(lib.b200sr_iqa_psnr_ssim_y(*args, C.c_void_p(stream)))
     return out
 
 

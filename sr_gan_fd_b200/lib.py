@@ -16,16 +16,17 @@ BUCKET_CB = C.CFUNCTYPE(None, C.c_void_p, C.c_int64, C.c_int64)
 class NetDesc(C.Structure):
     _fields_ = [(n, C.c_int32) for n in (
         "in_channels", "out_channels", "channels", "growth", "num_blocks", "n_up",
-        "batch", "height", "width", "training", "grad_bucket_rrdbs")]
+        "batch", "height", "width", "training", "grad_bucket_rrdbs", "deterministic")]
 
 
 class VggDesc(C.Structure):
     _fields_ = [(n, C.c_int32) for n in ("batch", "height", "width", "last_conv", "feat_mask", "grad_conv", "grad_images")] + \
-               [("mean", C.c_float * 3), ("std", C.c_float * 3)]
+               [("mean", C.c_float * 3), ("std", C.c_float * 3), ("deterministic", C.c_int32)]
 
 
 class DiscDesc(C.Structure):
-    _fields_ = [(n, C.c_int32) for n in ("in_channels", "out_channels", "channels", "batch", "height", "width", "training", "fp16")]
+    _fields_ = [(n, C.c_int32) for n in ("in_channels", "out_channels", "channels", "batch", "height", "width", "training", "fp16",
+                                         "deterministic")]
 
 
 _lock = threading.Lock()
@@ -62,6 +63,9 @@ SIGNATURES = {
                                         C.c_float, C.c_void_p, C.c_float, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "b200sr_iqa_psnr_ssim_y": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_double), C.c_void_p,
                                          C.c_void_p, C.c_void_p]),
+    "b200sr_iqa_det_scratch_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
+    "b200sr_iqa_psnr_ssim_y_det": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_double),
+                                             C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "b200sr_tensor_to_image_u8": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "b200sr_vgg_plan_create": (C.c_int, [C.POINTER(VggDesc), C.POINTER(C.c_void_p)]),
     "b200sr_vgg_forward": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(C.c_int64), C.c_void_p, C.c_void_p, C.c_void_p]),
@@ -98,6 +102,13 @@ def load() -> C.CDLL:
             fn.argtypes = args
         _lib = lib
         return lib
+
+
+def deterministic() -> bool:
+    """Whether the native calls run in deterministic mode: ``torch.use_deterministic_algorithms(True)`` (with or without
+    ``warn_only``) is in effect.  Read on every call; the plans of the two modes are cached side by side."""
+    import torch
+    return torch.are_deterministic_algorithms_enabled()
 
 
 def check(rc: int) -> None:

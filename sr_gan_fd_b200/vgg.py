@@ -56,11 +56,12 @@ class _VggRuntime:
         self.plans = {}
         self.packed = {}
 
-    def plan(self, batch, h, w, last_conv, feat_mask, grad_conv, grad_images, mean, std):
-        key = (batch, h, w, last_conv, feat_mask, grad_conv, grad_images)
+    def plan(self, batch, h, w, last_conv, feat_mask, grad_conv, grad_images, mean, std, deterministic=False):
+        key = (batch, h, w, last_conv, feat_mask, grad_conv, grad_images, deterministic)
         p = self.plans.get(key)
         if p is None:
-            d = _lib.VggDesc(batch, h, w, last_conv, feat_mask, grad_conv, grad_images, (C.c_float * 3)(*mean), (C.c_float * 3)(*std))
+            d = _lib.VggDesc(batch, h, w, last_conv, feat_mask, grad_conv, grad_images, (C.c_float * 3)(*mean), (C.c_float * 3)(*std),
+                             1 if deterministic else 0)
             handle = C.c_void_p()
             lib = _lib.load()
             _lib.check(lib.b200sr_vgg_plan_create(C.byref(d), C.byref(handle)))
@@ -154,7 +155,8 @@ class _ContentLossBase(nn.Module):
         lib = _lib.load()
         with torch.cuda.device(sr.device):
             stream = torch.cuda.current_stream().cuda_stream
-            plan = rt.plan(2 * pairs, h, w, max(convs), mask, grad_conv, pairs if grad_conv >= 0 else 0, self._mean, self._std)
+            plan = rt.plan(2 * pairs, h, w, max(convs), mask, grad_conv, pairs if grad_conv >= 0 else 0, self._mean, self._std,
+                           _lib.deterministic())
             packed = rt.packed_for(plan, params, stream)
             ws = torch.empty(plan["ws_bytes"], dtype=torch.uint8, device=sr.device)
             strides = (C.c_int64 * 4)(*x.stride())

@@ -163,7 +163,12 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--batch", type=int, default=16)
     ap.add_argument("--lr-size", type=int, default=64)
+    ap.add_argument("--deterministic", action="store_true",
+                    help="torch.use_deterministic_algorithms(True): bit-reproducible steps (needs CUBLAS_WORKSPACE_CONFIG=:4096:8)")
     args = ap.parse_args()
+    if args.deterministic:
+        os.environ.setdefault("CUBLAS_WORKSPACE_CONFIG", ":4096:8")  # torch's own cuBLAS calls (spectral norm) demand it
+        torch.use_deterministic_algorithms(True)
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -209,7 +214,7 @@ def main():
         print(json.dumps({
             "metric": "BSRGAN full GAN step imgs/s (BASELINE configs[4]: generator fwd+bwd + reference U-Net discriminator x3 + VGG19 content loss)",
             "generator": args.generator, "content_loss": args.content, "discriminator": args.disc, "optimizer": args.optim, "ema": bool(args.ema), "value": world * args.batch / (ms * 1e-3), "unit": "img/s", "n_gpus": world, "steps": args.steps,
-            "warmup": args.warmup, "ms_per_step": ms, "higher_is_better": True, "scaling": "weak", "data": "synthetic",
+            "warmup": args.warmup, "ms_per_step": ms, "deterministic": bool(args.deterministic), "higher_is_better": True, "scaling": "weak", "data": "synthetic",
             "config": {"batch_per_gpu": args.batch, "lr": args.lr_size, "scale": 4, "num_rrdb": 23, "critics": "reference DiscriminatorUNet(3,1,64) "
                        "+ ContentLoss on a SEEDED RANDOM-INIT VGG19 (ImageNet weights unavailable offline), autocast fp16 + GradScaler",
                        "discriminator_parallelism": "stock DDP" if world > 1 else "single", "g_loss": float(g_loss), "d_loss": float(d_loss)}}), flush=True)
