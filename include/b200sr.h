@@ -59,6 +59,17 @@ typedef struct b200sr_net_desc {
   int32_t deterministic; /* 1: bit-reproducible backward (see "Deterministic plans" below); 0: the default, atomic reductions */
 } b200sr_net_desc;
 
+/* Trunk plans (b200sr_trunk_plan_create): the stack of num_blocks RRDBs without conv1, the long skip and the tail -- what
+ * nn.Sequential(*RRDBs) computes, for generators that keep the RRDB trunk and change everything around it.  The descriptor is the
+ * generator's; a trunk plan requires n_up == 0 and in_channels == out_channels == channels == 64.  Every other entry point of a
+ * generator plan works on it, with these shapes:
+ *   x      [batch, 64, height, width], f32 / f16 / bf16, element strides x_strides[4] (NCHW or channels_last);
+ *   y      [batch, 64, height, width] fp32 contiguous, NOT clamped;
+ *   dy, dx [batch, 64, height, width] fp32 contiguous (dx: the gradient w.r.t. the trunk input);
+ *   params 2 x 5 x 3 x num_blocks pointers, the convs in the Sequential's state_dict order (0.rdb1.conv1.weight, 0.rdb1.conv1.bias, ...);
+ *   conv_wanted_or_null  5 x 3 x num_blocks bytes, same order.
+ * The trunk kernels are the generator's: for the same input, a trunk plan's y is bit for bit the generator's trunk output. */
+
 /* Deterministic plans (the `deterministic` member of the net, VGG and discriminator descriptors; torch.use_deterministic_algorithms).
  * A default plan sums weight and bias gradients (and the VGG loss value) with atomics, so their order -- and the last bits --
  * depend on CTA scheduling.  A deterministic plan gives bit-identical outputs for bit-identical inputs, for one GPU model,
@@ -74,6 +85,7 @@ typedef struct b200sr_net_desc {
 typedef void (*b200sr_bucket_cb)(void* user, int64_t offset, int64_t count);
 
 int b200sr_plan_create(const b200sr_net_desc* desc, b200sr_plan** out);
+int b200sr_trunk_plan_create(const b200sr_net_desc* desc, b200sr_plan** out); /* see "Trunk plans" above */
 void b200sr_plan_destroy(b200sr_plan* plan);
 
 /* sizes (bytes) of the caller-allocated buffers */
@@ -245,7 +257,8 @@ int b200sr_debug_read_profile(unsigned long long* out_host, int n);
  * does not have.  Discriminator plans name every tensor they keep: the ingested input "xin", the forward activations
  * "T0u" "T1u" "T2u" "T3" "B1" "A1" "B2" "A2" "B3" "A3" "S3" "A4" "A5" and, in training plans, the backward gradients "DYP" "G5"
  * "G4" "GS3" "G3" "GB3" "GS2" "GA2" "GB2" "GS1" "GA1" "GB1" "GT3" "GT2" "GT1" "G0" (build_disc_plan in b200sr.cu says what each
- * holds).  Generator plans name theirs too (build_plan in b200sr.cu): "xin", the fp32 carriers "T0" "TR" "C1" "C2" (tile-blocked),
+ * holds).  Generator plans name theirs too (build_plan in b200sr.cu; trunk plans only "TR" "C1" "C2", the "D" buffers and, in training
+ * plans, "GR" "GC1" "GC2" and the "DYB" buffers): "xin", the fp32 carriers "T0" "TR" "C1" "C2" (tile-blocked),
  * the dense-block buffers "D0" ... "D{R-1}" (R = 3 * num_blocks; inference plans keep only the ping-pong pair "D0" "D1"), the
  * tail activations "SPLT" "SPL0" ... "SPL{n_up}" "SPLC" and, in training plans, "CMASK" "DYP" "G3" "GU1" ... "GU{n_up}" "GT" "GTB"
  * "GR" "GC1" "GC2" "GO1" "DYB0" ... "DYB{R-1}".  VGG plans name none. */

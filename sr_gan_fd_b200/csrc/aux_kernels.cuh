@@ -414,4 +414,62 @@ __global__ void add_carriers_to_bf16_kernel(const float* __restrict__ a, const f
   *reinterpret_cast<uint2*>(o) = pk;
 }
 
+// ------------------------------------------------------------------------------------------------ trunk plans: both ends
+// One thread per slot (tile, half, pixel m) of the tile-blocked carrier layout above, so that consecutive threads touch consecutive
+// 16-byte carrier chunks (and, for NCHW tensors, consecutive x); padded slots outside the image are skipped -- the conv epilogues
+// never read them.  Launch: one 256-thread block per 8 x 32 tile.
+__device__ __forceinline__ bool trunk_slot(int N, int H, int W, int tiles_x, int tiles_y, long long& slot, int& n, int& y, int& x) {
+  slot = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;  // (tile * 2 + half) * 128 + m
+  const int m = static_cast<int>(slot & 127), half = static_cast<int>((slot >> 7) & 1);
+  const long long tile = slot >> 8;
+  const int tpi = tiles_x * tiles_y;
+  n = static_cast<int>(tile / tpi);
+  const int t2 = static_cast<int>(tile - static_cast<long long>(n) * tpi);
+  const int ty = t2 / tiles_x;
+  x = (t2 - ty * tiles_x) * 8 + (m & 7);
+  y = ty * 32 + half * 16 + (m >> 3);
+  return n < N && x < W && y < H;
+}
+
+// x: [N, 64, H, W], any strides, fp32 / fp16 / bf16 -> carrier (fp32, exact) and shadow[pixel][shadow_stride] channels [0, 64) =
+// bf16(scale * x).  With scale 1 this is what conv1's epilogue leaves for the trunk (T0 / TR and D0), with scale 0.04 what conv2's
+// data-gradient epilogue leaves (GR and dY5 of the last dense block).
+template <typename T>
+__global__ void __launch_bounds__(256) trunk_ingest_kernel(const T* __restrict__ x, long long sn, long long sc, long long sh, long long sw,
+                                                           int N, int H, int W, int tiles_x, int tiles_y, float scale,
+                                                           float* __restrict__ carrier, __nv_bfloat16* __restrict__ shadow, int shadow_stride) {
+  long long slot;
+  int n, y, xx;
+  if (!trunk_slot(N, H, W, tiles_x, tiles_y, slot, n, y, xx)) return;
+  const T* src = x + n * sn + y * sh + xx * sw;
+  float4* cp = reinterpret_cast<float4*>(carrier) + (slot >> 7) * 16 * 128 + (slot & 127);
+  uint4* sp = reinterpret_cast<uint4*>(shadow + ((static_cast<long long>(n) * H + y) * W + xx) * shadow_stride);
+#pragma unroll
+  for (int c8 = 0; c8 < 8; ++c8) {
+    float v[8];
+#pragma unroll
+    for (int k = 0; k < 8; ++k) v[k] = static_cast<float>(src[(8 * c8 + k) * sc]);
+    cp[(2 * c8) * 128] = make_float4(v[0], v[1], v[2], v[3]);
+    cp[(2 * c8 + 1) * 128] = make_float4(v[4], v[5], v[6], v[7]);
+    sp[c8] = make_uint4(pack_bf16x2(scale * v[0], scale * v[1]), pack_bf16x2(scale * v[2], scale * v[3]),
+                        pack_bf16x2(scale * v[4], scale * v[5]), pack_bf16x2(scale * v[6], scale * v[7]));
+  }
+}
+
+// carrier (fp32 tile-blocked) -> out [N, 64, H, W] fp32 contiguous: the trunk output y, or the trunk-input gradient dx
+__global__ void __launch_bounds__(256) trunk_export_kernel(const float* __restrict__ carrier, float* __restrict__ out, int N, int H, int W,
+                                                           int tiles_x, int tiles_y) {
+  long long slot;
+  int n, y, x;
+  if (!trunk_slot(N, H, W, tiles_x, tiles_y, slot, n, y, x)) return;
+  const float4* cp = reinterpret_cast<const float4*>(carrier) + (slot >> 7) * 16 * 128 + (slot & 127);
+  const long long plane = static_cast<long long>(H) * W;
+  float* o = out + static_cast<long long>(n) * 64 * plane + static_cast<long long>(y) * W + x;
+#pragma unroll
+  for (int q = 0; q < 16; ++q) {
+    const float4 v = cp[q * 128];
+    o[(4 * q) * plane] = v.x; o[(4 * q + 1) * plane] = v.y; o[(4 * q + 2) * plane] = v.z; o[(4 * q + 3) * plane] = v.w;
+  }
+}
+
 }  // namespace b200sr

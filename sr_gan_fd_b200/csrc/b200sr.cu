@@ -122,7 +122,8 @@ struct Bases { void* ws; void* packed; void* y; const void* dy; void* grads; };
 
 enum StepType { ST_CONV, ST_CHAIN, ST_WGRAD, ST_BIASGRAD, ST_UNPACK, ST_ADD, ST_MEMSET, ST_INGEST_X, ST_INGEST_DY,
                 ST_VGG_INGEST, ST_VGG_POOL, ST_VGG_POOL_BWD,
-                ST_DISC_UP, ST_DISC_UP_BWD, ST_DISC_ADD, ST_DISC_MASK, ST_DISC_INGEST_DY, ST_DISC_UNPACK };
+                ST_DISC_UP, ST_DISC_UP_BWD, ST_DISC_ADD, ST_DISC_MASK, ST_DISC_INGEST_DY, ST_DISC_UNPACK,
+                ST_TRUNK_INGEST, ST_TRUNK_EXPORT };
 
 struct Step {
   int type = ST_CONV;
@@ -148,6 +149,7 @@ struct Step {
   Ref a, b, c, d2;
   long long count = 0;
   int i0 = 0, i1 = 0;
+  float scale = 1.f;  // ST_TRUNK_INGEST: factor of the bf16 shadow
   // gradient-bucket announcement after this step
   long long cb_off = 0, cb_count = 0;
   bool needs_dx = false;  // only launched when the caller asks for the gradient w.r.t. the LR input
@@ -162,6 +164,8 @@ struct b200sr_plan {
   b200sr_net_desc d;
   int R = 0;  // dense blocks
   int L = 0;  // upsample stages
+  bool trunk = false;  // trunk plan (b200sr.h "Trunk plans"): the dense blocks alone, no conv1 / long skip / tail
+  int t0 = 1;          // state_dict conv index of the first trunk conv (0 in trunk plans)
   int xin_stride = 64;
   long long ws_bytes = 0;
   long long total_rows = 0, bias_floats = 0, packed_bytes = 0;
@@ -313,14 +317,14 @@ PackSeg nseg(int n0, int nlen, int k0, int klen, int w_index, int O, int I, int 
 }  // namespace
 
 // conv index helpers (state_dict order)
-static int conv_index_rdb(int r, int k /*1..5*/) { return 1 + r * 5 + (k - 1); }
+static int conv_index_rdb(const b200sr_plan& P, int r, int k /*1..5*/) { return P.t0 + r * 5 + (k - 1); }
 
 static void conv_dims(const b200sr_plan& P, int ci, int* O, int* I) {
   const b200sr_net_desc& d = P.d;
   const int ntrunk = P.R * 5;
-  if (ci == 0) { *O = d.channels; *I = d.in_channels; return; }
-  if (ci <= ntrunk) {
-    const int k = (ci - 1) % 5 + 1;
+  if (ci < P.t0) { *O = d.channels; *I = d.in_channels; return; }
+  if (ci < P.t0 + ntrunk) {
+    const int k = (ci - P.t0) % 5 + 1;
     *O = (k < 5) ? d.growth : d.channels;
     *I = d.channels + d.growth * (k - 1);
     return;
@@ -348,11 +352,15 @@ static int build_plan(b200sr_plan& P) {
   const b200sr_net_desc& d = P.d;
   if (d.channels != 64 || d.growth != 32) return fail(B200SR_ERR_INVALID, "only channels=64, growth=32 are supported (got %d, %d)", d.channels, d.growth);
   if (d.in_channels < 1 || d.in_channels > 64) return fail(B200SR_ERR_INVALID, "in_channels must be in [1,64]");
-  if (d.out_channels < 1 || d.out_channels > 16) return fail(B200SR_ERR_INVALID, "out_channels must be in [1,16]");
+  if ((d.out_channels < 1 || d.out_channels > 16) && !P.trunk) return fail(B200SR_ERR_INVALID, "out_channels must be in [1,16]");
   if (d.num_blocks < 1 || d.n_up < 0 || d.n_up > 3) return fail(B200SR_ERR_INVALID, "bad num_blocks / n_up");
   if (d.batch < 1 || d.height < 1 || d.width < 1) return fail(B200SR_ERR_INVALID, "bad geometry");
+  if (P.trunk && (d.n_up != 0 || d.in_channels != 64 || d.out_channels != 64))
+    return fail(B200SR_ERR_INVALID, "a trunk plan needs n_up = 0 and in_channels = out_channels = 64 (got %d, %d, %d)", d.n_up,
+                d.in_channels, d.out_channels);
   P.R = 3 * d.num_blocks;
   P.L = d.n_up;
+  P.t0 = P.trunk ? 0 : 1;
   {
     // Image groups: >= 2 whenever the batch allows (latency hiding between groups).  The re-associated dense block keeps
     // one work item's partial sums in a CTA's TMEM across five passes, so every group must fit one item per CTA.
@@ -370,8 +378,9 @@ static int build_plan(b200sr_plan& P) {
   const bool train = d.training != 0;
   const int N = d.batch, H = d.height, W = d.width;
   const long long Ppix = (long long)N * H * W;
-  const int nconv = 1 + R * 5 + 1 + L + 2;
-  const int ci_conv2 = 1 + R * 5, ci_up1 = ci_conv2 + 1, ci_conv3 = ci_conv2 + 1 + L, ci_conv4 = ci_conv3 + 1;
+  const bool trunk = P.trunk;
+  const int nconv = trunk ? R * 5 : 1 + R * 5 + 1 + L + 2;
+  const int ci_conv2 = 1 + R * 5, ci_up1 = ci_conv2 + 1, ci_conv3 = ci_conv2 + 1 + L, ci_conv4 = ci_conv3 + 1;  // (generator plans)
 
   // flat parameter offsets
   P.param_off.assign(2 * nconv + 1, 0);
@@ -390,11 +399,12 @@ static int build_plan(b200sr_plan& P) {
 
   Builder B(P);
   P.xin_stride = (int)align_up(3 * d.in_channels, 64);
-  // ---- workspace layout
-  P.o_xin = B.alloc("xin", Ppix * P.xin_stride * 2);
+  // ---- workspace layout (trunk plans keep only what the dense blocks read and write: the carriers TR / C1 / C2, the D buffers and,
+  // for the backward, GR / GC1 / GC2, the DYB buffers and the weight-gradient staging)
+  if (!trunk) P.o_xin = B.alloc("xin", Ppix * P.xin_stride * 2);
   // fp32 carriers: tile-blocked layout over the LR lattice's 8 x 32 tiles (padded to whole tiles)
   const long long carrier_bytes = (long long)N * ((W + kTileW - 1) / kTileW) * ((H + kTileH - 1) / kTileH) * kCarrierBytesPerTile;
-  P.o_t0 = B.alloc("T0", carrier_bytes);
+  if (!trunk) P.o_t0 = B.alloc("T0", carrier_bytes);
   P.o_tr = B.alloc("TR", carrier_bytes);
   P.o_c1 = B.alloc("C1", carrier_bytes);
   P.o_c2 = B.alloc("C2", carrier_bytes);
@@ -405,14 +415,18 @@ static int build_plan(b200sr_plan& P) {
   // the bf16 output gradients -- tcgen05 kind::f16 takes ONE 16-bit format for both operands, and the gradients stay bf16 for range)
   const bool tf16 = P.tail_f16;
   const int ts = (tf16 && !train) ? 64 : 128;  // channels per pixel of the tail activation buffers
-  P.o_splt = B.alloc("SPLT", Ppix * ts * 2);
-  for (int l = 0; l <= L; ++l) P.o_spl.push_back(B.alloc("SPL" + std::to_string(l), (Ppix << (2 * l)) * ts * 2));
-  P.o_splc = B.alloc("SPLC", (Ppix << (2 * L)) * ts * 2);
+  if (!trunk) {
+    P.o_splt = B.alloc("SPLT", Ppix * ts * 2);
+    for (int l = 0; l <= L; ++l) P.o_spl.push_back(B.alloc("SPL" + std::to_string(l), (Ppix << (2 * l)) * ts * 2));
+    P.o_splc = B.alloc("SPLC", (Ppix << (2 * L)) * ts * 2);
+  }
   const long long HRpix = Ppix << (2 * L);
   if (train) {
-    P.o_cmask = B.alloc("CMASK", HRpix * d.out_channels);
-    P.o_dyp = B.alloc("DYP", HRpix * 64 * 2);
-    P.o_g3 = B.alloc("G3", HRpix * 64 * 2);
+    if (!trunk) {
+      P.o_cmask = B.alloc("CMASK", HRpix * d.out_channels);
+      P.o_dyp = B.alloc("DYP", HRpix * 64 * 2);
+      P.o_g3 = B.alloc("G3", HRpix * 64 * 2);
+    }
     P.o_gu.assign(L + 1, 0);
     for (int l = 1; l <= L; ++l) P.o_gu[l] = B.alloc("GU" + std::to_string(l), (Ppix << (2 * (l - 1))) * 256 * 2);
     {
@@ -436,12 +450,14 @@ static int build_plan(b200sr_plan& P) {
       P.o_gw = B.alloc(off * 4);
       P.gw_bytes = off * 4;
     }
-    P.o_gt = B.alloc("GT", carrier_bytes);
-    P.o_gtb = B.alloc("GTB", Ppix * 64 * 2);
+    if (!trunk) {
+      P.o_gt = B.alloc("GT", carrier_bytes);
+      P.o_gtb = B.alloc("GTB", Ppix * 64 * 2);
+    }
     P.o_gr = B.alloc("GR", carrier_bytes);
     P.o_gc1 = B.alloc("GC1", carrier_bytes);
     P.o_gc2 = B.alloc("GC2", carrier_bytes);
-    P.o_go1 = B.alloc("GO1", Ppix * 64 * 2);
+    if (!trunk) P.o_go1 = B.alloc("GO1", Ppix * 64 * 2);
     P.o_dyb.assign(R, 0);
     for (size_t i = 0; i < P.o_dyb.size(); ++i) P.o_dyb[i] = B.alloc("DYB" + std::to_string(i), Ppix * 192 * 2);
   }
@@ -461,12 +477,15 @@ static int build_plan(b200sr_plan& P) {
   auto packed_bias = [&](long long off_floats) { Ref r; r.kind = RK_PACKED; r.off = -1 - off_floats; return r; };  // fixed up later
 
   // ================================================================ forward ================================================================
-  {
+  if (trunk) {  // the trunk input takes the place of conv1's output: fp32 carrier TR and its bf16 shadow in D0
+    Step s; s.type = ST_TRUNK_INGEST; s.a = ws(P.o_tr); s.c = ws(dense_off(0)); s.b.kind = RK_NULL;
+    P.fwd.push_back(s);
+  } else {
     Step s; s.type = ST_INGEST_X;
     P.fwd.push_back(s);
   }
   // conv1: [hi|lo|hi] input, weights [w_hi|w_hi|w_lo]
-  {
+  if (!trunk) {
     const int C = d.in_channels;
     PackOp op; memset(&op, 0, sizeof(op));
     op.n_total = 64; op.n_valid = 64; op.num_chunks = P.xin_stride / 64; op.mode = kPackFwd; op.nseg = 3;
@@ -497,7 +516,7 @@ static int build_plan(b200sr_plan& P) {
       s.of = ws(cout_c);
       if (r < R - 1) {
         s.ob = ws(dense_off(r + 1)); s.cp.epi.ob_stride = 192; s.cp.epi.ob_coff = 0;
-      } else {
+      } else if (!trunk) {  // (trunk plans: nothing reads a bf16 copy of the trunk output, the epilogue skips the store)
         s.ob = ws(P.o_splt); s.cp.epi.ob_stride = ts; s.cp.epi.ob_coff = 0; s.cp.epi.split_off = (ts == 128) ? 64 : 0;
         s.cp.epi.f16 = tf16;  // (only the STORE format: this layer's own operands are the trunk's bf16, mma_f16 stays 0)
       }
@@ -512,7 +531,7 @@ static int build_plan(b200sr_plan& P) {
       // FILLER layers without epilogue -- F1 = x (emitted after pass 2), F2 = o1|o2 (after pass 3) -- which the MMA warp
       // works off while the other image group's next pass waits for its cross-CTA dependency.  Only the o3|o4 share (K = 64)
       // and the epilogue are left for the block's last layer.
-      const int ci5 = conv_index_rdb(r, 5);
+      const int ci5 = conv_index_rdb(P, r, 5);
       auto conv5_piece = [&](int k0, int klen, bool first, bool last) {
         PackOp op; memset(&op, 0, sizeof(op));
         op.n_total = 64; op.n_cols = 64; op.n_valid = 64; op.num_chunks = 1; op.mode = kPackFwd; op.nseg = 1;
@@ -535,12 +554,12 @@ static int build_plan(b200sr_plan& P) {
         op.n_total = ncols; op.n_cols = ncols; op.n_valid = ncols; op.num_chunks = 1; op.mode = kPackFwd; op.nseg = 0;
         op.k32 = (klen == 32) ? 1 : 0;  // K = 32 pass layers carry 64-byte weight rows
         for (int k = q + 1; k <= 4; ++k)
-          op.seg[op.nseg++] = nseg(32 * (k - 1) - col_lo, 32, 0, klen, 2 * conv_index_rdb(r, k), 32, 64 + 32 * (k - 1), 0, c_q);
+          op.seg[op.nseg++] = nseg(32 * (k - 1) - col_lo, 32, 0, klen, 2 * conv_index_rdb(P, r, k), 32, 64 + 32 * (k - 1), 0, c_q);
         const int row0 = B.add_pack(op);
         ConvParams cp = base_conv_params(N, H, W, 1, klen / 16, c_q, 1 << 20, row0, ncols, ncols, op.k32);
         cp.acc_col0 = col_lo; cp.acc_first = (q == 0); cp.acc_hold = 1; cp.epi_cols = 32;
         Step s = conv_step(B.add_map(D, c_q + klen, 192, N, H, W, kABoxRows), cp, 1);
-        s.bias = packed_bias(B.add_bias(32, 2 * conv_index_rdb(r, q + 1) + 1, 32, 0));
+        s.bias = packed_bias(B.add_bias(32, 2 * conv_index_rdb(P, r, q + 1) + 1, 32, 0));
         s.cp.epi.act = 1;
         s.ob = ws(D); s.cp.epi.ob_stride = 192; s.cp.epi.ob_coff = 64 + 32 * q;
         P.fwd.push_back(s);
@@ -551,7 +570,7 @@ static int build_plan(b200sr_plan& P) {
       continue;
     }
     for (int k = 1; k <= 5; ++k) {
-      const int ci = conv_index_rdb(r, k);
+      const int ci = conv_index_rdb(P, r, k);
       const int cin = 64 + 32 * (k - 1), cout = (k < 5) ? 32 : 64;
       PackOp op; memset(&op, 0, sizeof(op));
       op.n_total = cout; op.n_valid = cout; op.num_chunks = (cin + 63) / 64; op.mode = kPackFwd; op.nseg = 1;
@@ -588,51 +607,56 @@ static int build_plan(b200sr_plan& P) {
     op.seg[2] = seg(128, 64, 2 * ci, O, I, 0, 0, 1);
     return B.add_pack(op);
   };
-  // conv2 (+ long skip)
-  {
-    const int row0 = split_pack(ci_conv2, 64, 64, kPackFwd);
-    ConvParams cp = base_conv_params(N, H, W, tch, 4, 0, twrap, row0, 64, 64);
-    Step s = conv_step(B.add_map(P.o_splt, tvalid, ts, N, H, W, kABoxRows), cp, 1);
-    s.bias = packed_bias(B.add_bias(64, 2 * ci_conv2 + 1, 64, 0));
-    s.r1 = ws(P.o_t0);
-    s.ob = ws(P.o_spl[0]); s.cp.epi.ob_stride = ts; s.cp.epi.split_off = tsplit; s.cp.epi.f16 = tf16; s.cp.mma_f16 = tf16;
-    P.fwd.push_back(s);
-  }
-  // upsample stages: nearest x2 + conv == 4 phase convs on the low-res lattice, pixel-shuffled on store
-  for (int l = 1; l <= L; ++l) {
-    const int ci = ci_up1 + (l - 1);
-    const int h = H << (l - 1), w = W << (l - 1);
-    const int row0 = split_pack(ci, 256, 256, kPackUpFwd);
-    ConvParams cp = base_conv_params(N, h, w, tch, 4, 0, twrap, row0, 64, 256);  // 4 column groups (phases) of 64
-    Step s = conv_step(B.add_map(P.o_spl[l - 1], tvalid, ts, N, h, w, kABoxRows), cp, 2);
-    s.bias = packed_bias(B.add_bias(256, 2 * ci + 1, 64, 64));
-    s.cp.epi.act = 1;
-    s.cp.epi.store_mode = kStoreShuffle;
-    s.ob = ws(P.o_spl[l]); s.cp.epi.ob_stride = ts; s.cp.epi.split_off = tsplit; s.cp.epi.f16 = tf16; s.cp.mma_f16 = tf16;
-    P.fwd.push_back(s);
-  }
   const int hH = H << L, hW = W << L;
-  // conv3
-  {
-    const int row0 = split_pack(ci_conv3, 64, 64, kPackFwd);
-    ConvParams cp = base_conv_params(N, hH, hW, tch, 4, 0, twrap, row0, 64, 64);
-    Step s = conv_step(B.add_map(P.o_spl[L], tvalid, ts, N, hH, hW, kABoxRows), cp, 1);
-    s.bias = packed_bias(B.add_bias(64, 2 * ci_conv3 + 1, 64, 0));
-    s.cp.epi.act = 1;
-    s.ob = ws(P.o_splc); s.cp.epi.ob_stride = ts; s.cp.epi.split_off = tsplit; s.cp.epi.f16 = tf16; s.cp.mma_f16 = tf16;
-    P.fwd.push_back(s);
-  }
-  // conv4 + clamp
-  {
-    const int row0 = split_pack(ci_conv4, 16, d.out_channels, kPackFwd);
-    ConvParams cp = base_conv_params(N, hH, hW, tch, 4, 0, twrap, row0, 16, 16);
-    Step s = conv_step(B.add_map(P.o_splc, tvalid, ts, N, hH, hW, kABoxRows), cp, 1);
-    s.cp.epi.f16 = tf16; s.cp.mma_f16 = tf16;
-    s.bias = packed_bias(B.add_bias(16, 2 * ci_conv4 + 1, d.out_channels, 0));
-    s.cp.epi.store_mode = kStoreFinal;
-    s.cp.epi.n_valid = d.out_channels;
-    s.of.kind = RK_Y;
-    if (train) s.cm = ws(P.o_cmask);
+  if (!trunk) {
+    // conv2 (+ long skip)
+    {
+      const int row0 = split_pack(ci_conv2, 64, 64, kPackFwd);
+      ConvParams cp = base_conv_params(N, H, W, tch, 4, 0, twrap, row0, 64, 64);
+      Step s = conv_step(B.add_map(P.o_splt, tvalid, ts, N, H, W, kABoxRows), cp, 1);
+      s.bias = packed_bias(B.add_bias(64, 2 * ci_conv2 + 1, 64, 0));
+      s.r1 = ws(P.o_t0);
+      s.ob = ws(P.o_spl[0]); s.cp.epi.ob_stride = ts; s.cp.epi.split_off = tsplit; s.cp.epi.f16 = tf16; s.cp.mma_f16 = tf16;
+      P.fwd.push_back(s);
+    }
+    // upsample stages: nearest x2 + conv == 4 phase convs on the low-res lattice, pixel-shuffled on store
+    for (int l = 1; l <= L; ++l) {
+      const int ci = ci_up1 + (l - 1);
+      const int h = H << (l - 1), w = W << (l - 1);
+      const int row0 = split_pack(ci, 256, 256, kPackUpFwd);
+      ConvParams cp = base_conv_params(N, h, w, tch, 4, 0, twrap, row0, 64, 256);  // 4 column groups (phases) of 64
+      Step s = conv_step(B.add_map(P.o_spl[l - 1], tvalid, ts, N, h, w, kABoxRows), cp, 2);
+      s.bias = packed_bias(B.add_bias(256, 2 * ci + 1, 64, 64));
+      s.cp.epi.act = 1;
+      s.cp.epi.store_mode = kStoreShuffle;
+      s.ob = ws(P.o_spl[l]); s.cp.epi.ob_stride = ts; s.cp.epi.split_off = tsplit; s.cp.epi.f16 = tf16; s.cp.mma_f16 = tf16;
+      P.fwd.push_back(s);
+    }
+    // conv3
+    {
+      const int row0 = split_pack(ci_conv3, 64, 64, kPackFwd);
+      ConvParams cp = base_conv_params(N, hH, hW, tch, 4, 0, twrap, row0, 64, 64);
+      Step s = conv_step(B.add_map(P.o_spl[L], tvalid, ts, N, hH, hW, kABoxRows), cp, 1);
+      s.bias = packed_bias(B.add_bias(64, 2 * ci_conv3 + 1, 64, 0));
+      s.cp.epi.act = 1;
+      s.ob = ws(P.o_splc); s.cp.epi.ob_stride = ts; s.cp.epi.split_off = tsplit; s.cp.epi.f16 = tf16; s.cp.mma_f16 = tf16;
+      P.fwd.push_back(s);
+    }
+    // conv4 + clamp
+    {
+      const int row0 = split_pack(ci_conv4, 16, d.out_channels, kPackFwd);
+      ConvParams cp = base_conv_params(N, hH, hW, tch, 4, 0, twrap, row0, 16, 16);
+      Step s = conv_step(B.add_map(P.o_splc, tvalid, ts, N, hH, hW, kABoxRows), cp, 1);
+      s.cp.epi.f16 = tf16; s.cp.mma_f16 = tf16;
+      s.bias = packed_bias(B.add_bias(16, 2 * ci_conv4 + 1, d.out_channels, 0));
+      s.cp.epi.store_mode = kStoreFinal;
+      s.cp.epi.n_valid = d.out_channels;
+      s.of.kind = RK_Y;
+      if (train) s.cm = ws(P.o_cmask);
+      P.fwd.push_back(s);
+    }
+  } else {  // the trunk output leaves as NCHW fp32
+    Step s; s.type = ST_TRUNK_EXPORT; s.a = ws(P.o_tr);
     P.fwd.push_back(s);
   }
 
@@ -706,6 +730,9 @@ static int build_plan(b200sr_plan& P) {
       Step m; m.type = ST_MEMSET; m.a = ws(P.o_gw); m.count = P.gw_bytes;
       P.bwd.push_back(m);
       Step g; g.type = ST_INGEST_DY;
+      if (trunk) {  // dy takes the place of conv2's data gradient: GR and the last dense block's dY5 = bf16(0.04 dy)
+        g.type = ST_TRUNK_INGEST; g.a = ws(P.o_gr); g.c = ws(P.o_dyb[R - 1]); g.b.kind = RK_DY; g.scale = 0.04f;
+      }
       P.bwd.push_back(g);
     }
     // Launch order inside one gradient bucket: all data-gradient convs first (they form ONE chain launch), then the
@@ -717,93 +744,95 @@ static int build_plan(b200sr_plan& P) {
       st.blk = cur_blk; st.wc0 = cur_c0; st.wc1 = cur_c1;
       if (st.type == ST_CONV) seg_convs.push_back(st); else seg_others.push_back(st);
     };
-    // conv4: wgrad, bias grad, dgrad (-> G3, masked by lrelu'(conv3 out))
-    {
-      serves(R, ci_conv4, ci_conv4 + 1);
-      Step w4 = wgrad_step(P.o_splc, wg_c0 + 64, ts, P.o_dyp, 16, 64, N, hH, hW, wg_c0, 0, 16);
-      add_seg(w4, 0, 16, wref(ci_conv4), 64, 0, (int)align_up(d.out_channels, 4));
-      emit(w4);
-      Step b4 = biasgrad_step(P.o_dyp, HRpix, 64, 0, 16);
-      add_bseg(b4, 0, 16, bref(ci_conv4), d.out_channels);
-      emit(b4);
-      const int row0 = dgrad_pack1(ci_conv4, 64, d.out_channels);
-      ConvParams cp = base_conv_params(N, hH, hW, 1, 1, 0, 1 << 20, row0, 64, 64);
-      Step s = conv_step(B.add_map(P.o_dyp, 16, 64, N, hH, hW, kABoxRows), cp, 1);
-      s.mask = ws(P.o_splc); s.cp.epi.mask_stride = ts; s.cp.epi.mask_coff = 0;
-      s.ob = ws(P.o_g3); s.cp.epi.ob_stride = 64;
-      emit(s);
-    }
-    // conv3
-    {
-      serves(R, ci_conv3, ci_conv3 + 1);
-      Step w3 = wgrad_step(P.o_spl[L], wg_c0 + 64, ts, P.o_g3, 64, 64, N, hH, hW, wg_c0, 0, 64);
-      add_seg(w3, 0, 64, wref(ci_conv3), 64, 0, 64);
-      emit(w3);
-      Step b3 = biasgrad_step(P.o_g3, HRpix, 64, 0, 64);
-      add_bseg(b3, 0, 64, bref(ci_conv3), 64);
-      emit(b3);
-      const int row0 = dgrad_pack1(ci_conv3, 64, 64);
-      ConvParams cp = base_conv_params(N, hH, hW, 1, 4, 0, 1 << 20, row0, 64, 64);
-      Step s = conv_step(B.add_map(P.o_g3, 64, 64, N, hH, hW, kABoxRows), cp, 1);
-      if (L >= 1) {
-        s.mask = ws(P.o_spl[L]); s.cp.epi.mask_stride = ts;
-        s.ob = ws(P.o_gu[L]); s.cp.epi.ob_stride = 256; s.cp.epi.store_mode = kStoreUnshuffle;
-      } else {
-        s.of = ws(P.o_gt);
-        s.ob = ws(P.o_gtb); s.cp.epi.ob_stride = 64;
-      }
-      emit(s);
-    }
-    // upsample stages, top down
-    for (int l = L; l >= 1; --l) {
-      const int ci = ci_up1 + (l - 1);
-      const int h = H << (l - 1), w = W << (l - 1);
-      const long long npix = Ppix << (2 * (l - 1));
-      serves(R, ci, ci + 1);
-      for (int half = 0; half < 2; ++half) {
-        Step wu = wgrad_step(P.o_spl[l - 1], wg_c0 + 64, ts, P.o_gu[l], 256, 256, N, h, w, wg_c0, 128 * half, 128);
-        Ref out = wref(ci);
-        out.off += (long long)half * 32 * 64 * 4 * 4;  // 16-byte column chunks [32*half, +32) of the [tap][64 chunks][64 ci][4] staging tensor
-        add_seg(wu, 0, 128, out, 64, 0, 256);
-        emit(wu);
-      }
+    if (!trunk) {  // the HR tail (trunk plans start at the last dense block: see the ingest above)
+      // conv4: wgrad, bias grad, dgrad (-> G3, masked by lrelu'(conv3 out))
       {
-        Step bu = biasgrad_step(P.o_gu[l], npix, 256, 0, 256);
-        for (int ph = 0; ph < 4; ++ph) add_bseg(bu, 64 * ph, 64 * ph + 64, bref(ci), 64);
-        emit(bu);
+        serves(R, ci_conv4, ci_conv4 + 1);
+        Step w4 = wgrad_step(P.o_splc, wg_c0 + 64, ts, P.o_dyp, 16, 64, N, hH, hW, wg_c0, 0, 16);
+        add_seg(w4, 0, 16, wref(ci_conv4), 64, 0, (int)align_up(d.out_channels, 4));
+        emit(w4);
+        Step b4 = biasgrad_step(P.o_dyp, HRpix, 64, 0, 16);
+        add_bseg(b4, 0, 16, bref(ci_conv4), d.out_channels);
+        emit(b4);
+        const int row0 = dgrad_pack1(ci_conv4, 64, d.out_channels);
+        ConvParams cp = base_conv_params(N, hH, hW, 1, 1, 0, 1 << 20, row0, 64, 64);
+        Step s = conv_step(B.add_map(P.o_dyp, 16, 64, N, hH, hW, kABoxRows), cp, 1);
+        s.mask = ws(P.o_splc); s.cp.epi.mask_stride = ts; s.cp.epi.mask_coff = 0;
+        s.ob = ws(P.o_g3); s.cp.epi.ob_stride = 64;
+        emit(s);
       }
-      PackOp op; memset(&op, 0, sizeof(op));
-      op.n_total = 64; op.n_valid = 64; op.num_chunks = 4; op.mode = kPackUpDgrad; op.nseg = 1;
-      op.seg[0] = seg(0, 256, 2 * ci, 64, 64, 0, 0, 0);
-      const int row0 = B.add_pack(op);
-      ConvParams cp = base_conv_params(N, h, w, 4, 4, 0, 1 << 20, row0, 64, 64);
-      Step s = conv_step(B.add_map(P.o_gu[l], 256, 256, N, h, w, kABoxRows), cp, 1);
-      if (l >= 2) {
-        s.mask = ws(P.o_spl[l - 1]); s.cp.epi.mask_stride = ts;
-        s.ob = ws(P.o_gu[l - 1]); s.cp.epi.ob_stride = 256; s.cp.epi.store_mode = kStoreUnshuffle;
-      } else {
-        s.of = ws(P.o_gt);
-        s.ob = ws(P.o_gtb); s.cp.epi.ob_stride = 64;
+      // conv3
+      {
+        serves(R, ci_conv3, ci_conv3 + 1);
+        Step w3 = wgrad_step(P.o_spl[L], wg_c0 + 64, ts, P.o_g3, 64, 64, N, hH, hW, wg_c0, 0, 64);
+        add_seg(w3, 0, 64, wref(ci_conv3), 64, 0, 64);
+        emit(w3);
+        Step b3 = biasgrad_step(P.o_g3, HRpix, 64, 0, 64);
+        add_bseg(b3, 0, 64, bref(ci_conv3), 64);
+        emit(b3);
+        const int row0 = dgrad_pack1(ci_conv3, 64, 64);
+        ConvParams cp = base_conv_params(N, hH, hW, 1, 4, 0, 1 << 20, row0, 64, 64);
+        Step s = conv_step(B.add_map(P.o_g3, 64, 64, N, hH, hW, kABoxRows), cp, 1);
+        if (L >= 1) {
+          s.mask = ws(P.o_spl[L]); s.cp.epi.mask_stride = ts;
+          s.ob = ws(P.o_gu[L]); s.cp.epi.ob_stride = 256; s.cp.epi.store_mode = kStoreUnshuffle;
+        } else {
+          s.of = ws(P.o_gt);
+          s.ob = ws(P.o_gtb); s.cp.epi.ob_stride = 64;
+        }
+        emit(s);
       }
-      emit(s);
-    }
-    // conv2
-    {
-      serves(R, ci_conv2, ci_conv2 + 1);
-      Step w2 = wgrad_step(P.o_splt, wg_c0 + 64, ts, P.o_gtb, 64, 64, N, H, W, wg_c0, 0, 64);
-      add_seg(w2, 0, 64, wref(ci_conv2), 64, 0, 64);
-      emit(w2);
-      Step b2 = biasgrad_step(P.o_gtb, Ppix, 64, 0, 64);
-      add_bseg(b2, 0, 64, bref(ci_conv2), 64);
-      emit(b2);
-      const int row0 = dgrad_pack1(ci_conv2, 64, 64);
-      ConvParams cp = base_conv_params(N, H, W, 1, 4, 0, 1 << 20, row0, 64, 64);
-      Step s = conv_step(B.add_map(P.o_gtb, 64, 64, N, H, W, kABoxRows), cp, 1);
-      s.of = ws(P.o_gr);
-      s.ob = ws(P.o_dyb[R - 1]); s.cp.epi.ob_stride = 192; s.cp.epi.delta = 0.04f;
-      emit(s);
-      // tail bucket: conv2 .. conv4 are contiguous at the end of the flat buffer
-      emit(unpack_step(ci_conv2, nconv));
+      // upsample stages, top down
+      for (int l = L; l >= 1; --l) {
+        const int ci = ci_up1 + (l - 1);
+        const int h = H << (l - 1), w = W << (l - 1);
+        const long long npix = Ppix << (2 * (l - 1));
+        serves(R, ci, ci + 1);
+        for (int half = 0; half < 2; ++half) {
+          Step wu = wgrad_step(P.o_spl[l - 1], wg_c0 + 64, ts, P.o_gu[l], 256, 256, N, h, w, wg_c0, 128 * half, 128);
+          Ref out = wref(ci);
+          out.off += (long long)half * 32 * 64 * 4 * 4;  // 16-byte column chunks [32*half, +32) of the [tap][64 chunks][64 ci][4] staging tensor
+          add_seg(wu, 0, 128, out, 64, 0, 256);
+          emit(wu);
+        }
+        {
+          Step bu = biasgrad_step(P.o_gu[l], npix, 256, 0, 256);
+          for (int ph = 0; ph < 4; ++ph) add_bseg(bu, 64 * ph, 64 * ph + 64, bref(ci), 64);
+          emit(bu);
+        }
+        PackOp op; memset(&op, 0, sizeof(op));
+        op.n_total = 64; op.n_valid = 64; op.num_chunks = 4; op.mode = kPackUpDgrad; op.nseg = 1;
+        op.seg[0] = seg(0, 256, 2 * ci, 64, 64, 0, 0, 0);
+        const int row0 = B.add_pack(op);
+        ConvParams cp = base_conv_params(N, h, w, 4, 4, 0, 1 << 20, row0, 64, 64);
+        Step s = conv_step(B.add_map(P.o_gu[l], 256, 256, N, h, w, kABoxRows), cp, 1);
+        if (l >= 2) {
+          s.mask = ws(P.o_spl[l - 1]); s.cp.epi.mask_stride = ts;
+          s.ob = ws(P.o_gu[l - 1]); s.cp.epi.ob_stride = 256; s.cp.epi.store_mode = kStoreUnshuffle;
+        } else {
+          s.of = ws(P.o_gt);
+          s.ob = ws(P.o_gtb); s.cp.epi.ob_stride = 64;
+        }
+        emit(s);
+      }
+      // conv2
+      {
+        serves(R, ci_conv2, ci_conv2 + 1);
+        Step w2 = wgrad_step(P.o_splt, wg_c0 + 64, ts, P.o_gtb, 64, 64, N, H, W, wg_c0, 0, 64);
+        add_seg(w2, 0, 64, wref(ci_conv2), 64, 0, 64);
+        emit(w2);
+        Step b2 = biasgrad_step(P.o_gtb, Ppix, 64, 0, 64);
+        add_bseg(b2, 0, 64, bref(ci_conv2), 64);
+        emit(b2);
+        const int row0 = dgrad_pack1(ci_conv2, 64, 64);
+        ConvParams cp = base_conv_params(N, H, W, 1, 4, 0, 1 << 20, row0, 64, 64);
+        Step s = conv_step(B.add_map(P.o_gtb, 64, 64, N, H, W, kABoxRows), cp, 1);
+        s.of = ws(P.o_gr);
+        s.ob = ws(P.o_dyb[R - 1]); s.cp.epi.ob_stride = 192; s.cp.epi.delta = 0.04f;
+        emit(s);
+        // tail bucket: conv2 .. conv4 are contiguous at the end of the flat buffer
+        emit(unpack_step(ci_conv2, nconv));
+      }
     }
     // The data-gradient chain is cut ONCE, behind the HR tail: the tail's weight / bias gradients (HR-sized, L2-heavy, 8 % of the
     // weight-gradient FLOPs but 12 % of their time) then run on the side streams WHILE the trunk chain -- latency-bound, launched on one
@@ -814,13 +843,13 @@ static int build_plan(b200sr_plan& P) {
       seg_convs.clear(); seg_others.clear();
     }
     // trunk, last dense block first
-    int bucket_hi = ci_conv2;  // conv index (exclusive) up to which trunk gradients have been announced
+    int bucket_hi = P.t0 + 5 * R;  // conv index (exclusive) up to which trunk gradients have been announced
     for (int r = R - 1; r >= 0; --r) {
       const int j = r % 3;
       const long long D = P.o_dense[r];
       const long long DYc = P.o_dyb[r];
       const long long DYn = P.o_dyb[r > 0 ? r - 1 : 0];
-      serves(r, conv_index_rdb(r, 1), conv_index_rdb(r, 5) + 1);
+      serves(r, conv_index_rdb(P, r, 1), conv_index_rdb(P, r, 5) + 1);
       // epilogue of the block-input (x) slice: fp32 gradient carriers and the next block's dY5
       auto xslice_epilogue = [&](Step& s) {
         if (j == 2) { s.r1 = ws(P.o_gr); s.cp.epi.beta1 = 0.2f; s.of = ws(P.o_gc2); s.cp.epi.delta = 0.2f; }
@@ -841,7 +870,7 @@ static int build_plan(b200sr_plan& P) {
             const int kc0 = (k == 5) ? 0 : 64 + 32 * (4 - k);   // dY_k inside [dY5|dY4|dY3|dY2|dY1]
             const int kcl = (k == 5) ? 64 : 32;
             if (kc0 < k0 || kc0 + kcl > k0 + klen) continue;
-            op.seg[op.nseg++] = seg(kc0 - k0, kcl, 2 * conv_index_rdb(r, k), kcl, 64 + 32 * (k - 1), 0, 0, 0);
+            op.seg[op.nseg++] = seg(kc0 - k0, kcl, 2 * conv_index_rdb(P, r, k), kcl, 64 + 32 * (k - 1), 0, 0, 0);
           }
           const int row0 = B.add_pack(op);
           ConvParams cp = base_conv_params(N, H, W, 1, klen / 16, k0, 1 << 20, row0, 64, 64);
@@ -854,7 +883,7 @@ static int build_plan(b200sr_plan& P) {
           const int kk = 5 - q;
           const int klen = (kk == 5) ? 64 : 32;
           const int a_c0 = (q == 0) ? 0 : 64 + 32 * (q - 1);
-          const int ci = conv_index_rdb(r, kk);
+          const int ci = conv_index_rdb(P, r, kk);
           const int col_lo = 32 * q, ncols = 128 - col_lo;
           PackOp op; memset(&op, 0, sizeof(op));
           op.n_total = ncols; op.n_cols = ncols; op.n_valid = ncols; op.num_chunks = 1; op.mode = kPackDgrad; op.nseg = 0;
@@ -883,7 +912,7 @@ static int build_plan(b200sr_plan& P) {
         op.n_total = nsl; op.n_valid = nsl; op.num_chunks = (kin + 63) / 64; op.mode = kPackDgrad;
         op.nseg = 0;
         for (int k = 5; k > sl; --k) {
-          const int ci = conv_index_rdb(r, k);
+          const int ci = conv_index_rdb(P, r, k);
           const int k0 = (k == 5) ? 0 : 64 + 32 * (4 - k);
           const int klen = (k == 5) ? 64 : 32;
           op.seg[op.nseg++] = seg(k0, klen, 2 * ci, klen, 64 + 32 * (k - 1), 0, c_s, 0);
@@ -905,8 +934,8 @@ static int build_plan(b200sr_plan& P) {
       // whose column sums are the bias gradients of all five convs.  Per 128-pixel tile: 7 CTA-units of (M = 128) x N x 24
       // MMAs (3 x 160 + 160 + 96 + 32 + 32 = 800 columns); three channel-block problems with idle M rows and a separate bias
       // problem would take 9 + 1/3 (928 columns).
-      const int c5 = conv_index_rdb(r, 5), c4 = conv_index_rdb(r, 4), c3 = conv_index_rdb(r, 3), c2 = conv_index_rdb(r, 2),
-                c1 = conv_index_rdb(r, 1);
+      const int c5 = conv_index_rdb(P, r, 5), c4 = conv_index_rdb(P, r, 4), c3 = conv_index_rdb(P, r, 3), c2 = conv_index_rdb(P, r, 2),
+                c1 = conv_index_rdb(P, r, 1);
       Step wg = wgrad_batch(D, 192, 192, DYc, 192, 192, N, H, W);
       add_problem(wg, 0, 0, 160);             // x, o1, o2 rows at the CTA's tap x [dY5|dY4|dY3|dY2]
       add_seg(wg, 0, 64, wref(c5), 192, 0, 64);
@@ -935,13 +964,13 @@ static int build_plan(b200sr_plan& P) {
         const int blk = r / 3;
         const int G = d.grad_bucket_rrdbs > 0 ? d.grad_bucket_rrdbs : 1;
         if (blk % G == 0 || (G > 2 && blk == 2)) {
-          emit(unpack_step(conv_index_rdb(r, 1), bucket_hi));
-          bucket_hi = conv_index_rdb(r, 1);
+          emit(unpack_step(conv_index_rdb(P, r, 1), bucket_hi));
+          bucket_hi = conv_index_rdb(P, r, 1);
         }
       }
     }
     // conv1: gradient of its output = trunk path (GR) + long skip (GT)
-    {
+    if (!trunk) {
       serves(-1, 0, 1);
       Step ad; ad.type = ST_ADD; ad.a = ws(P.o_gr); ad.b = ws(P.o_gt); ad.c = ws(P.o_go1); ad.count = Ppix * 64;
       emit(ad);
@@ -960,7 +989,7 @@ static int build_plan(b200sr_plan& P) {
     seg_convs.clear(); seg_others.clear();
     // Gradient w.r.t. the LR input = conv1's data gradient of GO1 (64 -> in_channels), stored fp32 NCHW to the caller's dx.
     // The reference produces it whenever x.requires_grad (input-gradient probes); it is launched only when dx != NULL.
-    {
+    if (!trunk) {
       const int C = d.in_channels;
       const int npad = (int)align_up(C, 16);
       PackOp op; memset(&op, 0, sizeof(op));
@@ -973,6 +1002,9 @@ static int build_plan(b200sr_plan& P) {
       s.cp.epi.n_valid = C;
       s.of.kind = RK_Y;
       s.needs_dx = true;
+      P.bwd.push_back(s);
+    } else {  // the trunk-input gradient is GR after the first dense block's epilogue
+      Step s; s.type = ST_TRUNK_EXPORT; s.a = ws(P.o_gr); s.needs_dx = true;
       P.bwd.push_back(s);
     }
   }
@@ -1015,7 +1047,7 @@ static int build_plan(b200sr_plan& P) {
     int nchains = 0, last = -1;
     for (size_t i = 0; i < P.bwd.size(); ++i)
       if (P.bwd[i].type == ST_CHAIN && !P.bwd[i].needs_dx) { ++nchains; last = (int)i; }
-    if (nchains >= 2 && P.groups >= 2) {
+    if (nchains >= 2 && P.groups >= 2 && !P.trunk) {  // (trunk plans: no tail gradients to run beside it)
       Step& c = P.bwd[last];
       int per_group = 0;
       for (int l = 0; l < c.nlayers; ++l) {
@@ -1414,6 +1446,7 @@ struct GradSelect {
   std::vector<uint8_t> want;  // per conv: its weight and/or bias gradient is wanted
   int stop_blk = -1;          // data-gradient layers of dense blocks below this one are not launched (R: tail only, R + 1: none)
   int R = 0;
+  int t0 = 1;                 // conv index of the first dense-block conv
   bool any(int c0, int c1) const {
     for (int c = c0; c < c1; ++c)
       if (want[c]) return true;
@@ -1421,8 +1454,8 @@ struct GradSelect {
   }
   // the convs a launch wrote: a dense block's one weight-gradient launch writes all five of its convs if any is wanted
   bool written(int c) const {
-    if (c < 1 || c > 5 * R) return want[c] != 0;
-    const int c0 = 1 + (c - 1) / 5 * 5;
+    if (c < t0 || c >= t0 + 5 * R) return want[c] != 0;
+    const int c0 = t0 + (c - t0) / 5 * 5;
     return any(c0, c0 + 5);
   }
 };
@@ -1432,17 +1465,19 @@ static GradSelect make_select(const b200sr_plan& P, const uint8_t* mask, bool gr
   const int nconv = ((int)P.param_off.size() - 1) / 2;
   GradSelect g;
   g.R = P.R;
+  g.t0 = P.t0;
   g.want.assign(nconv, 0);
   if (grads)
     for (int c = 0; c < nconv; ++c) g.want[c] = mask ? (mask[c] != 0) : 1;
-  // conv1's output gradient GO1 = GR + GT needs the whole trunk; otherwise the walk ends after the lowest wanted dense block
-  if (dx || g.want[0]) {
+  // conv1's output gradient GO1 = GR + GT needs the whole trunk (as does a trunk plan's dx); otherwise the walk ends after the lowest
+  // wanted dense block
+  if (dx || (!P.trunk && g.want[0])) {
     g.stop_blk = -1;
   } else {
     g.stop_blk = P.R + 1;
     for (int r = 0; r < P.R; ++r)
-      if (g.any(conv_index_rdb(r, 1), conv_index_rdb(r, 5) + 1)) { g.stop_blk = r; break; }
-    if (g.stop_blk > P.R && g.any(1 + 5 * P.R, nconv)) g.stop_blk = P.R;
+      if (g.any(conv_index_rdb(P, r, 1), conv_index_rdb(P, r, 5) + 1)) { g.stop_blk = r; break; }
+    if (g.stop_blk > P.R && g.any(P.t0 + 5 * P.R, nconv)) g.stop_blk = P.R;
   }
   return g;
 }
@@ -1560,6 +1595,7 @@ static int run_steps(b200sr_plan& P, std::vector<Step>& steps, const Bases& b, c
   for (size_t si = 0; si < steps.size(); ++si) {
     Step& s = steps[si];
     if (s.needs_wgrad && !b.grads) continue;  // discriminator backward for the generator update: data gradients only
+    if (s.needs_dx && !b.y) continue;         // nobody asked for the input gradient
     if (!step_selected(s, sel, b.grads != nullptr, b.y != nullptr, cb != nullptr)) continue;
     if (overlap_chain >= 0 && (int)si < overlap_chain && (s.type == ST_WGRAD || s.type == ST_BIASGRAD)) {
       deferred.push_back((int)si);
@@ -1597,7 +1633,6 @@ static int run_steps(b200sr_plan& P, std::vector<Step>& steps, const Bases& b, c
       case ST_CONV:
         return fail(B200SR_ERR_INVALID, "internal: unchained conv step");
       case ST_CHAIN: {
-        if (s.needs_dx && !b.y) break;  // nobody asked for the input gradient
         const int nl = chain_layers(P, s, sel);
         if (nl == 0) break;
         int rc = launch_chain_prefix(P, s, nl, b, st);
@@ -1755,6 +1790,36 @@ static int run_steps(b200sr_plan& P, std::vector<Step>& steps, const Bases& b, c
           unpack_wgrad_down_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>((const float*)((char*)b.ws + P.o_gw) + u.src_off, (float*)b.grads + u.dst_off, u.co, u.ci, u.co_pad);
           CUDA_TRY(cudaGetLastError());
         }
+        break;
+      }
+      case ST_TRUNK_INGEST: {
+        const int tx = (d.width + kTileW - 1) / kTileW, ty = (d.height + kTileH - 1) / kTileH;
+        const int blocks = d.batch * tx * ty;  // one 256-thread block per 8 x 32 tile
+        float* carrier = (float*)resolve(s.a, b);
+        __nv_bfloat16* shadow = (__nv_bfloat16*)resolve(s.c, b);
+        if (s.b.kind == RK_DY) {  // dy: fp32 contiguous NCHW
+          const long long plane = (long long)d.height * d.width;
+          trunk_ingest_kernel<float><<<blocks, 256, 0, st>>>((const float*)b.dy, 64 * plane, plane, d.width, 1, d.batch, d.height, d.width, tx, ty,
+                                                             s.scale, carrier, shadow, 192);
+        } else if (x_dtype == B200SR_F32) {
+          trunk_ingest_kernel<float><<<blocks, 256, 0, st>>>((const float*)x, xs[0], xs[1], xs[2], xs[3], d.batch, d.height, d.width, tx, ty, s.scale,
+                                                             carrier, shadow, 192);
+        } else if (x_dtype == B200SR_F16) {
+          trunk_ingest_kernel<__half><<<blocks, 256, 0, st>>>((const __half*)x, xs[0], xs[1], xs[2], xs[3], d.batch, d.height, d.width, tx, ty, s.scale,
+                                                              carrier, shadow, 192);
+        } else if (x_dtype == B200SR_BF16) {
+          trunk_ingest_kernel<__nv_bfloat16><<<blocks, 256, 0, st>>>((const __nv_bfloat16*)x, xs[0], xs[1], xs[2], xs[3], d.batch, d.height, d.width, tx,
+                                                                     ty, s.scale, carrier, shadow, 192);
+        } else {
+          return fail(B200SR_ERR_INVALID, "unknown x dtype %d", x_dtype);
+        }
+        CUDA_TRY(cudaGetLastError());
+        break;
+      }
+      case ST_TRUNK_EXPORT: {  // to the caller's y (forward) or dx (backward)
+        const int tx = (d.width + kTileW - 1) / kTileW, ty = (d.height + kTileH - 1) / kTileH;
+        trunk_export_kernel<<<d.batch * tx * ty, 256, 0, st>>>((const float*)resolve(s.a, b), (float*)b.y, d.batch, d.height, d.width, tx, ty);
+        CUDA_TRY(cudaGetLastError());
         break;
       }
       case ST_INGEST_DY: {
@@ -2236,7 +2301,7 @@ static int build_disc_plan(b200sr_plan& P) {
 extern "C" {
 
 const char* b200sr_last_error(void) { return g_err; }
-int b200sr_version(void) { return 101; }
+int b200sr_version(void) { return 102; }
 void b200sr_debug_set(int flags) { g_debug = flags; }
 int b200sr_debug_read_profile(unsigned long long* out_host, int n) {
   CUDA_TRY(cudaMemcpyFromSymbol(out_host, g_conv_prof, sizeof(unsigned long long) * (size_t)n));
@@ -2250,10 +2315,11 @@ int b200sr_debug_buffer(const b200sr_plan* p, const char* name, int64_t* offset_
   return fail(B200SR_ERR_INVALID, "the plan has no workspace tensor named '%s'", name);
 }
 
-int b200sr_plan_create(const b200sr_net_desc* desc, b200sr_plan** out) {
+static int net_plan_create(const b200sr_net_desc* desc, bool trunk, b200sr_plan** out) {
   if (!desc || !out) return fail(B200SR_ERR_INVALID, "null argument");
   b200sr_plan* p = new b200sr_plan();
   p->d = *desc;
+  p->trunk = trunk;
   p->det = desc->deterministic != 0;
   if (const char* e = getenv("B200SR_REASSOC")) p->reassoc = atoi(e) != 0;  // 0: per-conv schedule everywhere
   p->tail_f16 = desc->training == 0;  // training: the L1 loss' sign(sr - gt) amplifies the fp16 rounding of the tail past the 1e-2 gradient bar
@@ -2263,6 +2329,9 @@ int b200sr_plan_create(const b200sr_net_desc* desc, b200sr_plan** out) {
   *out = p;
   return 0;
 }
+
+int b200sr_plan_create(const b200sr_net_desc* desc, b200sr_plan** out) { return net_plan_create(desc, false, out); }
+int b200sr_trunk_plan_create(const b200sr_net_desc* desc, b200sr_plan** out) { return net_plan_create(desc, true, out); }
 
 void b200sr_plan_destroy(b200sr_plan* p) {
   if (!p) return;
@@ -2332,7 +2401,7 @@ double b200sr_flops(const b200sr_plan* p, int backward) {
       res = (t <= p->L) ? (double)(1 << (2 * t)) : (double)(1 << (2 * p->L));
     }
     const double fl = 2.0 * 9 * O * I * res * px;
-    total += backward ? fl * (c == 0 ? 1 : 2) : fl;
+    total += backward ? fl * (c < p->t0 ? 1 : 2) : fl;  // (conv1 has no data gradient; every trunk conv has one)
   }
   return total;
 }
@@ -2421,7 +2490,8 @@ int32_t b200sr_backward_launches(const b200sr_plan* p, const uint8_t* conv_wante
   int n = 0;
   for (const Step& s : p->bwd) {
     if (s.type == ST_MEMSET) continue;
-    if (s.type == ST_CHAIN) { n += s.needs_dx ? (with_dx != 0) : (chain_layers(*p, s, sel) > 0); continue; }
+    if (s.needs_dx) { n += with_dx != 0; continue; }
+    if (s.type == ST_CHAIN) { n += chain_layers(*p, s, sel) > 0; continue; }
     if (s.type == ST_UNPACK && !with_cb && s.i0 != 0) continue;
     n += step_selected(s, sel, true, with_dx != 0, with_cb != 0) * (1 + det_sums(*p, s));
   }

@@ -28,7 +28,8 @@ class _Plan:
                           desc["num_blocks"], desc["n_up"], batch, height, width, 1 if training else 0, grad_bucket_rrdbs,
                           1 if deterministic else 0)
         handle = C.c_void_p()
-        _lib.check(lib.b200sr_plan_create(C.byref(nd), C.byref(handle)))
+        create = lib.b200sr_trunk_plan_create if desc.get("trunk_only") else lib.b200sr_plan_create
+        _lib.check(create(C.byref(nd), C.byref(handle)))
         self.handle = handle
         self.training = training
         self.deterministic = deterministic
@@ -222,7 +223,8 @@ def conv_mask(need_params) -> "C.Array":
 
 
 def generator_forward(module, x: torch.Tensor) -> torch.Tensor:
-    """Entry used by the drop-in modules' ``forward``."""
+    """Entry used by the drop-in modules' ``forward`` (generators and :class:`~sr_gan_fd_b200.rrdbnet.RRDBTrunk`: the module's
+    ``net_desc()`` says which plan it runs, its ``_conv_list()`` which parameters)."""
     if x.dim() != 4:
         raise RuntimeError(f"expected NCHW input, got shape {tuple(x.shape)}")
     if not x.is_cuda:
@@ -268,24 +270,34 @@ def eager_forward(module, x: torch.Tensor) -> torch.Tensor:
     def act(t):
         return F.leaky_relu(t, 0.2)
 
-    def dense_block(rdb, t):
-        feats = [t]
-        for conv in (rdb.conv1, rdb.conv2, rdb.conv3, rdb.conv4):
-            feats.append(act(conv(torch.cat(feats, 1))))
-        return rdb.conv5(torch.cat(feats, 1)) * 0.2 + t
-
     head = module.conv1(x)
-    t = head
-    for rrdb in module.trunk:
-        inner = t
-        for rdb in (rrdb.rdb1, rrdb.rdb2, rrdb.rdb3):
-            inner = dense_block(rdb, inner)
-        t = inner * 0.2 + t
-    t = head + module.conv2(t)
+    t = head + module.conv2(eager_trunk(module.trunk, head))
     for u in range(1, module._n_up + 1):
         t = act(getattr(module, f"upsampling{u}")[0](F.interpolate(t, scale_factor=2, mode="nearest")))
     t = module.conv4(act(module.conv3[0](t)))
     return torch.clamp(t, 0.0, 1.0)
+
+
+def eager_trunk(trunk, t: torch.Tensor) -> torch.Tensor:
+    """The RRDB stack on its own ``nn.Conv2d`` children with stock torch ops (ESRGAN/model.py:49-60,77-86): what
+    :func:`eager_forward` runs between conv1 and conv2, and what :class:`~sr_gan_fd_b200.rrdbnet.RRDBTrunk` runs on the CPU."""
+    import torch.nn.functional as F
+
+    def act(v):
+        return F.leaky_relu(v, 0.2)
+
+    def dense_block(rdb, v):
+        feats = [v]
+        for conv in (rdb.conv1, rdb.conv2, rdb.conv3, rdb.conv4):
+            feats.append(act(conv(torch.cat(feats, 1))))
+        return rdb.conv5(torch.cat(feats, 1)) * 0.2 + v
+
+    for rrdb in trunk:
+        inner = t
+        for rdb in (rrdb.rdb1, rrdb.rdb2, rrdb.rdb3):
+            inner = dense_block(rdb, inner)
+        t = inner * 0.2 + t
+    return t
 
 
 def attach_grad_bucket_hook(module, hook: Optional[Callable[[torch.Tensor, int, int], None]]) -> None:

@@ -35,6 +35,7 @@ _lib = None
 # symbol -> (restype, argtypes); every entry point declared in include/b200sr.h
 SIGNATURES = {
     "b200sr_plan_create": (C.c_int, [C.POINTER(NetDesc), C.POINTER(C.c_void_p)]),
+    "b200sr_trunk_plan_create": (C.c_int, [C.POINTER(NetDesc), C.POINTER(C.c_void_p)]),
     "b200sr_plan_destroy": (None, [C.c_void_p]),
     "b200sr_workspace_bytes": (C.c_size_t, [C.c_void_p]),
     "b200sr_packed_bytes": (C.c_size_t, [C.c_void_p]),

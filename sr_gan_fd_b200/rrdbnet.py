@@ -14,6 +14,7 @@ C-ABI CUDA library (``include/b200sr.h``).  There is no CPU or eager-PyTorch fal
 """
 from __future__ import annotations
 
+from collections import OrderedDict
 from typing import Any, List
 
 import torch
@@ -22,7 +23,7 @@ from torch import nn
 from . import function as _function
 
 __all__ = [
-    "RRDBNet", "BSRGAN", "RealRRDBNet",
+    "RRDBNet", "BSRGAN", "RealRRDBNet", "RRDBTrunk", "native_trunk",
     "rrdbnet_x1", "rrdbnet_x2", "rrdbnet_x4", "rrdbnet_x8", "bsrgan_x2", "bsrgan_x4", "real_rrdbnet_x4",
 ]
 
@@ -70,12 +71,9 @@ def _up_stage(channels: int) -> nn.Sequential:
     return nn.Sequential(nn.Conv2d(channels, channels, (3, 3), (1, 1), (1, 1)), nn.LeakyReLU(0.2, True))
 
 
-class _GeneratorBase(nn.Module):
-    """Shared forward: collects the convs in ``state_dict`` order and hands them to the native path."""
-
-    upscale_factor: int
-    _n_up: int
-    _pixel_unshuffle: int = 1
+class _NativeState:
+    """Mixin of the modules whose forward runs in libb200sr.so: ESRGAN init, and native runtime state that is never part of
+    the module's persistent state."""
 
     def _finish_init(self) -> None:
         for module in self.modules():
@@ -108,6 +106,14 @@ class _GeneratorBase(nn.Module):
                 continue
             new.__dict__[k] = copy.deepcopy(v, memo)
         return new
+
+
+class _GeneratorBase(_NativeState, nn.Module):
+    """Shared forward: collects the convs in ``state_dict`` order and hands them to the native path."""
+
+    upscale_factor: int
+    _n_up: int
+    _pixel_unshuffle: int = 1
 
     def zero_grad(self, set_to_none: bool = True) -> None:
         """Same contract as ``nn.Module.zero_grad``; the ``set_to_none`` path skips the generic per-parameter work (the
@@ -223,6 +229,86 @@ class RealRRDBNet(_GeneratorBase):
     def _forward_impl(self, x: torch.Tensor) -> torch.Tensor:
         # nn.PixelUnshuffle is pure data movement on the 3-channel input (identity for x4); kept as the torch op.
         return _function.generator_forward(self, self.downsampling(x))
+
+
+class RRDBTrunk(_NativeState, nn.Sequential):
+    """The RRDB stack alone, as a drop-in for ``nn.Sequential(*RRDBs)`` in any generator built around it (BasicSR /
+    Real-ESRGAN ``RRDBNet``, A-ESRGAN's ``bsrgantrans_x2`` / ``gen_rrdb2x``, models with their own head, tail or
+    conditioning).  ``state_dict`` keys are those of the Sequential (``0.rdb1.conv1.weight`` ...).
+
+    Math contract (ESRGAN / BasicSR RRDB), for ``x`` of shape ``[N, 64, H, W]``::
+
+        dense block:  o_k = LeakyReLU_0.2(conv_k(cat(x, o_1 .. o_{k-1})))  for k = 1..4
+                      rdb(x) = 0.2 * conv5(cat(x, o_1 .. o_4)) + x
+        RRDB:         rrdb(x) = 0.2 * rdb3(rdb2(rdb1(x))) + x
+        trunk:        y = rrdb_{B-1}( ... rrdb_0(x))
+
+    3x3 convs, stride 1, padding 1, with bias; 64 channels, growth 32.  On a CUDA device forward and backward run in the
+    generator's kernels (``include/b200sr.h`` "Trunk plans"): ``x`` may be fp32, fp16 or bf16, NCHW or channels_last; ``y``
+    and the input gradient are fp32, ``y`` is not clamped.  On the CPU the children run through stock torch ops.
+    Build one with the constructor, or adopt an existing Sequential with :func:`native_trunk`."""
+
+    def __init__(self, channels: int = 64, growth_channels: int = 32, num_blocks: int = 23) -> None:
+        nn.Sequential.__init__(self, *[_ResidualResidualDenseBlock(channels, growth_channels) for _ in range(num_blocks)])
+        self._finish_init()
+
+    def __getitem__(self, idx):
+        if isinstance(idx, slice):  # nn.Sequential would call the constructor with the children
+            return _adopt(OrderedDict(list(self._modules.items())[idx]))
+        return nn.Sequential.__getitem__(self, idx)
+
+    def _conv_list(self) -> List[nn.Conv2d]:
+        return [getattr(getattr(rrdb, r), c) for rrdb in self for r in ("rdb1", "rdb2", "rdb3")
+                for c in ("conv1", "conv2", "conv3", "conv4", "conv5")]
+
+    def net_desc(self) -> dict:
+        conv1 = self[0].rdb1.conv1
+        return dict(in_channels=conv1.in_channels, out_channels=conv1.in_channels, channels=conv1.in_channels,
+                    growth=conv1.out_channels, num_blocks=len(self), n_up=0, trunk_only=1)
+
+    def forward(self, x: torch.Tensor) -> torch.Tensor:
+        if not x.is_cuda:
+            return _function.eager_trunk(self, x)
+        return _function.generator_forward(self, x)
+
+
+def _adopt(children: "OrderedDict[str, nn.Module]") -> RRDBTrunk:
+    trunk = RRDBTrunk.__new__(RRDBTrunk)
+    nn.Sequential.__init__(trunk, children)
+    return trunk
+
+
+def native_trunk(seq: nn.Sequential) -> RRDBTrunk:
+    """An :class:`RRDBTrunk` that adopts the children of ``seq`` (the same module objects: Parameter identity, optimizer state and
+    the parent model's ``state_dict`` are unchanged).  Usage: ``model.trunk = native_trunk(model.trunk)``.
+
+    Every child must hold exactly ``rdb1``, ``rdb2``, ``rdb3``, each with ``conv1`` .. ``conv5``: 3x3 ``nn.Conv2d`` with bias,
+    stride 1, padding 1, of the RRDB shapes for 64 channels and growth 32, and no other parameters or buffers
+    (parameter-free children such as a LeakyReLU module are fine).  Anything else raises ``ValueError``: the native path computes
+    the contract in :class:`RRDBTrunk`'s docstring and nothing else."""
+    if isinstance(seq, RRDBTrunk):
+        return seq
+    if not isinstance(seq, nn.Sequential) or len(seq) == 0:
+        raise ValueError("native_trunk expects a non-empty nn.Sequential of RRDBs")
+    for name, rrdb in seq.named_children():
+        if [n for n, _ in rrdb.named_children()] != ["rdb1", "rdb2", "rdb3"] or \
+                any(True for _ in rrdb.named_parameters(recurse=False)) or any(True for _ in rrdb.named_buffers(recurse=False)):
+            raise ValueError(f"trunk child {name!r} is not an RRDB of exactly rdb1, rdb2, rdb3")
+        for r in ("rdb1", "rdb2", "rdb3"):
+            rdb = getattr(rrdb, r)
+            expect = {f"conv{k}.{p}" for k in range(1, 6) for p in ("weight", "bias")}
+            params = {n for n, _ in rdb.named_parameters()}
+            if params != expect or any(True for _ in rdb.named_buffers()):
+                raise ValueError(f"{name}.{r}: expected the parameters of conv1..conv5 and nothing else, got {sorted(params)}")
+            for k in range(1, 6):
+                conv = getattr(rdb, f"conv{k}")
+                cin, cout = 64 + 32 * (k - 1), 32 if k < 5 else 64
+                if not (type(conv) is nn.Conv2d and conv.in_channels == cin and conv.out_channels == cout and
+                        conv.kernel_size == (3, 3) and conv.stride == (1, 1) and conv.padding == (1, 1) and
+                        conv.dilation == (1, 1) and conv.groups == 1 and conv.padding_mode == "zeros" and conv.bias is not None):
+                    raise ValueError(f"{name}.{r}.conv{k}: expected a 3x3 Conv2d({cin}, {cout}), stride 1, padding 1, with bias; "
+                                     f"got {conv!r}")
+    return _adopt(OrderedDict(seq.named_children()))
 
 
 # --- factories (names the reference scripts look up with model.__dict__[arch]) ------------------------------------
