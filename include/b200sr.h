@@ -70,6 +70,17 @@ typedef struct b200sr_net_desc {
  *   conv_wanted_or_null  5 x 3 x num_blocks bytes, same order.
  * The trunk kernels are the generator's: for the same input, a trunk plan's y is bit for bit the generator's trunk output. */
 
+/* Unclamped plans (b200sr_unclamped_plan_create): the whole generator for models whose output is conv4's, not clamped -- BasicSR /
+ * Real-ESRGAN RRDBNet, A-ESRGAN's Generator_RRDB.  It accepts exactly the descriptors b200sr_plan_create accepts, and every
+ * generator entry point works on it unchanged (packing, forward, backward, b200sr_backward_select, launch counts, buckets,
+ * deterministic mode, b200sr_debug_buffer).  What differs:
+ *   y   [batch, out_channels, s*height, s*width] fp32: conv4's output, NOT clamped to [0, 1];
+ *   dy  the gradient w.r.t. that unclamped y: it enters the backward as it is, with no clamp pass-through mask;
+ *   the training workspace holds no "CMASK", so it is smaller by that buffer (batch x out_channels x s*height x s*width bytes,
+ *   rounded up to 1024).
+ * Launch list, parameter order, flat-gradient layout and b200sr_pack_layout_id are those of the clamped plan of the same descriptor,
+ * so the packed buffer can be shared; for the same input, clamp(y_unclamped, 0, 1) is bit for bit the clamped plan's y. */
+
 /* Deterministic plans (the `deterministic` member of the net, VGG and discriminator descriptors; torch.use_deterministic_algorithms).
  * A default plan sums weight and bias gradients (and the VGG loss value) with atomics, so their order -- and the last bits --
  * depend on CTA scheduling.  A deterministic plan gives bit-identical outputs for bit-identical inputs, for one GPU model,
@@ -86,6 +97,7 @@ typedef void (*b200sr_bucket_cb)(void* user, int64_t offset, int64_t count);
 
 int b200sr_plan_create(const b200sr_net_desc* desc, b200sr_plan** out);
 int b200sr_trunk_plan_create(const b200sr_net_desc* desc, b200sr_plan** out); /* see "Trunk plans" above */
+int b200sr_unclamped_plan_create(const b200sr_net_desc* desc, b200sr_plan** out); /* see "Unclamped plans" above */
 void b200sr_plan_destroy(b200sr_plan* plan);
 
 /* sizes (bytes) of the caller-allocated buffers */
@@ -108,7 +120,7 @@ int32_t b200sr_num_launches(const b200sr_plan* plan, int backward);
 int b200sr_pack_weights(b200sr_plan* plan, const float* const* params, void* packed, b200sr_stream stream);
 
 /* x: [batch, in_channels, height, width] with element strides x_strides[4] (NCHW or channels_last), dtype per
- * b200sr_dtype.  y: [batch, out_channels, s*height, s*width] fp32 contiguous, clamped to [0,1]. */
+ * b200sr_dtype.  y: [batch, out_channels, s*height, s*width] fp32 contiguous, clamped to [0,1] (unclamped plans: not clamped). */
 int b200sr_forward(b200sr_plan* plan, const void* x, int x_dtype, const int64_t* x_strides, const void* packed,
                    void* workspace, float* y, b200sr_stream stream);
 
@@ -260,8 +272,8 @@ int b200sr_debug_read_profile(unsigned long long* out_host, int n);
  * holds).  Generator plans name theirs too (build_plan in b200sr.cu; trunk plans only "TR" "C1" "C2", the "D" buffers and, in training
  * plans, "GR" "GC1" "GC2" and the "DYB" buffers): "xin", the fp32 carriers "T0" "TR" "C1" "C2" (tile-blocked),
  * the dense-block buffers "D0" ... "D{R-1}" (R = 3 * num_blocks; inference plans keep only the ping-pong pair "D0" "D1"), the
- * tail activations "SPLT" "SPL0" ... "SPL{n_up}" "SPLC" and, in training plans, "CMASK" "DYP" "G3" "GU1" ... "GU{n_up}" "GT" "GTB"
- * "GR" "GC1" "GC2" "GO1" "DYB0" ... "DYB{R-1}".  VGG plans name none. */
+ * tail activations "SPLT" "SPL0" ... "SPL{n_up}" "SPLC" and, in training plans, "CMASK" (not in unclamped plans) "DYP" "G3"
+ * "GU1" ... "GU{n_up}" "GT" "GTB" "GR" "GC1" "GC2" "GO1" "DYB0" ... "DYB{R-1}".  VGG plans name none. */
 int b200sr_debug_buffer(const b200sr_plan* plan, const char* name, int64_t* offset_bytes, int64_t* bytes);
 
 #ifdef __cplusplus

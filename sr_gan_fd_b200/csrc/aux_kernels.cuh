@@ -180,8 +180,9 @@ __global__ void ingest_input_kernel(const T* __restrict__ x, long long sn, long 
   for (int c = 3 * C; c < out_stride; ++c) o[c] = __float2bfloat16_rn(0.f);
 }
 
-// dy: [N, C, H, W] fp32 contiguous (gradient of the clamped image) -> [N*H*W, 64] bf16, channels >= C zero,
-// multiplied by the clamp pass-through mask recorded in the forward.
+// dy: [N, C, H, W] fp32 contiguous (gradient of the generator output) -> [N*H*W, 64] bf16, channels >= C zero.  kMasked (clamped
+// plans): multiplied by the clamp pass-through mask recorded in the forward; otherwise (unclamped plans) mask is unused.
+template <bool kMasked>
 __global__ void ingest_grad_kernel(const float* __restrict__ dy, const unsigned char* __restrict__ mask, int N, int C,
                                    int H, int W, __nv_bfloat16* __restrict__ out, int out_stride) {
   const long long pix = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
@@ -196,7 +197,7 @@ __global__ void ingest_grad_kernel(const float* __restrict__ dy, const unsigned 
     v[c] = 0.f;
     if (c < C) {
       const long long i = (n * C + c) * plane + r;
-      v[c] = mask[i] ? dy[i] : 0.f;
+      v[c] = (!kMasked || mask[i]) ? dy[i] : 0.f;
     }
   }
   // 16 channels = 32 bytes per pixel: two 16-byte stores (out_stride is a multiple of 8 channels)

@@ -166,6 +166,7 @@ struct b200sr_plan {
   int L = 0;  // upsample stages
   bool trunk = false;  // trunk plan (b200sr.h "Trunk plans"): the dense blocks alone, no conv1 / long skip / tail
   int t0 = 1;          // state_dict conv index of the first trunk conv (0 in trunk plans)
+  bool unclamped = false;  // unclamped generator plan (b200sr.h "Unclamped plans"): y = conv4's output, no CMASK, dy ingested unmasked
   int xin_stride = 64;
   long long ws_bytes = 0;
   long long total_rows = 0, bias_floats = 0, packed_bytes = 0;
@@ -423,7 +424,7 @@ static int build_plan(b200sr_plan& P) {
   const long long HRpix = Ppix << (2 * L);
   if (train) {
     if (!trunk) {
-      P.o_cmask = B.alloc("CMASK", HRpix * d.out_channels);
+      if (!P.unclamped) P.o_cmask = B.alloc("CMASK", HRpix * d.out_channels);
       P.o_dyp = B.alloc("DYP", HRpix * 64 * 2);
       P.o_g3 = B.alloc("G3", HRpix * 64 * 2);
     }
@@ -642,7 +643,7 @@ static int build_plan(b200sr_plan& P) {
       s.ob = ws(P.o_splc); s.cp.epi.ob_stride = ts; s.cp.epi.split_off = tsplit; s.cp.epi.f16 = tf16; s.cp.mma_f16 = tf16;
       P.fwd.push_back(s);
     }
-    // conv4 + clamp
+    // conv4 + clamp (unclamped plans: conv4 alone)
     {
       const int row0 = split_pack(ci_conv4, 16, d.out_channels, kPackFwd);
       ConvParams cp = base_conv_params(N, hH, hW, tch, 4, 0, twrap, row0, 16, 16);
@@ -651,8 +652,9 @@ static int build_plan(b200sr_plan& P) {
       s.bias = packed_bias(B.add_bias(16, 2 * ci_conv4 + 1, d.out_channels, 0));
       s.cp.epi.store_mode = kStoreFinal;
       s.cp.epi.n_valid = d.out_channels;
+      s.cp.epi.unclamped = P.unclamped;
       s.of.kind = RK_Y;
-      if (train) s.cm = ws(P.o_cmask);
+      if (train && !P.unclamped) s.cm = ws(P.o_cmask);
       P.fwd.push_back(s);
     }
   } else {  // the trunk output leaves as NCHW fp32
@@ -1825,8 +1827,9 @@ static int run_steps(b200sr_plan& P, std::vector<Step>& steps, const Bases& b, c
       case ST_INGEST_DY: {
         const int hH = d.height << P.L, hW = d.width << P.L;
         const long long npix = (long long)d.batch * hH * hW;
-        ingest_grad_kernel<<<(int)((npix + 127) / 128), 128, 0, st>>>((const float*)b.dy, (const unsigned char*)((char*)b.ws + P.o_cmask), d.batch,
-                                                                     d.out_channels, hH, hW, (__nv_bfloat16*)((char*)b.ws + P.o_dyp), 64);
+        (P.unclamped ? ingest_grad_kernel<false> : ingest_grad_kernel<true>)<<<(int)((npix + 127) / 128), 128, 0, st>>>(
+            (const float*)b.dy, (const unsigned char*)((char*)b.ws + P.o_cmask), d.batch, d.out_channels, hH, hW,
+            (__nv_bfloat16*)((char*)b.ws + P.o_dyp), 64);
         CUDA_TRY(cudaGetLastError());
         break;
       }
@@ -2301,7 +2304,7 @@ static int build_disc_plan(b200sr_plan& P) {
 extern "C" {
 
 const char* b200sr_last_error(void) { return g_err; }
-int b200sr_version(void) { return 102; }
+int b200sr_version(void) { return 103; }
 void b200sr_debug_set(int flags) { g_debug = flags; }
 int b200sr_debug_read_profile(unsigned long long* out_host, int n) {
   CUDA_TRY(cudaMemcpyFromSymbol(out_host, g_conv_prof, sizeof(unsigned long long) * (size_t)n));
@@ -2315,11 +2318,12 @@ int b200sr_debug_buffer(const b200sr_plan* p, const char* name, int64_t* offset_
   return fail(B200SR_ERR_INVALID, "the plan has no workspace tensor named '%s'", name);
 }
 
-static int net_plan_create(const b200sr_net_desc* desc, bool trunk, b200sr_plan** out) {
+static int net_plan_create(const b200sr_net_desc* desc, bool trunk, bool unclamped, b200sr_plan** out) {
   if (!desc || !out) return fail(B200SR_ERR_INVALID, "null argument");
   b200sr_plan* p = new b200sr_plan();
   p->d = *desc;
   p->trunk = trunk;
+  p->unclamped = unclamped;
   p->det = desc->deterministic != 0;
   if (const char* e = getenv("B200SR_REASSOC")) p->reassoc = atoi(e) != 0;  // 0: per-conv schedule everywhere
   p->tail_f16 = desc->training == 0;  // training: the L1 loss' sign(sr - gt) amplifies the fp16 rounding of the tail past the 1e-2 gradient bar
@@ -2330,8 +2334,9 @@ static int net_plan_create(const b200sr_net_desc* desc, bool trunk, b200sr_plan*
   return 0;
 }
 
-int b200sr_plan_create(const b200sr_net_desc* desc, b200sr_plan** out) { return net_plan_create(desc, false, out); }
-int b200sr_trunk_plan_create(const b200sr_net_desc* desc, b200sr_plan** out) { return net_plan_create(desc, true, out); }
+int b200sr_plan_create(const b200sr_net_desc* desc, b200sr_plan** out) { return net_plan_create(desc, false, false, out); }
+int b200sr_unclamped_plan_create(const b200sr_net_desc* desc, b200sr_plan** out) { return net_plan_create(desc, false, true, out); }
+int b200sr_trunk_plan_create(const b200sr_net_desc* desc, b200sr_plan** out) { return net_plan_create(desc, true, false, out); }
 
 void b200sr_plan_destroy(b200sr_plan* p) {
   if (!p) return;

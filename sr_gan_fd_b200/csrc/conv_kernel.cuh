@@ -38,7 +38,7 @@ enum StoreMode : int {
   kStorePix = 0,        // same lattice position
   kStoreShuffle = 1,    // pixel-shuffle: column group (col / 64) = phase (a, b) -> pixel (2y+a, 2x+b), channel col % 64
   kStoreUnshuffle = 2,  // pixel-unshuffle: pixel (y, x) -> (y/2, x/2), channel ((y&1)*2 + (x&1)) * 64 + col
-  kStoreFinal = 3,      // clamp to [0,1], NCHW fp32 image + clamp mask bytes (generator output head)
+  kStoreFinal = 3,      // clamp to [0,1], NCHW fp32 image + clamp mask bytes (generator output head); epi.unclamped: no clamp, no mask
   kStoreNCHW = 4        // plain NCHW fp32 store of channels < n_valid to the per-launch output pointer (gradient w.r.t. the LR input)
 };
 
@@ -81,6 +81,8 @@ struct ConvEpilogue {
   int shuf_c;
   int f16;  // 1: this layer's 16-bit operands / outputs / residual are fp16 instead of bf16 (same tcgen05 kind::f16 instruction): the
             // generator's head / tail convs (one fp16 product instead of three split-bf16 ones) and the discriminator plans
+  int unclamped;  // kStoreFinal only: store the conv output as it is, no clamp (unclamped generator plans; clamp_mask is nullptr).
+                  // Occupies what was the struct's tail padding: sizeof(ConvParams) and the staging copy are unchanged
 };
 
 struct ConvParams {
@@ -261,11 +263,12 @@ __device__ __forceinline__ void conv_epilogue_write(const HW p, const ConvEpilog
     if (!ok) return;
     const long long plane = static_cast<long long>(p.H) * p.W;
     const long long base = static_cast<long long>(n) * e.n_valid * plane + static_cast<long long>(y) * p.W + x;
+    const bool unclamped = e.unclamped;  // read once: the stores below are volatile asm, which would reload it per channel
 #pragma unroll
     for (int i = 0; i < 16; ++i) {
       if (i < e.n_valid) {
         float pre = v[i];
-        float cl = fminf(fmaxf(pre, 0.f), 1.f);
+        float cl = unclamped ? pre : fminf(fmaxf(pre, 0.f), 1.f);
         st_global_f32(y_dyn + base + i * plane, cl);  // the generator output tensor is passed per launch, not baked into the layer list
         if (e.clamp_mask) st_global_u8(e.clamp_mask + base + i * plane, (pre >= 0.f && pre <= 1.f) ? 1u : 0u);
       }

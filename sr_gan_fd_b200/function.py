@@ -28,7 +28,12 @@ class _Plan:
                           desc["num_blocks"], desc["n_up"], batch, height, width, 1 if training else 0, grad_bucket_rrdbs,
                           1 if deterministic else 0)
         handle = C.c_void_p()
-        create = lib.b200sr_trunk_plan_create if desc.get("trunk_only") else lib.b200sr_plan_create
+        if desc.get("trunk_only"):
+            create = lib.b200sr_trunk_plan_create
+        elif desc.get("clamp", 1) == 0:  # generators whose output is conv4's (BasicSR layout)
+            create = lib.b200sr_unclamped_plan_create
+        else:
+            create = lib.b200sr_plan_create
         _lib.check(create(C.byref(nd), C.byref(handle)))
         self.handle = handle
         self.training = training

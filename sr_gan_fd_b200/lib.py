@@ -36,6 +36,7 @@ _lib = None
 SIGNATURES = {
     "b200sr_plan_create": (C.c_int, [C.POINTER(NetDesc), C.POINTER(C.c_void_p)]),
     "b200sr_trunk_plan_create": (C.c_int, [C.POINTER(NetDesc), C.POINTER(C.c_void_p)]),
+    "b200sr_unclamped_plan_create": (C.c_int, [C.POINTER(NetDesc), C.POINTER(C.c_void_p)]),
     "b200sr_plan_destroy": (None, [C.c_void_p]),
     "b200sr_workspace_bytes": (C.c_size_t, [C.c_void_p]),
     "b200sr_packed_bytes": (C.c_size_t, [C.c_void_p]),

@@ -18,12 +18,13 @@ from collections import OrderedDict
 from typing import Any, List
 
 import torch
+import torch.nn.functional as F
 from torch import nn
 
 from . import function as _function
 
 __all__ = [
-    "RRDBNet", "BSRGAN", "RealRRDBNet", "RRDBTrunk", "native_trunk",
+    "RRDBNet", "BSRGAN", "RealRRDBNet", "RRDBTrunk", "native_trunk", "BasicSRRRDBNet", "native_generator",
     "rrdbnet_x1", "rrdbnet_x2", "rrdbnet_x4", "rrdbnet_x8", "bsrgan_x2", "bsrgan_x4", "real_rrdbnet_x4",
 ]
 
@@ -288,6 +289,14 @@ def native_trunk(seq: nn.Sequential) -> RRDBTrunk:
     the contract in :class:`RRDBTrunk`'s docstring and nothing else."""
     if isinstance(seq, RRDBTrunk):
         return seq
+    _check_rrdb_stack(seq)
+    return _adopt(OrderedDict(seq.named_children()))
+
+
+def _check_rrdb_stack(seq: nn.Module) -> None:
+    """Raise ``ValueError`` unless ``seq`` is what :func:`native_trunk` accepts (an :class:`RRDBTrunk` always is)."""
+    if isinstance(seq, RRDBTrunk):
+        return
     if not isinstance(seq, nn.Sequential) or len(seq) == 0:
         raise ValueError("native_trunk expects a non-empty nn.Sequential of RRDBs")
     for name, rrdb in seq.named_children():
@@ -301,14 +310,124 @@ def native_trunk(seq: nn.Sequential) -> RRDBTrunk:
             if params != expect or any(True for _ in rdb.named_buffers()):
                 raise ValueError(f"{name}.{r}: expected the parameters of conv1..conv5 and nothing else, got {sorted(params)}")
             for k in range(1, 6):
-                conv = getattr(rdb, f"conv{k}")
-                cin, cout = 64 + 32 * (k - 1), 32 if k < 5 else 64
-                if not (type(conv) is nn.Conv2d and conv.in_channels == cin and conv.out_channels == cout and
-                        conv.kernel_size == (3, 3) and conv.stride == (1, 1) and conv.padding == (1, 1) and
-                        conv.dilation == (1, 1) and conv.groups == 1 and conv.padding_mode == "zeros" and conv.bias is not None):
-                    raise ValueError(f"{name}.{r}.conv{k}: expected a 3x3 Conv2d({cin}, {cout}), stride 1, padding 1, with bias; "
-                                     f"got {conv!r}")
-    return _adopt(OrderedDict(seq.named_children()))
+                _check_conv3x3(getattr(rdb, f"conv{k}"), f"{name}.{r}.conv{k}", 64 + 32 * (k - 1), 32 if k < 5 else 64)
+
+
+def _check_conv3x3(conv: nn.Module, name: str, cin: int, cout: int) -> None:
+    """Raise ``ValueError`` unless ``conv`` is a 3x3 ``nn.Conv2d(cin, cout)``, stride 1, padding 1, with bias: the only conv the native
+    kernels compute."""
+    if not (type(conv) is nn.Conv2d and conv.in_channels == cin and conv.out_channels == cout and
+            conv.kernel_size == (3, 3) and conv.stride == (1, 1) and conv.padding == (1, 1) and
+            conv.dilation == (1, 1) and conv.groups == 1 and conv.padding_mode == "zeros" and conv.bias is not None):
+        raise ValueError(f"{name}: expected a 3x3 Conv2d({cin}, {cout}), stride 1, padding 1, with bias; got {conv!r}")
+
+
+class BasicSRRRDBNet(_GeneratorBase):
+    """BasicSR's ``RRDBNet`` (``basicsr/archs/rrdbnet_arch.py``), the generator of the Real-ESRGAN release checkpoints: same
+    constructor, children (``conv_first``, ``body``, ``conv_body``, ``conv_up1``, ``conv_up2``, ``conv_hr``, ``conv_last``,
+    ``lrelu``), init and ``state_dict``, so a Real-ESRGAN ``params_ema`` dict loads unchanged.  ``scale`` 2 and 1 pixel-unshuffle
+    the input by 2 and 4 first (``conv_first`` takes ``num_in_ch * 4`` / ``* 16`` channels).  Math::
+
+        feat = conv_first(unshuffle(x));  feat = feat + conv_body(body(feat))        (body: the RRDBs of RRDBTrunk)
+        feat = lrelu(conv_up1(nearest_x2(feat)));  feat = lrelu(conv_up2(nearest_x2(feat)))
+        out  = conv_last(lrelu(conv_hr(feat)))                                        -- NOT clamped
+
+    On a CUDA device forward and backward run in the generator's kernels through an unclamped plan (``include/b200sr.h``
+    "Unclamped plans"); on the CPU the children run through stock torch ops.  Adopt an existing module of this layout with
+    :func:`native_generator`."""
+
+    _n_up = 2
+
+    def __init__(self, num_in_ch: int, num_out_ch: int, scale: int = 4, num_feat: int = 64, num_block: int = 23,
+                 num_grow_ch: int = 32) -> None:
+        super().__init__()
+        if scale not in (1, 2, 4):
+            raise ValueError(f"BasicSRRRDBNet supports scale 1, 2 and 4, got {scale}")
+        self._set_scale(scale)
+        self.conv_first = nn.Conv2d(num_in_ch * self._pixel_unshuffle ** 2, num_feat, 3, 1, 1)
+        # BasicSR's ResidualDenseBlock runs default_init_weights(..., 0.1) in its constructor: the reinit=True dense block
+        self.body = nn.Sequential(*[_ResidualResidualDenseBlock(num_feat, num_grow_ch, reinit=True) for _ in range(num_block)])
+        self.conv_body = nn.Conv2d(num_feat, num_feat, 3, 1, 1)
+        self.conv_up1 = nn.Conv2d(num_feat, num_feat, 3, 1, 1)
+        self.conv_up2 = nn.Conv2d(num_feat, num_feat, 3, 1, 1)
+        self.conv_hr = nn.Conv2d(num_feat, num_feat, 3, 1, 1)
+        self.conv_last = nn.Conv2d(num_feat, num_out_ch, 3, 1, 1)
+        self.lrelu = nn.LeakyReLU(negative_slope=0.2, inplace=True)
+
+    def _set_scale(self, scale: int) -> None:
+        self.scale = self.upscale_factor = scale
+        self._pixel_unshuffle = {4: 1, 2: 2, 1: 4}[scale]
+
+    def _conv_list(self) -> List[nn.Conv2d]:
+        convs = [self.conv_first]
+        for rrdb in self.body:
+            for rdb in (rrdb.rdb1, rrdb.rdb2, rrdb.rdb3):
+                convs += [rdb.conv1, rdb.conv2, rdb.conv3, rdb.conv4, rdb.conv5]
+        return convs + [self.conv_body, self.conv_up1, self.conv_up2, self.conv_hr, self.conv_last]
+
+    def net_desc(self) -> dict:
+        return dict(in_channels=self.conv_first.in_channels, out_channels=self.conv_last.out_channels,
+                    channels=self.conv_first.out_channels, growth=self.body[0].rdb1.conv1.out_channels, num_blocks=len(self.body),
+                    n_up=2, pixel_unshuffle=self._pixel_unshuffle, clamp=0)
+
+    def _forward_impl(self, x: torch.Tensor) -> torch.Tensor:
+        if self._pixel_unshuffle > 1:  # pure data movement on the few input channels; kept as the torch op
+            x = F.pixel_unshuffle(x, self._pixel_unshuffle)
+        if x.dim() == 4 and not x.is_cuda:
+            return self._eager_forward(x)
+        return _function.generator_forward(self, x)
+
+    def _eager_forward(self, x: torch.Tensor) -> torch.Tensor:
+        feat = self.conv_first(x)
+        feat = feat + self.conv_body(_function.eager_trunk(self.body, feat))
+        feat = self.lrelu(self.conv_up1(F.interpolate(feat, scale_factor=2, mode="nearest")))
+        feat = self.lrelu(self.conv_up2(F.interpolate(feat, scale_factor=2, mode="nearest")))
+        return self.conv_last(self.lrelu(self.conv_hr(feat)))
+
+
+_BASICSR_CHILDREN = ["conv_first", "body", "conv_body", "conv_up1", "conv_up2", "conv_hr", "conv_last", "lrelu"]
+
+
+def native_generator(model: nn.Module) -> BasicSRRRDBNet:
+    """A :class:`BasicSRRRDBNet` that adopts the children of ``model``, a module of BasicSR's ``RRDBNet`` layout (for example an
+    instance of BasicSR's own class).  The same module objects are kept: Parameter identity, optimizer state and the ``state_dict``
+    (keys, order and values) are unchanged.  Usage: ``net = native_generator(net)``.
+
+    ``model`` must have exactly the children ``conv_first``, ``body``, ``conv_body``, ``conv_up1``, ``conv_up2``, ``conv_hr``,
+    ``conv_last``, ``lrelu`` in that order, a ``scale`` of 1, 2 or 4, 64 features, a ``body`` that :func:`native_trunk` accepts,
+    3x3 convs with bias, a LeakyReLU(0.2) and no other parameters or buffers.  Anything else raises ``ValueError``."""
+    if isinstance(model, BasicSRRRDBNet):
+        return model
+    names = [n for n, _ in model.named_children()]
+    if names != _BASICSR_CHILDREN:
+        raise ValueError(f"expected the children {_BASICSR_CHILDREN} of BasicSR's RRDBNet, got {names}")
+    if any(True for _ in model.named_parameters(recurse=False)) or any(True for _ in model.named_buffers(recurse=False)):
+        raise ValueError("the model holds parameters or buffers of its own besides its children's")
+    scale = getattr(model, "scale", None)
+    if scale not in (1, 2, 4):
+        raise ValueError(f"the BasicSR layout runs natively at scale 1, 2 and 4, got {scale!r}")
+    unshuffle = {4: 1, 2: 2, 1: 4}[scale]
+    cin, cout = model.conv_first.in_channels, model.conv_last.out_channels
+    if cin % (unshuffle * unshuffle) or not 1 <= cin <= 64:
+        raise ValueError(f"conv_first takes {cin} channels: not a multiple of {unshuffle * unshuffle} in [1, 64] (scale {scale})")
+    if not 1 <= cout <= 16:
+        raise ValueError(f"conv_last gives {cout} channels, the native tail supports 1..16")
+    for name, ci, co in (("conv_first", cin, 64), ("conv_body", 64, 64), ("conv_up1", 64, 64), ("conv_up2", 64, 64),
+                         ("conv_hr", 64, 64), ("conv_last", 64, cout)):
+        conv = getattr(model, name)
+        _check_conv3x3(conv, name, ci, co)
+        if [n for n, _ in conv.named_parameters()] != ["weight", "bias"] or any(True for _ in conv.named_buffers()):
+            raise ValueError(f"{name}: expected the parameters weight and bias and nothing else")
+    if not (type(model.lrelu) is nn.LeakyReLU and model.lrelu.negative_slope == 0.2):
+        raise ValueError(f"lrelu: expected LeakyReLU(negative_slope=0.2), got {model.lrelu!r}")
+    _check_rrdb_stack(model.body)
+    net = BasicSRRRDBNet.__new__(BasicSRRRDBNet)
+    nn.Module.__init__(net)
+    net._set_scale(scale)
+    for name, child in model.named_children():
+        net.add_module(name, child)
+    net.train(model.training)
+    return net
 
 
 # --- factories (names the reference scripts look up with model.__dict__[arch]) ------------------------------------
