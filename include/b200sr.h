@@ -273,7 +273,13 @@ int b200sr_debug_read_profile(unsigned long long* out_host, int n);
  * plans, "GR" "GC1" "GC2" and the "DYB" buffers): "xin", the fp32 carriers "T0" "TR" "C1" "C2" (tile-blocked),
  * the dense-block buffers "D0" ... "D{R-1}" (R = 3 * num_blocks; inference plans keep only the ping-pong pair "D0" "D1"), the
  * tail activations "SPLT" "SPL0" ... "SPL{n_up}" "SPLC" and, in training plans, "CMASK" (not in unclamped plans) "DYP" "G3"
- * "GU1" ... "GU{n_up}" "GT" "GTB" "GR" "GC1" "GC2" "GO1" "DYB0" ... "DYB{R-1}".  VGG plans name none. */
+ * "GU1" ... "GU{n_up}" "GT" "GTB" "GR" "GC1" "GC2" "GO1" "DYB0" ... "DYB{R-1}".  VGG plans (build_vgg_plan; l = conv index, h_l x w_l
+ * its lattice, C_l its output channels, N = batch, NB = grad_images) name: "xin" [N, H, W, 64] bf16 [hi(3) | lo(3) | hi(3) | 0] of
+ * (x - mean) / std; "A{l}" (l <= last_conv) [N, h_l, w_l, C_l] bf16, conv l's output after the ReLU; "P{l}" (l = 1, 3, 7, 11 and
+ * l < last_conv) [N, h_l/2, w_l/2, C_l] bf16, its 2x2 max-pool; "F{l}" (feat_mask bit l) [N, h_l, w_l, C_l] fp32, the feature node
+ * (before the ReLU for l == last_conv, after it otherwise); and in plans with a gradient request "G{l}" (l <= grad_conv)
+ * [NB, h_l, w_l, C_l] bf16, the gradient w.r.t. conv l's pre-activation output, and "GP{l}" (pool after l, l < grad_conv)
+ * [NB, h_l/2, w_l/2, C_l] bf16, that gradient on the pooled lattice. */
 int b200sr_debug_buffer(const b200sr_plan* plan, const char* name, int64_t* offset_bytes, int64_t* bytes);
 
 #ifdef __cplusplus

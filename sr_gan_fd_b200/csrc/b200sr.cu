@@ -1870,23 +1870,25 @@ static int build_vgg_plan(b200sr_plan& P) {
   }
   int h = v.height, w = v.width;
   P.xin_stride = 64;
-  P.o_xin = B.alloc((long long)N * h * w * 64 * 2);
+  P.o_xin = B.alloc("xin", (long long)N * h * w * 64 * 2);
   std::vector<long long> o_act(NL, 0), o_pool(NL, 0);
   for (int l = 0; l < NL; ++l) {
     if (h < 1 || w < 1) return fail(B200SR_ERR_INVALID, "input too small for conv %d", l);
     P.vgg_h[l] = h; P.vgg_w[l] = w;
-    o_act[l] = B.alloc((long long)N * h * w * kVggCout[l] * 2);
-    if ((v.feat_mask >> l) & 1) P.o_vgg_feat[l] = B.alloc((long long)N * h * w * kVggCout[l] * 4) + 1;  // +1: 0 means absent
+    const std::string ls = std::to_string(l);
+    o_act[l] = B.alloc("A" + ls, (long long)N * h * w * kVggCout[l] * 2);
+    if ((v.feat_mask >> l) & 1) P.o_vgg_feat[l] = B.alloc("F" + ls, (long long)N * h * w * kVggCout[l] * 4) + 1;  // +1: 0 means absent
     if (kVggPoolAfter[l] && l + 1 < NL) {
-      o_pool[l] = B.alloc((long long)N * (h >> 1) * (w >> 1) * kVggCout[l] * 2);
+      o_pool[l] = B.alloc("P" + ls, (long long)N * (h >> 1) * (w >> 1) * kVggCout[l] * 2);
       h >>= 1; w >>= 1;
     }
   }
   std::vector<long long> o_gpool(NL, 0);
   if (bwd) {
     for (int l = 0; l <= v.grad_conv; ++l) {
-      P.o_vgg_g[l] = B.alloc((long long)NB * P.vgg_h[l] * P.vgg_w[l] * kVggCout[l] * 2) + 1;
-      if (kVggPoolAfter[l] && l + 1 <= v.grad_conv) o_gpool[l] = B.alloc((long long)NB * (P.vgg_h[l] >> 1) * (P.vgg_w[l] >> 1) * kVggCout[l] * 2);
+      const std::string ls = std::to_string(l);
+      P.o_vgg_g[l] = B.alloc("G" + ls, (long long)NB * P.vgg_h[l] * P.vgg_w[l] * kVggCout[l] * 2) + 1;
+      if (kVggPoolAfter[l] && l + 1 <= v.grad_conv) o_gpool[l] = B.alloc("GP" + ls, (long long)NB * (P.vgg_h[l] >> 1) * (P.vgg_w[l] >> 1) * kVggCout[l] * 2);
     }
   }
   if (P.det) P.o_det = B.alloc(kVggL1MaxBlocks * sizeof(double));  // per-block partials of b200sr_vgg_feature_l1
@@ -2847,8 +2849,9 @@ int b200sr_vgg_backward(b200sr_plan* p, const float* upstream, const void* packe
   if (rc) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   const long long half = (long long)nb * p->vgg_h[gc] * p->vgg_w[gc] * kVggCout[gc];
+  const int post_relu = gc < p->vd.last_conv;  // the node's feature was stored after its ReLU (build_vgg_plan, mask_relu bit 1)
   vgg_l1_grad_kernel<<<(unsigned)((half / 4 + 255) / 256), 256, 0, st>>>((const float*)((char*)workspace + p->o_vgg_feat[gc] - 1), half, upstream,
-                                                                         (__nv_bfloat16*)((char*)workspace + p->o_vgg_g[gc] - 1));
+                                                                         post_relu, (__nv_bfloat16*)((char*)workspace + p->o_vgg_g[gc] - 1));
   CUDA_TRY(cudaGetLastError());
   Bases b{workspace, (void*)packed, dx, nullptr, nullptr};
   return run_steps(*p, p->bwd, b, nullptr, 0, nullptr, nullptr, nullptr, (cudaStream_t)stream);

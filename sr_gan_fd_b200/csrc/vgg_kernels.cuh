@@ -129,16 +129,23 @@ __global__ void __launch_bounds__(256) vgg_l1_pair_sum_kernel(const float* __res
   }
 }
 
-// g[i] = bf16(sign(f[i] - f[i + half]) * scale[0] / half): gradient of mean |f_sr - f_gt| w.r.t. f_sr times the upstream gradient
-__global__ void vgg_l1_grad_kernel(const float* __restrict__ f, long long half, const float* __restrict__ scale, __nv_bfloat16* __restrict__ g) {
+// g[i] = bf16(sign(f[i] - f[i + half]) * scale[0] / half): gradient of mean |f_sr - f_gt| w.r.t. f_sr times the upstream gradient.
+// g is the gradient w.r.t. the conv's PRE-activation output.  post_relu: f holds max(pre, 0) (a feature node before the last conv),
+// so the ReLU derivative [f_sr > 0] -- equal to [pre > 0], f being fmaxf(pre, 0) in fp32 -- multiplies the sign.
+__global__ void vgg_l1_grad_kernel(const float* __restrict__ f, long long half, const float* __restrict__ scale, int post_relu,
+                                   __nv_bfloat16* __restrict__ g) {
   const long long i = (static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x) * 4;
   if (i >= half) return;
   const float s = scale[0] / static_cast<float>(half);
   const float4 a = *reinterpret_cast<const float4*>(f + i), b = *reinterpret_cast<const float4*>(f + half + i);
-  auto sg = [&](float d) { return d > 0.f ? s : (d < 0.f ? -s : 0.f); };
+  auto sg = [&](float fs, float fg) {
+    if (post_relu && !(fs > 0.f)) return 0.f;
+    const float d = fs - fg;
+    return d > 0.f ? s : (d < 0.f ? -s : 0.f);
+  };
   uint2 o;
-  o.x = pack_bf16x2(sg(a.x - b.x), sg(a.y - b.y));
-  o.y = pack_bf16x2(sg(a.z - b.z), sg(a.w - b.w));
+  o.x = pack_bf16x2(sg(a.x, b.x), sg(a.y, b.y));
+  o.y = pack_bf16x2(sg(a.z, b.z), sg(a.w, b.w));
   *reinterpret_cast<uint2*>(g + i) = o;
 }
 

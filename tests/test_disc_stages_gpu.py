@@ -118,7 +118,11 @@ def test_debug_buffer_rejects_unknown_and_foreign_names(L):
     handle = C.c_void_p()
     assert L.b200sr_vgg_plan_create(C.byref(vd), C.byref(handle)) == 0
     try:
-        assert _lookup(L, handle, "xin")[0] == -1
+        # a VGG plan names its own tensors (test_vgg_stages_gpu.py): every discriminator-only name is rejected
+        for name in set(FWD_LAYOUT) | set(BWD_LAYOUT):
+            if name not in ("xin", "A1", "A2", "A3", "A4", "A5"):
+                assert _lookup(L, handle, name)[0] == -1, name
+        assert _lookup(L, handle, "xin")[2] == 2 * 32 * 32 * 64 * 2  # [hi(3) | lo(3) | hi(3) | 0], 64 channels
     finally:
         L.b200sr_plan_destroy(handle)
 
@@ -171,6 +175,7 @@ def _up_adjoint(g):
 class _Stages:
     """collects every stage's worst normalised error before anything is asserted, so one run reports them all; worst_index is
     (image among the checked ones, channel, y, x) of the NCHW view, or the index into the weight / bias gradient"""
+    jsonl = "disc_stages.jsonl"
 
     def __init__(self, case, fmt):
         self.case, self.fmt, self.rows = case, fmt, []
@@ -202,7 +207,7 @@ class _Stages:
 
     def finish(self):
         for row in self.rows:
-            _record(self.case, row, "disc_stages.jsonl")
+            _record(self.case, row, self.jsonl)
         scored = [r for r in self.rows if "gamma_needed" in r]
         if scored:
             worst = max(scored, key=lambda r: r["gamma_needed"] / BARS[r["format"]][0])
